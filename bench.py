@@ -21,6 +21,10 @@ config-2 and config-5-row blocks.
 
 --impl reference times the reference's CPU algorithm (oracle port of CafRustFFTThreadpool, all host
 cores) on the same workload; the Rust crate itself cannot be compiled in this image (DESIGN.md).
+
+--dump-outputs DIR writes what the timed path returned in its last timed step (rank 0) as DIR/<name>.npy, float64
+(float32 for cfg2's surface and row peak values): surface, row_peak_value, row_peak_index and peak.  The inputs are seeded, so two
+builds run with the same arguments can be compared array for array.  The bench writes nothing into the source tree.
 """
 from __future__ import annotations
 
@@ -36,6 +40,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the bench writes nothing into the tree: it imports modules the build never does (scripts/bench_stream,
+# caf_cookoff_b200.generate / .dist), whose bytecode caches would otherwise be created next to them
+sys.dont_write_bytecode = True
 
 FS = 48000
 L = 4096
@@ -69,6 +76,22 @@ def emit(line: dict):
         sys.stdout.write(data.decode()); sys.stdout.flush()
     else:
         os.write(_JSON_FD, data)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, surface, row_peak_val, row_peak_idx, peak):
+    """The outputs of one step as the caller receives them: the D x 2L surface, every row's peak value and delay index,
+    and find_peak's answer as [value, freq_hz, doppler_idx, delay_idx].  Indices are stored as float64 (exact below 2^53)."""
+    arrays = {"surface": np.asarray(surface), "row_peak_value": np.asarray(row_peak_val),
+              "row_peak_index": np.asarray(row_peak_idx).astype(np.float64),
+              "peak": np.asarray(peak, dtype=np.float64)}
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def algorithmic_flops(d: int, n: int) -> float:
@@ -496,17 +519,15 @@ def run_reference(args):
     from oracle import oracle as O
     for _ in range(max(args.warmup, 1)):
         O.caf_surface(needle, hay, freqs, FS, threads=threads, want_surface=True)
-    # a bounded sample: at most 400 surfaces / ~60 s whatever --steps says (the GPU arm's K is sized for 50 us steps)
-    steps = max(1, min(args.steps, 400))
     times = []
-    t_end = time.perf_counter() + 60.0
-    for _ in range(steps):
+    for _ in range(args.steps):
         t0 = time.perf_counter()
         surf, pidx, pval = O.caf_surface(needle, hay, freqs, FS, threads=threads, want_surface=True)
         pk = O.find_peak(freqs, pidx, pval)
         times.append(time.perf_counter() - t0)
-        if time.perf_counter() > t_end:
-            break
+    if args.dump_outputs:
+        row = int(np.argmax(pval))         # find_peak's strict `>` keeps the first row holding the maximum
+        dump_outputs(args.dump_outputs, surf, pval, pidx, [pval[row], pk[0], row, pk[1]])
     med = float(np.median(times))          # the same statistic the GPU arm's cpu_baseline reports
     cells = freqs.size * N
     value = cells / med
@@ -644,6 +665,13 @@ def run_b200(args):
     barrier()
     sampler.stop()
     launches = h.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        k_last = warm + args.steps - 1          # its surface buffer is not written again before this copy
+        i_last = k_last % n_pairs
+        pk_last = pk_all[i_last].cpu().numpy()
+        dump_outputs(args.dump_outputs, surfs[k_last % n_surf].cpu().numpy(), rv_all[i_last].cpu().numpy(),
+                     ri_all[i_last].cpu().numpy(), [pk_last.view(np.float64)[0], pk_last.view(np.float64)[1],
+                                                    pk_last.view(np.uint64)[2], pk_last.view(np.uint64)[3]])
     total_ms = float(e0.elapsed_time(e1))
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -974,7 +1002,10 @@ def main():
     ap.add_argument("--cpu-budget-s", type=float, default=3.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-blocks", action="store_true", help="skip the cfg2/cfg3/cfg4/cfg5 blocks (development)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     claim_stdout()
     if args.impl == "reference":
         run_reference(args)

@@ -7,7 +7,11 @@ import os
 import subprocess
 import sys
 
-from conftest import ROOT
+import numpy as np
+import pytest
+
+from conftest import FS, ROOT, rel_max
+from oracle import oracle as O
 
 REQUIRED = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better",
             "scaling", "vs_baseline", "dtype", "data", "config", "e2e", "cpu_baseline")
@@ -45,3 +49,56 @@ def test_reference_arm_other_ranks_exit_without_work():
     r = run_bench({"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"}, "--gpus", "2", "--steps", "2", "--warmup", "1")
     assert r.returncode == 0, r.stderr[-2000:]
     assert r.stdout.strip() == ""
+
+
+def test_steps_must_be_positive():
+    r = run_bench(None, "--steps", "0")
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
+DUMPED = ("peak", "row_peak_index", "row_peak_value", "surface")
+
+
+def load_dump(path, dtype):
+    assert sorted(os.listdir(path)) == [n + ".npy" for n in DUMPED]
+    got = {n: np.load(os.path.join(path, n + ".npy")) for n in DUMPED}
+    assert got["surface"].dtype == dtype and all(got[n].dtype == np.float64 for n in DUMPED if n != "surface")
+    assert sum(a.nbytes for a in got.values()) <= 64 << 20
+    assert got["surface"].shape == (400, 8192) and got["row_peak_value"].shape == got["row_peak_index"].shape == (400,)
+    assert got["peak"].shape == (4,)
+    return got
+
+
+def test_reference_arm_dumps_its_last_step(tmp_path, chirp0):
+    """--dump-outputs: the surface, the row peaks and find_peak's answer of the README pair on the 0.5 Hz grid."""
+    from caf_cookoff_b200 import bench_shifts
+    r = run_bench(None, "--steps", "2", "--warmup", "0", "--dump-outputs", str(tmp_path))
+    assert r.returncode == 0, r.stderr[-2000:]
+    got = load_dump(tmp_path, np.float64)
+    surf, pidx, pval = O.caf_surface(*chirp0, bench_shifts(), FS)
+    assert rel_max(got["surface"], surf) <= 1e-12
+    assert np.array_equal(got["row_peak_index"], pidx.astype(np.float64))
+    assert np.array_equal(got["row_peak_value"], got["surface"][np.arange(400), pidx.astype(np.int64)])
+    assert list(got["peak"][1:]) == [69.0, 338, 202] and got["peak"][0] == pval.max()
+
+
+@pytest.mark.gpu
+def test_b200_arm_dumps_its_last_timed_step(tmp_path):
+    """The b200 arm runs exactly --steps timed launches and dumps the last one: rotation pair (warmup + steps - 1) mod 320,
+    drawn ten per seed from seed 0 on rank 0, against the oracle on the same inputs."""
+    from caf_cookoff_b200 import bench_shifts, generate as G
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "8", "--warmup", "3", "--no-blocks",
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       cwd=ROOT, capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout)
+    assert line["steps"] == 8 and line["gpu_launches"] == 8 and line["check_ok"]
+    got = load_dump(tmp_path, np.float64)
+    needle, hay = G.as_inputs(G.pair(0, seed=1))                  # last timed step k = 3 + 8 - 1 = 10: seed 1, pair 0
+    freqs = bench_shifts()
+    surf, pidx, pval = O.caf_surface(needle, hay[:needle.size], freqs, FS, threads=os.cpu_count() or 1)
+    assert rel_max(got["surface"], surf) <= 1e-9
+    assert np.array_equal(got["row_peak_index"], pidx.astype(np.float64))
+    assert rel_max(got["row_peak_value"], pval) <= 1e-9
+    freq, delay = O.find_peak(freqs, pidx, pval)
+    assert (got["peak"][1], got["peak"][3]) == (freq, delay) and got["peak"][2] == int(np.argmax(pval))

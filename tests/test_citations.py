@@ -1,5 +1,7 @@
 """Every `file:line` citation of the reference in the boundary header, the oracle and the design documents points
-inside a file that exists under /root/reference (skipped where the reference is absent, e.g. on the GPU box)."""
+inside a file that exists in the reference project (Teque5/caf_cookoff).  The reference is not part of this repository
+and no stored copy of its line counts or cited lines exists yet (tests/golden/ has none), so these tests read a checkout
+of it from CAF_REFERENCE_DIR and skip without one."""
 import os
 import re
 
@@ -7,7 +9,8 @@ import pytest
 
 from conftest import ROOT
 
-REF = "/root/reference"
+REF = os.environ.get("CAF_REFERENCE_DIR", "")
+NO_REF = "needs a checkout of the reference project in CAF_REFERENCE_DIR"
 DOCS = ["include/caf_b200.h", "include/caf_b200.hpp", "oracle/caf_oracle.c", "oracle/np_oracle.py", "oracle/oracle.py",
         "DESIGN.md", "INTEGRATION.md", "caf_cookoff_b200/api.py", "caf_cookoff_b200/io.py", "caf_cookoff_b200/generate.py",
         "caf_cookoff_b200/siblings.py", "caf_cookoff_b200/dist.py", "tools/caf_cli.cpp", "rust/src/caf/mod.rs",
@@ -30,7 +33,7 @@ def _index():
     return by_name
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree is only present in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason=NO_REF)
 def test_reference_citations_point_inside_existing_files():
     by_name = _index()
     lengths = {}
@@ -78,7 +81,7 @@ KEY = [
 ]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree is only present in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF), reason=NO_REF)
 @pytest.mark.parametrize("path,first,last,needle", KEY, ids=lambda v: str(v))
 def test_key_citations_hold_what_they_name(path, first, last, needle):
     lines = open(os.path.join(REF, path), errors="replace").read().splitlines()
