@@ -9,49 +9,51 @@ import pytest
 from caf_cookoff_b200 import _lib
 from conftest import DATA, ROOT
 
-BIN = os.path.join(ROOT, "tests", "cpp", "test_rs")
+@pytest.fixture(scope="module")
+def out_dir(tmp_path_factory):
+    """Where the native programs are built: outside the repository tree, which may be read-only."""
+    return tmp_path_factory.mktemp("native")
 
 
-def _build():
+def _build(out_dir):
     gxx = shutil.which("g++")
     assert gxx, "g++ is required for the C++ mirror test"
     so_dir = os.path.dirname(_lib.SO_PATH)
+    exe = str(out_dir / "test_rs")
     cmd = [gxx, "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), os.path.join(ROOT, "tests", "cpp", "test_rs.cpp"),
-           "-o", BIN, "-L", so_dir, "-lcaf_b200", f"-Wl,-rpath,{so_dir}"]
+           "-o", exe, "-L", so_dir, "-lcaf_b200", f"-Wl,-rpath,{so_dir}"]
     subprocess.check_call(cmd)
+    return exe
 
 
-def test_cpp_mirror_compiles_without_gpu():
+def test_cpp_mirror_compiles_without_gpu(out_dir):
     """CPU check: the header-only mirror and the C ABI header compile and link against the built library."""
-    _build()
-    assert os.path.exists(BIN)
+    assert os.path.exists(_build(out_dir))
 
 
 @pytest.mark.gpu
-def test_cpp_restatement_of_test_rs():
-    _build()
-    res = subprocess.run([BIN, DATA], capture_output=True, text=True, timeout=300)
+def test_cpp_restatement_of_test_rs(out_dir):
+    res = subprocess.run([_build(out_dir), DATA], capture_output=True, text=True, timeout=300)
     print(res.stdout[-3000:], res.stderr[-2000:])
     assert res.returncode == 0
     assert "all tests passed" in res.stdout
     assert "Frequency offset: 69.0Hz" in res.stdout and "Time offset: 202 samples (4.208ms)" in res.stdout
 
 
-CLI = os.path.join(ROOT, "tools", "caf_cli")
-
-
-def _build_cli():
+def _build_cli(out_dir):
     gxx = shutil.which("g++")
     assert gxx, "g++ is required for the CLI"
     so_dir = os.path.dirname(_lib.SO_PATH)
+    exe = str(out_dir / "caf_cli")
     subprocess.check_call([gxx, "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), os.path.join(ROOT, "tools", "caf_cli.cpp"),
-                           "-o", CLI, "-L", so_dir, "-lcaf_b200", f"-Wl,-rpath,{so_dir}"])
+                           "-o", exe, "-L", so_dir, "-lcaf_b200", f"-Wl,-rpath,{so_dir}"])
+    return exe
 
 
-def test_cli_builds_and_parses_arguments():
+def test_cli_builds_and_parses_arguments(out_dir):
     """CPU: tools/caf_cli (main.rs:10-32 with the arguments its TODO asks for) builds, documents itself and rejects
     bad command lines without touching a GPU."""
-    _build_cli()
+    CLI = _build_cli(out_dir)
     assert "usage: caf_cli NEEDLE.c64 HAYSTACK.c64" in subprocess.run([CLI, "--help"], capture_output=True, text=True).stdout
     assert subprocess.run([CLI, "only_one.c64"], capture_output=True, text=True).returncode == 2
     assert subprocess.run([CLI, "a", "b", "--bogus"], capture_output=True, text=True).returncode == 2
@@ -59,9 +61,9 @@ def test_cli_builds_and_parses_arguments():
 
 
 @pytest.mark.gpu
-def test_cli_prints_what_main_rs_prints(tmp_path):
+def test_cli_prints_what_main_rs_prints(tmp_path, out_dir):
     import numpy as np
-    _build_cli()
+    CLI = _build_cli(out_dir)
     a, b = os.path.join(DATA, "chirp_0_raw.c64"), os.path.join(DATA, "chirp_0_T+202samp_F+69.25Hz.c64")
     res = subprocess.run([CLI, a, b], capture_output=True, text=True, timeout=120)
     assert res.returncode == 0, res.stderr
@@ -85,14 +87,13 @@ def test_cli_prints_what_main_rs_prints(tmp_path):
     assert res.returncode == 0 and res.stdout.startswith("amb_surf (400, 4096) float64 -> 70 83")
 
 
-def test_native_programs_fail_loudly_without_a_gpu():
+def test_native_programs_fail_loudly_without_a_gpu(out_dir):
     """CPU box only: the CLI and the C++ restatement of test.rs stop with the library's ENODEVICE message and a
     non-zero exit code — neither has (or falls back to) a CPU path."""
     import torch
     if torch.cuda.is_available():
         pytest.skip("a GPU is present; the failure path is exercised on the CPU-only box")
-    _build()
-    _build_cli()
+    BIN, CLI = _build(out_dir), _build_cli(out_dir)
     a, b = os.path.join(DATA, "chirp_0_raw.c64"), os.path.join(DATA, "chirp_0_T+202samp_F+69.25Hz.c64")
     res = subprocess.run([CLI, a, b], capture_output=True, text=True, timeout=120)
     assert res.returncode == 1 and res.stdout == ""

@@ -17,6 +17,8 @@ import caf_cookoff_b200 as caf
 from caf_cookoff_b200 import _lib, api
 from conftest import DATA, FS, load_case, rel_max
 from oracle import oracle as O
+from surface_checks import (assert_indices_match_oracle, assert_peak_is_find_peak, assert_peak_matches_oracle,
+                            assert_row_peaks_are_cells, tol_of)
 
 pytestmark = pytest.mark.gpu
 
@@ -338,20 +340,24 @@ def test_repeated_calls_are_deterministic(chirp0):
     assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
 
 
-@pytest.mark.parametrize("l", [1, 2, 3, 17, 100, 1000, 2048, 4095, 4096])
-def test_ragged_lengths(l, chirp0):
-    """Any input length up to 4096 (the reference plans any n): same 2l-cell layout, same peaks."""
+@pytest.mark.parametrize("l,variant", [pytest.param(l, v, id=str(l) if v is api._Variant else f"{l}-f32")
+                                       for v in (api._Variant, api._Variant32) for l in (1, 2, 3, 17, 100, 1000, 2048, 4095, 4096)])
+def test_ragged_lengths(l, variant, chirp0):
+    """Any input length up to 4096 (the reference plans any n): same 2l-cell layout, same peaks, in both precisions."""
     needle, hay = chirp0
     n, h = needle[:l], hay[:l]
+    tol, exact = tol_of(variant), variant.rdt == np.float64
     shifts = np.array([-99.5, -3.25, 0.0, 68.75, 69.25, 70.0])
-    surf, pidx, pval, pk = caf.surface_arrays(n, h, shifts, FS)
+    surf, pidx, pval, pk = caf.surface_arrays(n, h, shifts, FS, variant=variant)
     osurf, opidx, opval = O.caf_surface(n, h, shifts, FS)
-    assert surf.shape == (6, 2 * l)
+    assert surf.shape == (6, 2 * l) and surf.dtype == variant.rdt
     if osurf.max() > 0:
-        assert rel_max(surf, osurf) <= TOL64
+        assert rel_max(surf.astype(np.float64), osurf) <= tol
+    assert_row_peaks_are_cells(surf, pidx, pval, range(6))
     if l >= 100:            # (tiny inputs have near-tied cells; index equality is only meaningful with a real peak)
-        assert np.array_equal(pidx, opidx)
-        assert (pk.freq_hz, int(pk.delay_idx)) == O.find_peak(shifts, opidx, opval)
+        assert_indices_match_oracle(pidx, osurf, opidx, range(6), tol, exact)
+        assert_peak_is_find_peak(pk, shifts, pidx, pval)
+        assert_peak_matches_oracle(pk, opidx, opval, tol, exact)
 
 
 def test_random_inputs_and_odd_grid():
@@ -532,11 +538,12 @@ def test_apply_freq_shift_f32():
     assert rel_max(got.astype(np.complex128), O.apply_freq_shift(x, -31.5, FS)) <= 1e-6
 
 
-@pytest.mark.parametrize("n", [4097, 5000, 16384, 70001, 1 << 19])
+@pytest.mark.parametrize("n", [4097, 5000, 16384, 20000, 40000, 70001, 140000, 1 << 19])
 def test_xcor_any_length(n):
     """Xcor::new(n) plans any n (RustFFT): lengths other than 8192 and <= 4096 go through one row of the long-row kernels
     (complex cells) and a fold of the linear correlation.  Checked against numpy's FFT form of xcor_rustfft.rs:58-76
-    (the C oracle's DFT for non-power-of-two n is O(n^2)) and, for the power of two, against the C oracle."""
+    (the C oracle's DFT for non-power-of-two n is O(n^2)) and, for the power of two, against the C oracle.  The lengths
+    reach every long-row class (top radix 2, 4, 8, 16; two levels 2, 4, 8), in complex128 and complex64."""
     rng = np.random.default_rng(n)
     a = rng.normal(size=n) + 1j * rng.normal(size=n)
     b = rng.normal(size=n) + 1j * rng.normal(size=n)
@@ -545,9 +552,8 @@ def test_xcor_any_length(n):
     assert got.shape == (n,) and rel_max(got, want) <= 1e-12
     if n == 16384:
         assert rel_max(got, O.xcor(a, b)) <= 1e-12
-    if n == 5000:      # the complex64 twin
-        got32 = api.XcorF32.new(n).run(a.astype(np.complex64), b.astype(np.complex64))
-        assert rel_max(got32.astype(np.complex128), want) <= 1e-5
+    got32 = api.XcorF32.new(n).run(a.astype(np.complex64), b.astype(np.complex64))
+    assert got32.dtype == np.complex64 and rel_max(got32.astype(np.complex128), want) <= 1e-5
 
 
 @pytest.mark.parametrize("n", [1, 2, 37, 1000, 4096, 8192])
@@ -559,6 +565,9 @@ def test_xcor(n):
     x = caf.Xcor.new(n)
     assert rel_max(x.run(a, b), O.xcor(a, b)) <= 1e-12
     assert rel_max(x.clone().run(b, a), O.xcor(b, a)) <= 1e-12
+    a32, b32 = a.astype(np.complex64), b.astype(np.complex64)       # the complex64 twin (kXcorFull / kXcorHalf, float)
+    got32 = api.XcorF32.new(n).run(a32, b32)
+    assert got32.dtype == np.complex64 and rel_max(got32.astype(np.complex128), O.xcor(a32, b32)) <= 1e-5
     with pytest.raises(caf.CafPanic):
         x.run(a, b[:-1]) if n > 1 else x.run(a, np.zeros(2, complex))
 
@@ -588,18 +597,24 @@ def _pairs(k):
 
 
 def test_batch_of_pairs_matches_single_calls_and_oracle():
-    """BASELINE config 4 in miniature: independent pairs, one shared grid, more pairs than fit one CTA's range."""
+    """BASELINE config 4 in miniature: independent pairs, one shared grid, more pairs than fit one CTA's range; in
+    complex128 and complex64."""
     ns, hs = _pairs(10)
     shifts = caf.gen_float_shifts(-100.0, 100.0, 5.0)          # 40 rows
-    surf, pidx, pval, peaks = caf.batch_arrays(ns, hs, shifts, FS, want_surface=True)
-    assert surf.shape == (10, 40, 8192)
-    for i in range(10):
-        osurf, opidx, opval = O.caf_surface(ns[i], hs[i], shifts, FS)
-        assert rel_max(surf[i], osurf) <= TOL64
-        assert np.array_equal(pidx[i], opidx)
-        assert (peaks[i].freq_hz, int(peaks[i].delay_idx)) == O.find_peak(shifts, opidx, opval)
-        s1, p1, v1, k1 = caf.surface_arrays(ns[i], hs[i], shifts, FS)
-        assert np.array_equal(s1, surf[i]) and np.array_equal(p1, pidx[i])      # batching does not change a bit
+    oracle = [O.caf_surface(ns[i], hs[i], shifts, FS) for i in range(10)]
+    for variant in (api._Variant, api._Variant32):
+        tol, exact = tol_of(variant), variant.rdt == np.float64
+        surf, pidx, pval, peaks = caf.batch_arrays(ns, hs, shifts, FS, variant=variant, want_surface=True)
+        assert surf.shape == (10, 40, 8192) and surf.dtype == variant.rdt
+        for i in range(10):
+            osurf, opidx, opval = oracle[i]
+            assert rel_max(surf[i].astype(np.float64), osurf) <= tol
+            assert_indices_match_oracle(pidx[i], osurf, opidx, range(40), tol, exact)
+            assert_row_peaks_are_cells(surf[i], pidx[i], pval[i], range(40))
+            assert_peak_is_find_peak(peaks[i], shifts, pidx[i], pval[i])
+            assert_peak_matches_oracle(peaks[i], opidx, opval, tol, exact)
+            s1, p1, v1, k1 = caf.surface_arrays(ns[i], hs[i], shifts, FS, variant=variant)
+            assert np.array_equal(s1, surf[i]) and np.array_equal(p1, pidx[i])      # batching does not change a bit
 
 
 def test_many_pairs_peaks_only():
