@@ -6,7 +6,7 @@ kernels and the C ABI (include/caf_b200.h); api.py mirrors `caf_rust::caf::*`; i
 """
 from .api import (CafB200, CafB200F32, CafError, CafFFTW, CafPanic, CafRustFFT, CafRustFFTIter,
                   CafRustFFTIterRayon, CafRustFFTRayon, CafRustFFTThreadpool, CafRustFFTThreads,
-                  CafSurface, CafSurfaceRow, Handle, Surface, Xcor, XcorF32, batch_arrays, default_handle,
+                  CafSurface, CafSurfaceRow, DeviceSurface, Handle, Surface, Xcor, XcorF32, batch_arrays, default_handle, detect_dev,
                   peak_pack, peak_resolve, surface_arrays)
 from .io import DeviceSamples, bench_shifts, gen_float_shifts, read_file_c64, read_file_c64_dev, write_file_binary
 from .siblings import GoSibling, PythonSibling, surface_layout

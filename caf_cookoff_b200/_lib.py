@@ -62,6 +62,13 @@ class Peak(C.Structure):
                 ("doppler_idx", C.c_uint64), ("delay_idx", C.c_uint64)]
 
 
+class Detection(C.Structure):
+    """caf_b200_detection: the first four fields are caf_b200_peak's"""
+    _fields_ = [("value", C.c_double), ("freq_hz", C.c_double),
+                ("doppler_idx", C.c_uint64), ("delay_idx", C.c_uint64),
+                ("lag_samples", C.c_double), ("freq_hz_interp", C.c_double)]
+
+
 # every symbol include/caf_b200.h declares: name -> (restype, argtypes)
 _vp, _sz, _u32, _dbl, _int = C.c_void_p, C.c_size_t, C.c_uint32, C.c_double, C.c_int
 _PK = C.POINTER(Peak)
@@ -70,6 +77,7 @@ _surf = [_vp, _vp, _vp, _sz, _vp, _sz, _u32, _vp, _vp, _vp, _vp]
 _peak = [_vp, _vp, _vp, _sz, _vp, _sz, _u32, _vp]
 _shift = [_vp, _vp, _sz, _dbl, _u32, _vp]
 _xcor = [_vp, _vp, _vp, _sz, _vp]
+_detect_dev = [_vp, _vp, _sz, _sz, _sz, _vp, _sz, _u32, _u32, _dbl, _vp, _vp]
 SYMBOLS = {
     "caf_b200_create": (_int, [_int, C.POINTER(_vp)]),
     "caf_b200_create_on_stream": (_int, [_int, _vp, C.POINTER(_vp)]),
@@ -124,6 +132,9 @@ SYMBOLS = {
     "caf_b200_surface_find_peak": (_int, [_vp, _PK]),
     "caf_b200_surface_fetch_rows": (_int, [_vp, _sz, _sz, _vp]),
     "caf_b200_surface_destroy": (_int, [_vp]),
+    "caf_b200_surface_detect": (_int, [_vp, _sz, _u32, _u32, _dbl, C.POINTER(Detection), C.POINTER(_sz)]),
+    "caf_b200_detect_f64_dev": (_int, _detect_dev),
+    "caf_b200_detect_f32_dev": (_int, _detect_dev),
     "caf_b200_peak_resolve_status": (_int, [C.POINTER(C.c_uint64), _sz, _PK]),
     "caf_b200_peak_allgather_async": (_int, [_vp, _vp, _vp, C.c_uint64, _vp]),
     "caf_b200_comm_remote_error": (_int, [_vp, C.POINTER(_int)]),

@@ -261,6 +261,75 @@ class XcorF32(Xcor):
     _variant = _Variant32
 
 
+class DeviceSurface:
+    """A surface kept in device memory (caf_b200_surface_create_*): find_peak and row peaks come back at once, rows
+    cross PCIe only when fetched, and detect() searches the surface where it lies."""
+
+    def __init__(self, needle, haystack, freqs_hz, fs: int, *, variant=_Variant, handle: Optional[Handle] = None):
+        n_ = np.ascontiguousarray(needle, dtype=variant.cdt).ravel()
+        h_ = np.ascontiguousarray(haystack, dtype=variant.cdt).ravel()
+        f_ = np.ascontiguousarray(freqs_hz, dtype=np.float64).ravel()
+        if n_.size != h_.size:
+            raise CafPanic("assertion failed: a.len() == self.n (xcor_rustfft.rs:54-55)")
+        self.handle = handle or default_handle()
+        self.variant = variant
+        self._lib = _lib.load()
+        self._s = C.c_void_p()
+        fn = getattr(self._lib, "caf_b200_surface_create_" + variant.sfx)
+        _check(fn(self.handle.raw, _ptr(n_), _ptr(h_), n_.size, _ptr(f_), f_.size, int(fs), C.byref(self._s)))
+        self.freqs_hz = f_
+        rows, cells = C.c_size_t(), C.c_size_t()
+        _check(self._lib.caf_b200_surface_shape(self._s, C.byref(rows), C.byref(cells)))
+        self.shape = (rows.value, cells.value)
+
+    @property
+    def raw(self):
+        return self._s
+
+    def find_peak(self) -> _lib.Peak:
+        pk = _lib.Peak()
+        _check(self._lib.caf_b200_surface_find_peak(self._s, C.byref(pk)))
+        return pk
+
+    def fetch_rows(self, row0: int = 0, count: Optional[int] = None) -> np.ndarray:
+        count = self.shape[0] - row0 if count is None else count
+        out = np.empty((count, self.shape[1]), dtype=self.variant.rdt)
+        _check(self._lib.caf_b200_surface_fetch_rows(self._s, int(row0), int(count), _ptr(out)))
+        return out
+
+    def detect(self, k_max: int, guard_doppler: int = 1, guard_delay: int = 1,
+               min_ratio: float = 0.0) -> List[_lib.Detection]:
+        """caf_b200_surface_detect: the strongest local maxima, best first (only the `count` valid records).  It runs on
+        self.handle, so like every call on a handle it must not run at the same time as another call on that handle."""
+        out = (_lib.Detection * max(int(k_max), 1))()
+        count = C.c_size_t()
+        _check(self._lib.caf_b200_surface_detect(self._s, int(k_max), int(guard_doppler), int(guard_delay),
+                                                 float(min_ratio), out, C.byref(count)))
+        return list(out)[:count.value]
+
+    def close(self):
+        if getattr(self, "_s", None) is not None and self._s:
+            self._lib.caf_b200_surface_destroy(self._s)
+            self._s = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def detect_dev(surface_ptr: int, p: int, d: int, n: int, freqs_ptr: int, k_max: int, out_ptr: int, counts_ptr: int, *,
+               guard_doppler: int = 1, guard_delay: int = 1, min_ratio: float = 0.0, f32: bool = False,
+               handle: Optional[Handle] = None):
+    """caf_b200_detect_{f64,f32}_dev on device pointers (e.g. torch tensors' data_ptr()): surface [p][d][n], freqs [d],
+    out [p][k_max] caf_b200_detection records (48 bytes each), counts [p] uint64.  Asynchronous on the handle's stream."""
+    h = handle or default_handle()
+    fn = getattr(_lib.load(), "caf_b200_detect_f32_dev" if f32 else "caf_b200_detect_f64_dev")
+    _check(fn(h.raw, C.c_void_p(surface_ptr), int(p), int(d), int(n), C.c_void_p(freqs_ptr), int(k_max),
+              int(guard_doppler), int(guard_delay), float(min_ratio), C.c_void_p(out_ptr), C.c_void_p(counts_ptr)))
+
+
 def peak_pack(pk: _lib.Peak, global_row_offset: int) -> np.ndarray:
     """caf_b200_peak_pack -> 4 uint64 words for the NCCL exchange."""
     words = (C.c_uint64 * 4)()

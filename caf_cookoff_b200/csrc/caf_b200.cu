@@ -24,6 +24,7 @@
 #include "../../include/caf_b200.h"
 #include "caf_kernels.cuh"
 #include "caf_large.cuh"
+#include "caf_detect.cuh"
 #include "overlap_policy.hpp"
 
 namespace {
@@ -141,6 +142,7 @@ struct caf_b200_handle_s {
     void* h_stage = nullptr;    // pinned host mirror of in_block for callers whose three inputs are not one contiguous block
     size_t h_stage_cap = 0;
     DevBuf lwbuf, lhtmp, lhbig, lpart;      // long-row path: chunk scratch, scratch of the H transform, H, partial row maxima
+    DevBuf det, det_io;                     // detection: counters | candidate lists; host calls' grid | records | count
     long long* trace = nullptr;   // CAF_TRACE builds: device buffer for phase stamps
     // Launch-private state of single-pair surface launches, a ring of kRing slots indexed by launch number (epoch % kRing):
     // several such launches can be in flight at once (overlap, below).
@@ -305,6 +307,14 @@ cudaError_t configure_fused() {
     if ((e = cudaFuncSetAttribute(caf::caf_large_spread2<T, RT, kFusedJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return e;
     if ((e = cudaFuncSetAttribute(caf::caf_large_gather2<T, RT, kFusedJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return e;
     return cudaFuncSetAttribute(caf::caf_large_gather2<T, RT, kFusedJ, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+}
+
+// detection tiles: allowed the largest dynamic shared memory run_detect_dev can ask for, once per handle (the attribute
+// belongs to the device, so every handle sets the same value and no handle can lower it under another)
+template <typename T>
+cudaError_t configure_detect() {
+    return cudaFuncSetAttribute(caf::caf_detect_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)caf::det_tile_smem_max<T>());
 }
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point query: no link-time dependency on libcuda
@@ -1100,7 +1110,9 @@ static int create_impl(int device, bool own_stream, void* cuda_stream, caf_b200_
         (e = upload_tables<double>(h->td, h->stream)) != cudaSuccess ||
         (e = upload_tables<float>(h->tf, h->stream)) != cudaSuccess ||
         (e = configure_all<double>(&h->occ_d)) != cudaSuccess ||
-        (e = configure_all<float>(&h->occ_f)) != cudaSuccess) {
+        (e = configure_all<float>(&h->occ_f)) != cudaSuccess ||
+        (e = configure_detect<double>()) != cudaSuccess ||
+        (e = configure_detect<float>()) != cudaSuccess) {
         std::string m = std::string("handle setup failed: ") + cudaGetErrorString(e);
         caf_b200_destroy(h);
         return fail(CAF_B200_ECUDA, m);
@@ -1123,7 +1135,7 @@ int caf_b200_destroy(caf_b200_handle h) {
     h->surf_pool.clear();
     if (h->copy_stream) cudaStreamSynchronize(h->copy_stream);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    for (DevBuf* b : {&h->in_block, &h->needle, &h->hay, &h->hperm, &h->freqs, &h->surface, &h->rowval, &h->rowidx, &h->peaks, &h->scratch, &h->layout, &h->lwbuf, &h->lhtmp, &h->lhbig, &h->lpart})
+    for (DevBuf* b : {&h->in_block, &h->needle, &h->hay, &h->hperm, &h->freqs, &h->surface, &h->rowval, &h->rowidx, &h->peaks, &h->scratch, &h->layout, &h->lwbuf, &h->lhtmp, &h->lhbig, &h->lpart, &h->det, &h->det_io})
         b->release();
     for (void* q : {(void*)h->td.tw1, (void*)h->td.tw2, (void*)h->td.g, (void*)h->tf.tw1, (void*)h->tf.tw2, (void*)h->tf.g})
         if (q) cudaFree(q);
@@ -1465,6 +1477,113 @@ int caf_b200_surface_destroy(caf_b200_surface s) {
     }
     delete s;
     return CAF_B200_OK;
+}
+
+// ---- detection: the K strongest local maxima of stored surfaces (caf_detect.cuh) ------------------------------------
+static_assert(sizeof(caf_b200_detection) == sizeof(caf::DetectOut), "detection layouts must match");
+extern "C++" {
+namespace {
+int check_detect(size_t d, size_t n, size_t k_max, uint32_t gr, uint32_t gd, double min_ratio) {
+    if (k_max < 1 || k_max > (size_t)caf::kDetMaxK) return fail(CAF_B200_EINVAL, "k_max must be 1 ... 1024");
+    if (gr > (uint32_t)caf::kDetMaxGuardDoppler) return fail(CAF_B200_EINVAL, "guard_doppler must be 0 ... 32 rows");
+    if (gd > (uint32_t)caf::kDetMaxGuardDelay) return fail(CAF_B200_EINVAL, "guard_delay must be 0 ... 256 cells");
+    if (d && n && 2 * (size_t)gd + 1 > n) return fail(CAF_B200_EINVAL, "2 * guard_delay + 1 exceeds the cells per row");
+    if (!(min_ratio >= 0.0 && min_ratio <= 1.0)) return fail(CAF_B200_EINVAL, "min_ratio must be in [0, 1]");
+    if (d > (1ull << 31) || n > (1ull << 31)) return fail(CAF_B200_EUNSUPPORTED, "more than 2^31 rows or cells per row");
+    return CAF_B200_OK;
+}
+
+// Both passes on the handle's stream; every pointer is device memory.  Arguments are already checked.
+template <typename T>
+int run_detect_dev(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs, size_t k_max,
+                   uint32_t gr, uint32_t gd, double min_ratio, caf::DetectOut* out, unsigned long long* counts) {
+    using namespace caf;
+    if (p == 0) return CAF_B200_OK;
+    const bool cells = d && n;
+    // tile height: the tallest of 16 / 8 / 4 / 2 / 1 rows whose shared memory leaves room for two CTAs per SM; rows
+    // beyond the surface's own are not worth their halo
+    int tr = 16;
+    while (tr > 1 && (det_tile_smem<T>(tr, (int)gr, (int)gd) > kDetSmemBudget || (size_t)(tr / 2) >= d)) tr /= 2;
+    const size_t smem = det_tile_smem<T>(tr, (int)gr, (int)gd);      // <= det_tile_smem_max<T>(), set at handle creation
+    const long long tiles_c = (long long)((n + kDetCols - 1) / kDetCols), tiles_r = (long long)((d + tr - 1) / tr);
+    const long long tiles = cells ? tiles_c * tiles_r : 0;
+    const long long slots = (long long)std::min(k_max, det_tile_max_maxima(tr, (int)gr, (int)gd));   // entries one tile can append
+    const long long cap = tiles * slots;
+    if ((double)p * (double)tiles > 2147483647.0) return fail(CAF_B200_EUNSUPPORTED, "too many tiles for one launch");
+    const size_t ctr_bytes = (16 * p + 255) & ~(size_t)255;
+    CK(h->det.ensure(ctr_bytes + sizeof(DetEntry) * (size_t)cap * p));
+    unsigned long long* ctr = reinterpret_cast<unsigned long long*>(h->det.p);
+    DetEntry* entries = reinterpret_cast<DetEntry*>((char*)h->det.p + ctr_bytes);
+    CK(cudaMemsetAsync(ctr, 0, 16 * p, h->stream));
+    if (tiles) {
+        caf_detect_tiles_kernel<T><<<(unsigned)(p * tiles), kDetCols, smem, h->stream>>>(
+            surface, (long long)d, (long long)n, (int)gr, (int)gd, tr, tiles_c, tiles, (unsigned)k_max, cap, entries, ctr);
+        h->launches++;
+        CK(cudaGetLastError());
+    }
+    caf_detect_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
+        surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, min_ratio, out, counts);
+    h->launches++;
+    CK(cudaGetLastError());
+    return CAF_B200_OK;
+}
+
+template <typename T>
+int detect_dev_impl(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs, size_t k_max,
+                    uint32_t gr, uint32_t gd, double min_ratio, caf_b200_detection* out, uint64_t* counts) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_detect(d, n, k_max, gr, gd, min_ratio);
+    if (rc) return rc;
+    if (p && (!out || !counts)) return fail(CAF_B200_EINVAL, "null out / counts");
+    if (p && d && n && !surface) return fail(CAF_B200_EINVAL, "null surface");
+    if (p && d && !freqs) return fail(CAF_B200_EINVAL, "null freqs_hz");
+    if ((double)p * (double)d * (double)n > 9.0e18) return fail(CAF_B200_EUNSUPPORTED, "surface too large");
+    CK(cudaSetDevice(h->device));
+    return run_detect_dev<T>(h, surface, p, d, n, freqs, k_max, gr, gd, min_ratio, (caf::DetectOut*)out,
+                             (unsigned long long*)counts);
+}
+}  // namespace
+}  // extern "C++"
+
+int caf_b200_surface_detect(caf_b200_surface s, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                            double min_ratio, caf_b200_detection* out, size_t* count) {
+    if (!s || !out || !count) return fail(CAF_B200_EINVAL, "null argument");
+    int rc = check_detect(s->d, s->n, k_max, guard_doppler, guard_delay, min_ratio);
+    if (rc) return rc;
+    {
+        std::lock_guard<std::mutex> lk(g_live_mu);
+        if (!g_live_handles.count(s->h)) return fail(CAF_B200_EINVAL, "the surface's handle was destroyed");
+    }
+    caf_b200_handle h = s->h;
+    CK(cudaSetDevice(h->device));
+    // device block: grid | records | count
+    const size_t fr_bytes = (sizeof(double) * s->d + 255) & ~(size_t)255, rec_bytes = sizeof(caf_b200_detection) * k_max;
+    CK(h->det_io.ensure(fr_bytes + rec_bytes + 8));
+    double* d_freqs = (double*)h->det_io.p;
+    caf::DetectOut* d_out = (caf::DetectOut*)((char*)h->det_io.p + fr_bytes);
+    unsigned long long* d_count = (unsigned long long*)((char*)d_out + rec_bytes);
+    if (s->d) CK(cudaMemcpyAsync(d_freqs, s->freqs.data(), sizeof(double) * s->d, cudaMemcpyHostToDevice, h->stream));
+    if (s->f32) rc = run_detect_dev<float>(h, (const float*)s->dev, 1, s->d, s->n, d_freqs, k_max, guard_doppler, guard_delay, min_ratio, d_out, d_count);
+    else rc = run_detect_dev<double>(h, (const double*)s->dev, 1, s->d, s->n, d_freqs, k_max, guard_doppler, guard_delay, min_ratio, d_out, d_count);
+    if (rc) return rc;
+    std::vector<caf_b200_detection> rec(k_max);
+    unsigned long long cnt = 0;
+    CK(cudaMemcpyAsync(rec.data(), d_out, rec_bytes, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(&cnt, d_count, 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    std::memcpy(out, rec.data(), rec_bytes);
+    *count = (size_t)cnt;
+    return CAF_B200_OK;
+}
+int caf_b200_detect_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n, const double* freqs_hz,
+                            size_t k_max, uint32_t guard_doppler, uint32_t guard_delay, double min_ratio,
+                            caf_b200_detection* out, uint64_t* counts) {
+    return detect_dev_impl<double>(h, surface, p, d, n, freqs_hz, k_max, guard_doppler, guard_delay, min_ratio, out, counts);
+}
+int caf_b200_detect_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n, const double* freqs_hz,
+                            size_t k_max, uint32_t guard_doppler, uint32_t guard_delay, double min_ratio,
+                            caf_b200_detection* out, uint64_t* counts) {
+    return detect_dev_impl<float>(h, surface, p, d, n, freqs_hz, k_max, guard_doppler, guard_delay, min_ratio, out, counts);
 }
 
 // ---- multi-GPU peak words: [0] = bits(value), [1] = global doppler row (UINT64_MAX if none),

@@ -211,6 +211,46 @@ int caf_b200_surface_find_peak(caf_b200_surface s, caf_b200_peak* out);
 int caf_b200_surface_fetch_rows(caf_b200_surface s, size_t row0, size_t count, void* out);
 int caf_b200_surface_destroy(caf_b200_surface s);
 
+/* ---- detection: the k_max strongest local maxima of a stored surface, refined below the grid -----------------------
+ * Surfaces are the Rust layout above: p pairs x d rows x n cells of |xcor|^2, rows in freqs_hz order, cell k holding lag k
+ * when 2k < n and k - n otherwise.  The window of cell (r, k) is rows r +- guard_doppler (clipped to the surface) times
+ * cells (k + j) mod n for |j| <= guard_delay (the delay axis is circular), without the cell itself.  A cell of value v is a
+ * local maximum when v > 0, no window cell exceeds v, and no window cell equal to v has a smaller flat index r * n + k
+ * (one cell per plateau; NaN cells never qualify and never block).  Local maxima are ordered by value descending, then
+ * flat index ascending; the first k_max are kept, then every one below min_ratio x the first is dropped.  Detection 0 is
+ * therefore find_peak's cell whenever the surface has a positive cell.
+ * Refinement, in double from the stored values: a 3-point parabola through (k - 1, k, k + 1) of the row (cells wrap; no fit
+ * when n < 3) and through rows (r - 1, r, r + 1) at cell k (no fit on the first and last row); each offset is clamped to
+ * +-0.5 and is 0 where the three points do not curve down.  lag_samples = signed lag + delay offset; freq_hz_interp moves
+ * from freqs_hz[r] by the Doppler offset times the grid step on that side (non-uniform grids work).
+ * Slots [count, k_max) hold value 0, freq 0, doppler_idx UINT64_MAX, delay 0, lag 0, freq_interp 0.
+ * Limits: 1 <= k_max <= 1024, guard_doppler <= 32, guard_delay <= 256 with 2 * guard_delay + 1 <= n (n > 0),
+ * 0 <= min_ratio <= 1; anything else, or a null pointer, is CAF_B200_EINVAL and writes nothing.  An empty surface gives a
+ * count of 0.  Scratch comes from the handle's grow-only workspace: per tile of tr <= 16 rows x 256 cells, 16 bytes x
+ * min(k_max, ceil(tr / (guard_doppler + 1)) x ceil(256 / (guard_delay + 1))) -- no tile holds more local maxima than that
+ * (at most 4 bytes per cell with guards of 1 x 1, 16 with none). */
+typedef struct {
+    double value;           /* |xcor|^2 at the cell (the first four fields are caf_b200_peak's) */
+    double freq_hz;         /* freqs_hz[doppler_idx] */
+    uint64_t doppler_idx;   /* row */
+    uint64_t delay_idx;     /* cell */
+    double lag_samples;     /* signed lag of delay_idx + parabolic offset */
+    double freq_hz_interp;  /* freqs_hz interpolated at doppler_idx + parabolic offset */
+} caf_b200_detection;
+/* a surface object (f64 or f32); synchronous, host output (k_max records); needs the surface's handle alive (else EINVAL).
+ * It runs on the surface's handle (its stream, workspace and launch count), so unlike fetch_rows it follows the handle's
+ * threading rule: call it where that handle may be used, never at the same time as another call on it. */
+int caf_b200_surface_detect(caf_b200_surface s, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                            double min_ratio, caf_b200_detection* out, size_t* count);
+/* device surfaces [p][d][n] (e.g. from caf_b200_batch_*_dev); out [p][k_max] and counts [p] in device memory; two plain
+ * stream-ordered launches on the handle's stream (they see every earlier launch complete and count in launch_count) */
+int caf_b200_detect_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
+                            const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                            double min_ratio, caf_b200_detection* out, uint64_t* counts);
+int caf_b200_detect_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n,
+                            const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                            double min_ratio, caf_b200_detection* out, uint64_t* counts);
+
 /* ---- the sibling programs' layouts of the same surface (SURVEY.md section 8(f)4) -------------------
  * The reference's Go and Python programs compute this correlation with the operands swapped and keep the
  * magnitude |xcor| (cmplx.Abs, np.abs) where the Rust crate keeps |xcor|^2 (norm_sqr):

@@ -16,6 +16,7 @@
 #include <memory>
 #include <stdexcept>
 #include <string>
+#include <thread>
 #include <utility>
 #include <vector>
 
@@ -44,11 +45,14 @@ inline caf_b200_handle thread_handle() {
     return holder.h;
 }
 
+using Detection = caf_b200_detection;   // the strongest local maxima of a surface, refined below the grid (caf_b200.h)
+
 // One surface on the GPU, shared by its rows (caf_b200_surface_*).  The reference's CafSurfaceRow owns a Vec<f64> per row
 // (mod.rs:17-22) but keeps every field PRIVATE, so no caller of the crate can read it: here a row is (surface, row number)
 // and the 2L doubles of xcor_mag cross PCIe only when xcor_mag() is called.
 class DeviceSurface {
     caf_b200_surface s_ = nullptr;
+    std::thread::id owner_ = std::this_thread::get_id();   // the thread whose handle made it (thread_handle())
     std::size_t rows_ = 0, cells_ = 0;
     mutable bool have_peaks_ = false;
     mutable std::vector<double> freq_, pval_;
@@ -73,6 +77,17 @@ public:
     std::vector<double> fetch_rows(std::size_t row0, std::size_t count) const {
         std::vector<double> out(count * cells_);
         check(caf_b200_surface_fetch_rows(s_, row0, count, out.data()));
+        return out;
+    }
+    // caf_b200_surface_detect: the count valid detections, best first
+    std::vector<Detection> detect(std::size_t k_max, uint32_t guard_doppler = 1, uint32_t guard_delay = 1,
+                                  double min_ratio = 0.0) const {
+        // detection runs on the surface's handle, which belongs to the creating thread (caf_b200.h threading rule)
+        if (std::this_thread::get_id() != owner_) throw Panic("detect: a surface is searched on the thread that created it");
+        std::vector<Detection> out(k_max);
+        std::size_t count = 0;
+        check(caf_b200_surface_detect(s_, k_max, guard_doppler, guard_delay, min_ratio, out.data(), &count));
+        out.resize(count);
         return out;
     }
 };
@@ -128,6 +143,15 @@ struct CafB200 {
         for (const auto& row : arr)
             if (row.xcor_peak_val() > best) { best = row.xcor_peak_val(); f = row.freq(); idx = row.xcor_peak_idx(); }
         return {f, idx};
+    }
+    // Detection on the surface behind `arr`, which must be what caf_surface returned, untouched (every row of one surface,
+    // in order): a reordered or partial vector no longer names a surface, so it is refused (Panic).
+    static std::vector<Detection> detect(const std::vector<CafSurfaceRow>& arr, std::size_t k_max, uint32_t guard_doppler = 1,
+                                         uint32_t guard_delay = 1, double min_ratio = 0.0) {
+        bool whole = !arr.empty() && arr[0].surface() && arr.size() == arr[0].surface()->rows();
+        for (std::size_t i = 0; i < arr.size() && whole; ++i) whole = arr[i].surface() == arr[0].surface() && arr[i].row() == i;
+        if (!whole) throw Panic("detect needs the untouched rows of one caf_surface call");
+        return arr[0].surface()->detect(k_max, guard_doppler, guard_delay, min_ratio);
     }
     // caf_surface + find_peak fused on the GPU, the surface never leaves the chip
     static std::pair<double, std::size_t> caf_peak(const std::vector<Complex64>& needle, const std::vector<Complex64>& haystack,

@@ -18,8 +18,10 @@ pub struct DeviceSurface {
     rows: usize,
     cells: usize,
     peaks: OnceCell<(Vec<f64>, Vec<f64>, Vec<u64>)>,      // (freq, xcor_peak_val, xcor_peak_idx), 24 bytes per row, on demand
+    owner: std::thread::ThreadId,                          // the thread whose HANDLE made it: detection runs on that handle
 }
-// the object is immutable after creation and caf_b200_surface_fetch_rows / _row_peaks do not touch the handle's stream
+// the object is immutable after creation and caf_b200_surface_fetch_rows / _row_peaks do not touch the handle's stream;
+// caf_b200_surface_detect does, so detect() checks that it runs on the owner thread (a handle is not thread-safe)
 unsafe impl Send for DeviceSurface {}
 unsafe impl Sync for DeviceSurface {}
 impl DeviceSurface {
@@ -29,6 +31,16 @@ impl DeviceSurface {
             ffi::check(unsafe { ffi::caf_b200_surface_row_peaks(self.raw, f.as_mut_ptr(), v.as_mut_ptr(), i.as_mut_ptr()) });
             (f, v, i)
         })
+    }
+    fn detect(&self, k_max: usize, guard_doppler: u32, guard_delay: u32, min_ratio: f64) -> Vec<ffi::caf_b200_detection> {
+        assert!(std::thread::current().id() == self.owner, "detect: a surface is searched on the thread that created it");
+        let mut out = vec![ffi::caf_b200_detection::default(); k_max];
+        let mut count = 0usize;
+        ffi::check(unsafe {
+            ffi::caf_b200_surface_detect(self.raw, k_max, guard_doppler, guard_delay, min_ratio, out.as_mut_ptr(), &mut count)
+        });
+        out.truncate(count);
+        out
     }
     fn fused_peak(&self) -> ffi::caf_b200_peak {
         let mut pk = ffi::caf_b200_peak::default();
@@ -67,7 +79,8 @@ fn surface_on_gpu(needle: &[Complex64], haystack: &[Complex64], freqs_hz: &[f64]
         ffi::caf_b200_surface_create_f64(h.0, needle.as_ptr(), haystack.as_ptr(), needle.len(), freqs_hz.as_ptr(),
                                          freqs_hz.len(), fs, &mut raw)
     }));
-    let surface = Arc::new(DeviceSurface { raw, rows: freqs_hz.len(), cells: 2 * needle.len(), peaks: OnceCell::new() });
+    let surface = Arc::new(DeviceSurface { raw, rows: freqs_hz.len(), cells: 2 * needle.len(), peaks: OnceCell::new(),
+                                           owner: std::thread::current().id() });
     (0..freqs_hz.len()).map(|row| CafSurfaceRow { surface: surface.clone(), row }).collect()
 }
 
@@ -113,6 +126,21 @@ pub trait CafSurface {
 macro_rules! strategy { ($($name:ident),*) => { $(pub struct $name {} impl CafSurface for $name {})* } }
 strategy!(CafB200, CafFFTW, CafRustFFT, CafRustFFTRayon, CafRustFFTIter, CafRustFFTIterRayon, CafRustFFTThreads,
           CafRustFFTThreadpool);
+
+impl CafB200 {
+    /// The `k_max` strongest local maxima of the surface behind `arr`, best first, each refined below the grid
+    /// (include/caf_b200.h, caf_b200_surface_detect).  `arr` must be what `caf_surface` returned, untouched: a reordered or
+    /// partial vector no longer names one surface, so it panics.  It also panics off the thread that called `caf_surface`:
+    /// the search runs on that thread's handle.
+    pub fn detect(arr: &[CafSurfaceRow], k_max: usize, guard_doppler: u32, guard_delay: u32, min_ratio: f64)
+                  -> Vec<ffi::caf_b200_detection> {
+        let first = arr.first().expect("detect needs the untouched rows of one caf_surface call");
+        let whole = arr.len() == first.surface.rows
+            && arr.iter().enumerate().all(|(i, r)| r.row == i && Arc::ptr_eq(&r.surface, &first.surface));
+        assert!(whole, "detect needs the untouched rows of one caf_surface call");
+        first.surface.detect(k_max, guard_doppler, guard_delay, min_ratio)
+    }
+}
 
 /// caf_surface + find_peak fused on the GPU; the surface never leaves the chip.
 pub fn caf_peak(needle: &[Complex64], haystack: &[Complex64], freqs_hz: &[f64], fs: u32) -> (f64, usize) {

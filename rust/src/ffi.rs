@@ -16,6 +16,18 @@ pub struct caf_b200_peak {
     pub delay_idx: u64,
 }
 
+/// caf_b200_detection: a local maximum of a surface, refined below the grid (the first four fields are caf_b200_peak's)
+#[repr(C)]
+#[derive(Clone, Copy, Default, Debug)]
+pub struct caf_b200_detection {
+    pub value: f64,
+    pub freq_hz: f64,
+    pub doppler_idx: u64,
+    pub delay_idx: u64,
+    pub lag_samples: f64,
+    pub freq_hz_interp: f64,
+}
+
 extern "C" {
     pub fn caf_b200_create(device: c_int, out: *mut caf_b200_handle) -> c_int;
     pub fn caf_b200_destroy(h: caf_b200_handle) -> c_int;
@@ -38,6 +50,15 @@ extern "C" {
     pub fn caf_b200_surface_find_peak(s: caf_b200_surface, out: *mut caf_b200_peak) -> c_int;
     pub fn caf_b200_surface_fetch_rows(s: caf_b200_surface, row0: usize, count: usize, out: *mut c_void) -> c_int;
     pub fn caf_b200_surface_destroy(s: caf_b200_surface) -> c_int;
+    // detection: the strongest local maxima of a stored surface (host records), or of device surfaces [p][d][n]
+    pub fn caf_b200_surface_detect(s: caf_b200_surface, k_max: usize, guard_doppler: u32, guard_delay: u32, min_ratio: f64,
+                                   out: *mut caf_b200_detection, count: *mut usize) -> c_int;
+    pub fn caf_b200_detect_f64_dev(h: caf_b200_handle, surface: *const f64, p: usize, d: usize, n: usize,
+                                   freqs_hz: *const f64, k_max: usize, guard_doppler: u32, guard_delay: u32, min_ratio: f64,
+                                   out: *mut caf_b200_detection, counts: *mut u64) -> c_int;
+    pub fn caf_b200_detect_f32_dev(h: caf_b200_handle, surface: *const f32, p: usize, d: usize, n: usize,
+                                   freqs_hz: *const f64, k_max: usize, guard_doppler: u32, guard_delay: u32, min_ratio: f64,
+                                   out: *mut caf_b200_detection, counts: *mut u64) -> c_int;
     // read_file_c64 straight onto the device, and device memory for callers without a CUDA runtime of their own
     pub fn caf_b200_load_c64_dev_f64(h: caf_b200_handle, path: *const c_char, first_sample: usize, max_samples: usize,
                                      dev_out: *mut *mut Complex64, n_out: *mut usize) -> c_int;

@@ -5,6 +5,7 @@
 //
 //   caf_cli NEEDLE.c64 HAYSTACK.c64 [--fmin HZ] [--fmax HZ] [--fstep HZ] [--fs HZ]
 //           [--layout rust|go|python] [--dump FILE] [--device-load]
+//           [--detect K [--guard-doppler R] [--guard-delay C] [--min-db X]]
 //
 // With no options it prints exactly what main.rs prints for the same two files:
 //     Frequency offset: 69.0Hz
@@ -13,7 +14,11 @@
 // sibling program's convention for the dump and for the reported delay (caf.go / caf.py, include/caf_b200.h).
 // --device-load reads both files through pinned memory straight onto the GPU (read_file_c64_dev): the samples never exist
 // as a widened Vec on the host.
+// --detect K prints, after those two lines, one line per detection: the K strongest local maxima of the surface
+// (caf_b200_surface_detect; guards default to 1 row x 1 cell), each refined below the grid, dropping those more than X dB
+// below the first (--min-db X, min_ratio = 10^(-X/10); default: keep all K).
 // Build: g++ -std=c++17 -O2 -Iinclude tools/caf_cli.cpp -Lcaf_cookoff_b200 -lcaf_b200 -Wl,-rpath,$PWD/caf_cookoff_b200
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -23,6 +28,17 @@
 
 #include "caf_b200.hpp"
 
+// a whole number in [lo, hi] or exit 2 (no sign, no trailing characters)
+static std::size_t count_arg(const char* what, const char* v, unsigned long lo, unsigned long hi) {
+    char* end = nullptr;
+    const unsigned long x = std::strtoul(v, &end, 10);
+    if (!(*v >= '0' && *v <= '9') || *end || x < lo || x > hi) {
+        std::fprintf(stderr, "caf_cli: %s needs a whole number in [%lu, %lu], got '%s'\n", what, lo, hi, v);
+        std::exit(2);
+    }
+    return (std::size_t)x;
+}
+
 int main(int argc, char** argv) {
     using namespace caf;
     std::vector<std::string> pos;
@@ -30,6 +46,9 @@ int main(int argc, char** argv) {
     uint32_t fs = 48000;
     std::string layout = "rust", dump;
     bool device_load = false;
+    std::size_t detect_k = 0;
+    uint32_t guard_doppler = 1, guard_delay = 1;
+    double min_db = INFINITY;
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
         auto need = [&](const char* what) -> const char* {
@@ -43,15 +62,30 @@ int main(int argc, char** argv) {
         else if (a == "--layout") layout = need("--layout");
         else if (a == "--dump") dump = need("--dump");
         else if (a == "--device-load") device_load = true;
+        else if (a == "--detect") detect_k = count_arg("--detect", need("--detect"), 1, 1024);
+        else if (a == "--guard-doppler") guard_doppler = (uint32_t)count_arg("--guard-doppler", need("--guard-doppler"), 0, 32);
+        else if (a == "--guard-delay") guard_delay = (uint32_t)count_arg("--guard-delay", need("--guard-delay"), 0, 256);
+        else if (a == "--min-db") {
+            const char* v = need("--min-db");
+            char* end = nullptr;
+            min_db = std::strtod(v, &end);
+            if (end == v || *end || !(min_db >= 0.0)) { std::fprintf(stderr, "caf_cli: --min-db needs a number >= 0, got '%s'\n", v); std::exit(2); }
+        }
         else if (a == "-h" || a == "--help") {
             std::printf("usage: caf_cli NEEDLE.c64 HAYSTACK.c64 [--fmin HZ] [--fmax HZ] [--fstep HZ] [--fs HZ] "
-                        "[--layout rust|go|python] [--dump FILE] [--device-load]\n");
+                        "[--layout rust|go|python] [--dump FILE] [--device-load] "
+                        "[--detect K [--guard-doppler R] [--guard-delay C] [--min-db X]]\n");
             return 0;
         } else if (a.rfind("--", 0) == 0) { std::fprintf(stderr, "caf_cli: unknown option %s\n", a.c_str()); return 2; }
         else pos.push_back(a);
     }
     if (pos.size() != 2) { std::fprintf(stderr, "caf_cli: expected NEEDLE.c64 HAYSTACK.c64 (see --help)\n"); return 2; }
     if (!(fstep > 0.0) || fs == 0) { std::fprintf(stderr, "caf_cli: --fstep and --fs must be positive\n"); return 2; }
+    const bool detecting = detect_k > 0;
+    if (detecting && (device_load || layout != "rust" || !dump.empty())) {
+        std::fprintf(stderr, "caf_cli: --detect goes with the default report (no --layout / --dump / --device-load)\n");
+        return 2;
+    }
     try {
         if (device_load) {
             if (layout != "rust" || !dump.empty()) { std::fprintf(stderr, "caf_cli: --device-load goes with the default report (no --layout / --dump)\n"); return 2; }
@@ -67,7 +101,17 @@ int main(int argc, char** argv) {
         const auto shifts = gen_float_shifts(fmin, fmax, fstep);         // integer milli-Hz range, main.rs:18-22 / test.rs:335-352
         const std::size_t l = needle.size(), d = shifts.size();
         if (layout == "rust") {
-            if (dump.empty()) {
+            if (detecting) {
+                const auto rows = CafB200::caf_surface(needle, haystack, shifts, fs);          // the surface stays on the GPU
+                const auto [freq, idx] = CafB200::find_peak(rows);
+                std::printf("Frequency offset: %.1fHz\nTime offset: %zu samples (%.3fms)\n", freq, idx, (double)idx / ((double)fs / 1e3));
+                const double min_ratio = std::isinf(min_db) ? 0.0 : std::pow(10.0, -min_db / 10.0);
+                const auto dets = CafB200::detect(rows, detect_k, guard_doppler, guard_delay, min_ratio);
+                for (std::size_t i = 0; i < dets.size(); ++i)
+                    std::printf("Detection %zu: %.4fHz (grid %.2fHz), %.3f samples (cell %llu), %.2f dB below the first\n", i,
+                                dets[i].freq_hz_interp, dets[i].freq_hz, dets[i].lag_samples,
+                                (unsigned long long)dets[i].delay_idx, 10.0 * std::log10(dets[0].value / dets[i].value));
+            } else if (dump.empty()) {
                 const auto [freq, idx] = CafB200::caf_peak(needle, haystack, shifts, fs);     // the surface never leaves the GPU
                 std::printf("Frequency offset: %.1fHz\nTime offset: %zu samples (%.3fms)\n", freq, idx, (double)idx / ((double)fs / 1e3));
             } else {
