@@ -69,6 +69,11 @@ class Detection(C.Structure):
                 ("lag_samples", C.c_double), ("freq_hz_interp", C.c_double)]
 
 
+class CfarDetection(C.Structure):
+    """caf_b200_cfar_detection: caf_b200_detection's six fields, then the cell's noise estimate and its training cells"""
+    _fields_ = Detection._fields_ + [("noise", C.c_double), ("train_cells", C.c_uint64)]
+
+
 # every symbol include/caf_b200.h declares: name -> (restype, argtypes)
 _vp, _sz, _u32, _dbl, _int = C.c_void_p, C.c_size_t, C.c_uint32, C.c_double, C.c_int
 _PK = C.POINTER(Peak)
@@ -78,6 +83,8 @@ _peak = [_vp, _vp, _vp, _sz, _vp, _sz, _u32, _vp]
 _shift = [_vp, _vp, _sz, _dbl, _u32, _vp]
 _xcor = [_vp, _vp, _vp, _sz, _vp]
 _detect_dev = [_vp, _vp, _sz, _sz, _sz, _vp, _sz, _u32, _u32, _dbl, _vp, _vp]
+_cfar_dev = [_vp, _vp, _sz, _sz, _sz, _vp, _sz, _u32, _u32, _u32, _u32, _dbl, _vp, _vp]
+_cfar_noise = [_vp, _vp, _sz, _sz, _sz, _u32, _u32, _u32, _u32, _vp]
 SYMBOLS = {
     "caf_b200_create": (_int, [_int, C.POINTER(_vp)]),
     "caf_b200_create_on_stream": (_int, [_int, _vp, C.POINTER(_vp)]),
@@ -135,6 +142,12 @@ SYMBOLS = {
     "caf_b200_surface_detect": (_int, [_vp, _sz, _u32, _u32, _dbl, C.POINTER(Detection), C.POINTER(_sz)]),
     "caf_b200_detect_f64_dev": (_int, _detect_dev),
     "caf_b200_detect_f32_dev": (_int, _detect_dev),
+    "caf_b200_surface_detect_cfar": (_int, [_vp, _sz, _u32, _u32, _u32, _u32, _dbl, C.POINTER(CfarDetection),
+                                            C.POINTER(_sz)]),
+    "caf_b200_detect_cfar_f64_dev": (_int, _cfar_dev),
+    "caf_b200_detect_cfar_f32_dev": (_int, _cfar_dev),
+    "caf_b200_cfar_noise_f64_dev": (_int, _cfar_noise),
+    "caf_b200_cfar_noise_f32_dev": (_int, _cfar_noise),
     "caf_b200_peak_resolve_status": (_int, [C.POINTER(C.c_uint64), _sz, _PK]),
     "caf_b200_peak_allgather_async": (_int, [_vp, _vp, _vp, C.c_uint64, _vp]),
     "caf_b200_comm_remote_error": (_int, [_vp, C.POINTER(_int)]),

@@ -307,6 +307,20 @@ class DeviceSurface:
                                                  float(min_ratio), out, C.byref(count)))
         return list(out)[:count.value]
 
+    def detect_cfar(self, k_max: int, guard_doppler: int = 1, guard_delay: int = 1, train_doppler: int = 2,
+                    train_delay: int = 16, scale: Optional[float] = None) -> List[_lib.CfarDetection]:
+        """caf_b200_surface_detect_cfar: the local maxima that exceed scale x their local noise estimate, best first (only
+        the `count` valid records; possibly none).  scale defaults to cfar_scale(1e-6, cfar_train_cells(...)).  Same
+        handle rule as detect()."""
+        if scale is None:
+            scale = cfar_scale(1e-6, cfar_train_cells(guard_doppler, guard_delay, train_doppler, train_delay))
+        out = (_lib.CfarDetection * max(int(k_max), 1))()
+        count = C.c_size_t()
+        _check(self._lib.caf_b200_surface_detect_cfar(self._s, int(k_max), int(guard_doppler), int(guard_delay),
+                                                      int(train_doppler), int(train_delay), float(scale), out,
+                                                      C.byref(count)))
+        return list(out)[:count.value]
+
     def close(self):
         if getattr(self, "_s", None) is not None and self._s:
             self._lib.caf_b200_surface_destroy(self._s)
@@ -328,6 +342,51 @@ def detect_dev(surface_ptr: int, p: int, d: int, n: int, freqs_ptr: int, k_max: 
     fn = getattr(_lib.load(), "caf_b200_detect_f32_dev" if f32 else "caf_b200_detect_f64_dev")
     _check(fn(h.raw, C.c_void_p(surface_ptr), int(p), int(d), int(n), C.c_void_p(freqs_ptr), int(k_max),
               int(guard_doppler), int(guard_delay), float(min_ratio), C.c_void_p(out_ptr), C.c_void_p(counts_ptr)))
+
+
+def cfar_train_cells(guard_doppler: int, guard_delay: int, train_doppler: int, train_delay: int) -> int:
+    """N = (2R+1)(2C+1) - (2gr+1)(2gd+1), R = gr + tr, C = gd + tc: the training cells of a cell at least R rows from
+    either edge of the surface (rows nearer an edge have fewer) and without NaN neighbours."""
+    R, Cd = guard_doppler + train_doppler, guard_delay + train_delay
+    return (2 * R + 1) * (2 * Cd + 1) - (2 * guard_doppler + 1) * (2 * guard_delay + 1)
+
+
+def cfar_scale(pfa: float, train_cells: int) -> float:
+    """The CA-CFAR threshold factor alpha = N (Pfa^(-1/N) - 1) for N training cells.
+
+    For N i.i.d. exponential training cells (|.|^2 of complex Gaussian noise) and a test cell of the same law,
+    P(v > alpha * mean) = (1 + alpha / N)^-N = Pfa.  That is the false-alarm probability of the threshold test alone,
+    before the local-maximum rule, at a cell with all N training cells; edge rows have fewer, and the correlation a CAF
+    puts between neighbouring cells is not modelled.  Pure host arithmetic."""
+    pfa, n = float(pfa), int(train_cells)
+    if not 0.0 < pfa < 1.0:
+        raise ValueError("pfa must be in (0, 1)")
+    if n < 1:
+        raise ValueError("train_cells must be >= 1")
+    return n * (pfa ** (-1.0 / n) - 1.0)
+
+
+def detect_cfar_dev(surface_ptr: int, p: int, d: int, n: int, freqs_ptr: int, k_max: int, out_ptr: int, counts_ptr: int,
+                    *, scale: float, guard_doppler: int = 1, guard_delay: int = 1, train_doppler: int = 2,
+                    train_delay: int = 16, f32: bool = False, handle: Optional[Handle] = None):
+    """caf_b200_detect_cfar_{f64,f32}_dev on device pointers: surface [p][d][n], freqs [d], out [p][k_max]
+    caf_b200_cfar_detection records (64 bytes each), counts [p] uint64.  Asynchronous on the handle's stream."""
+    h = handle or default_handle()
+    fn = getattr(_lib.load(), "caf_b200_detect_cfar_f32_dev" if f32 else "caf_b200_detect_cfar_f64_dev")
+    _check(fn(h.raw, C.c_void_p(surface_ptr), int(p), int(d), int(n), C.c_void_p(freqs_ptr), int(k_max),
+              int(guard_doppler), int(guard_delay), int(train_doppler), int(train_delay), float(scale),
+              C.c_void_p(out_ptr), C.c_void_p(counts_ptr)))
+
+
+def cfar_noise_dev(surface_ptr: int, p: int, d: int, n: int, noise_ptr: int, *, guard_doppler: int = 1,
+                   guard_delay: int = 1, train_doppler: int = 2, train_delay: int = 16, f32: bool = False,
+                   handle: Optional[Handle] = None):
+    """caf_b200_cfar_noise_{f64,f32}_dev: noise [p][d][n] doubles (NaN where a cell has no training cell), the same bits
+    as the `noise` of detect_cfar's records.  Asynchronous on the handle's stream."""
+    h = handle or default_handle()
+    fn = getattr(_lib.load(), "caf_b200_cfar_noise_f32_dev" if f32 else "caf_b200_cfar_noise_f64_dev")
+    _check(fn(h.raw, C.c_void_p(surface_ptr), int(p), int(d), int(n), int(guard_doppler), int(guard_delay),
+              int(train_doppler), int(train_delay), C.c_void_p(noise_ptr)))
 
 
 def peak_pack(pk: _lib.Peak, global_row_offset: int) -> np.ndarray:

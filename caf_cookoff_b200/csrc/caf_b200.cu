@@ -25,6 +25,7 @@
 #include "caf_kernels.cuh"
 #include "caf_large.cuh"
 #include "caf_detect.cuh"
+#include "caf_cfar.cuh"
 #include "overlap_policy.hpp"
 
 namespace {
@@ -315,6 +316,13 @@ template <typename T>
 cudaError_t configure_detect() {
     return cudaFuncSetAttribute(caf::caf_detect_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)caf::det_tile_smem_max<T>());
+}
+
+// CFAR tiles: the same rule, at the most run_cfar_dev can ask for (a one-row tile staging its training region)
+template <typename T>
+cudaError_t configure_cfar() {
+    return cudaFuncSetAttribute(caf::caf_cfar_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)caf::kCfarSmemMax);
 }
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point query: no link-time dependency on libcuda
@@ -1112,7 +1120,9 @@ static int create_impl(int device, bool own_stream, void* cuda_stream, caf_b200_
         (e = configure_all<double>(&h->occ_d)) != cudaSuccess ||
         (e = configure_all<float>(&h->occ_f)) != cudaSuccess ||
         (e = configure_detect<double>()) != cudaSuccess ||
-        (e = configure_detect<float>()) != cudaSuccess) {
+        (e = configure_detect<float>()) != cudaSuccess ||
+        (e = configure_cfar<double>()) != cudaSuccess ||
+        (e = configure_cfar<float>()) != cudaSuccess) {
         std::string m = std::string("handle setup failed: ") + cudaGetErrorString(e);
         caf_b200_destroy(h);
         return fail(CAF_B200_ECUDA, m);
@@ -1584,6 +1594,167 @@ int caf_b200_detect_f32_dev(caf_b200_handle h, const float* surface, size_t p, s
                             size_t k_max, uint32_t guard_doppler, uint32_t guard_delay, double min_ratio,
                             caf_b200_detection* out, uint64_t* counts) {
     return detect_dev_impl<float>(h, surface, p, d, n, freqs_hz, k_max, guard_doppler, guard_delay, min_ratio, out, counts);
+}
+
+// ---- CFAR detection and the noise map (caf_cfar.cuh) ----------------------------------------------------------------
+static_assert(sizeof(caf_b200_cfar_detection) == sizeof(caf::CfarOut) && sizeof(caf::CfarOut) == 64,
+              "CFAR record layouts must match");
+extern "C++" {
+namespace {
+int check_cfar_window(size_t d, size_t n, uint32_t gr, uint32_t gd, uint32_t tr, uint32_t tc) {
+    if ((uint64_t)gr + tr > (uint64_t)caf::kCfarMaxTrainDoppler) return fail(CAF_B200_EINVAL, "guard_doppler + train_doppler must be <= 32 rows");
+    if ((uint64_t)gd + tc > (uint64_t)caf::kCfarMaxTrainDelay) return fail(CAF_B200_EINVAL, "guard_delay + train_delay must be <= 256 cells");
+    if ((uint64_t)tr + tc < 1) return fail(CAF_B200_EINVAL, "train_doppler + train_delay must be >= 1");
+    if (d && n && 2 * ((size_t)gd + tc) + 1 > n) return fail(CAF_B200_EINVAL, "2 * (guard_delay + train_delay) + 1 exceeds the cells per row");
+    if (d > (1ull << 31) || n > (1ull << 31)) return fail(CAF_B200_EUNSUPPORTED, "more than 2^31 rows or cells per row");
+    return CAF_B200_OK;
+}
+int check_cfar(size_t d, size_t n, size_t k_max, uint32_t gr, uint32_t gd, uint32_t tr, uint32_t tc, double scale) {
+    if (k_max < 1 || k_max > (size_t)caf::kDetMaxK) return fail(CAF_B200_EINVAL, "k_max must be 1 ... 1024");
+    if (!(scale > 0.0 && scale <= 1.7976931348623157e308)) return fail(CAF_B200_EINVAL, "scale must be finite and > 0");
+    return check_cfar_window(d, n, gr, gd, tr, tc);
+}
+
+// Both passes on the handle's stream; every pointer is device memory.  Arguments are already checked.
+template <typename T>
+int run_cfar_dev(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs, size_t k_max,
+                 uint32_t gr, uint32_t gd, uint32_t trd, uint32_t tcd, double scale, caf::CfarOut* out,
+                 unsigned long long* counts) {
+    using namespace caf;
+    if (p == 0) return CAF_B200_OK;
+    const bool cells = d && n;
+    const int R = (int)(gr + trd), C = (int)(gd + tcd);
+    // tile height: the tallest of 16 / 8 / 4 / 2 / 1 rows that stages its training region and leaves room for two CTAs
+    // per SM; else one row staging up to kCfarSmemMax; else (the largest windows) the tallest tile that reads its
+    // training cells from the surface
+    auto smem = [&](int tr, bool staged) {
+        return cfar_tile_layout<T>(tr, (int)gr, (int)gd, R, C, staged, (int)det_tile_max_maxima(tr, (int)gr, (int)gd)).total;
+    };
+    int tr = 16;
+    bool staged = true;
+    while (tr > 1 && (smem(tr, true) > kDetSmemBudget || (size_t)(tr / 2) >= d)) tr /= 2;
+    if (smem(tr, true) > kCfarSmemMax) {
+        staged = false;
+        tr = 16;
+        while (tr > 1 && (smem(tr, false) > kDetSmemBudget || (size_t)(tr / 2) >= d)) tr /= 2;
+    }
+    const size_t bytes = smem(tr, staged);                       // <= kCfarSmemMax, set at handle creation
+    const int mx = (int)det_tile_max_maxima(tr, (int)gr, (int)gd);
+    const long long tiles_c = (long long)((n + kDetCols - 1) / kDetCols), tiles_r = (long long)((d + tr - 1) / tr);
+    const long long tiles = cells ? tiles_c * tiles_r : 0;
+    const long long slots = (long long)std::min(k_max, (size_t)mx);   // entries one tile can append
+    const long long cap = tiles * slots;
+    if ((double)p * (double)tiles > 2147483647.0) return fail(CAF_B200_EUNSUPPORTED, "too many tiles for one launch");
+    const size_t ctr_bytes = (16 * p + 255) & ~(size_t)255;
+    CK(h->det.ensure(ctr_bytes + sizeof(CfarEntry) * (size_t)cap * p));
+    unsigned long long* ctr = reinterpret_cast<unsigned long long*>(h->det.p);
+    CfarEntry* entries = reinterpret_cast<CfarEntry*>((char*)h->det.p + ctr_bytes);
+    CK(cudaMemsetAsync(ctr, 0, 16 * p, h->stream));
+    if (tiles) {
+        caf_cfar_tiles_kernel<T><<<(unsigned)(p * tiles), kDetCols, bytes, h->stream>>>(
+            surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, scale, tiles_c, tiles,
+            (unsigned)k_max, cap, entries, ctr);
+        h->launches++;
+        CK(cudaGetLastError());
+    }
+    caf_cfar_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
+        surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, out, counts);
+    h->launches++;
+    CK(cudaGetLastError());
+    return CAF_B200_OK;
+}
+
+template <typename T>
+int detect_cfar_dev_impl(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs,
+                         size_t k_max, uint32_t gr, uint32_t gd, uint32_t tr, uint32_t tc, double scale,
+                         caf_b200_cfar_detection* out, uint64_t* counts) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_cfar(d, n, k_max, gr, gd, tr, tc, scale);
+    if (rc) return rc;
+    if (!out || !counts) return fail(CAF_B200_EINVAL, "null out / counts");
+    if (!surface) return fail(CAF_B200_EINVAL, "null surface");
+    if (!freqs) return fail(CAF_B200_EINVAL, "null freqs_hz");
+    if ((double)p * (double)d * (double)n > 9.0e18) return fail(CAF_B200_EUNSUPPORTED, "surface too large");
+    CK(cudaSetDevice(h->device));
+    return run_cfar_dev<T>(h, surface, p, d, n, freqs, k_max, gr, gd, tr, tc, scale, (caf::CfarOut*)out,
+                           (unsigned long long*)counts);
+}
+
+template <typename T>
+int cfar_noise_dev_impl(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, uint32_t gr, uint32_t gd,
+                        uint32_t tr, uint32_t tc, double* noise_out) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_cfar_window(d, n, gr, gd, tr, tc);
+    if (rc) return rc;
+    if (!surface || !noise_out) return fail(CAF_B200_EINVAL, "null surface / noise_out");
+    if ((double)p * (double)d * (double)n > 9.0e18) return fail(CAF_B200_EUNSUPPORTED, "surface too large");
+    const long long cells = (long long)(p * d * n);
+    if (cells == 0) return CAF_B200_OK;
+    CK(cudaSetDevice(h->device));
+    const long long blocks = std::min<long long>((cells + 255) / 256, (long long)h->sm_count * 64);
+    caf::caf_cfar_noise_kernel<T><<<(unsigned)blocks, 256, 0, h->stream>>>(
+        surface, (long long)p, (long long)d, (long long)n, (int)gr, (int)gd, (int)(gr + tr), (int)(gd + tc), noise_out);
+    h->launches++;
+    CK(cudaGetLastError());
+    return CAF_B200_OK;
+}
+}  // namespace
+}  // extern "C++"
+
+int caf_b200_surface_detect_cfar(caf_b200_surface s, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                 uint32_t train_doppler, uint32_t train_delay, double scale, caf_b200_cfar_detection* out,
+                                 size_t* count) {
+    if (!s || !out || !count) return fail(CAF_B200_EINVAL, "null argument");
+    int rc = check_cfar(s->d, s->n, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale);
+    if (rc) return rc;
+    {
+        std::lock_guard<std::mutex> lk(g_live_mu);
+        if (!g_live_handles.count(s->h)) return fail(CAF_B200_EINVAL, "the surface's handle was destroyed");
+    }
+    caf_b200_handle h = s->h;
+    CK(cudaSetDevice(h->device));
+    // device block: grid | records | count
+    const size_t fr_bytes = (sizeof(double) * s->d + 255) & ~(size_t)255, rec_bytes = sizeof(caf_b200_cfar_detection) * k_max;
+    CK(h->det_io.ensure(fr_bytes + rec_bytes + 8));
+    double* d_freqs = (double*)h->det_io.p;
+    caf::CfarOut* d_out = (caf::CfarOut*)((char*)h->det_io.p + fr_bytes);
+    unsigned long long* d_count = (unsigned long long*)((char*)d_out + rec_bytes);
+    if (s->d) CK(cudaMemcpyAsync(d_freqs, s->freqs.data(), sizeof(double) * s->d, cudaMemcpyHostToDevice, h->stream));
+    if (s->f32) rc = run_cfar_dev<float>(h, (const float*)s->dev, 1, s->d, s->n, d_freqs, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale, d_out, d_count);
+    else rc = run_cfar_dev<double>(h, (const double*)s->dev, 1, s->d, s->n, d_freqs, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale, d_out, d_count);
+    if (rc) return rc;
+    std::vector<caf_b200_cfar_detection> rec(k_max);
+    unsigned long long cnt = 0;
+    CK(cudaMemcpyAsync(rec.data(), d_out, rec_bytes, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(&cnt, d_count, 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    std::memcpy(out, rec.data(), rec_bytes);
+    *count = (size_t)cnt;
+    return CAF_B200_OK;
+}
+int caf_b200_detect_cfar_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
+                                 const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                 uint32_t train_doppler, uint32_t train_delay, double scale, caf_b200_cfar_detection* out,
+                                 uint64_t* counts) {
+    return detect_cfar_dev_impl<double>(h, surface, p, d, n, freqs_hz, k_max, guard_doppler, guard_delay, train_doppler,
+                                        train_delay, scale, out, counts);
+}
+int caf_b200_detect_cfar_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n,
+                                 const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                 uint32_t train_doppler, uint32_t train_delay, double scale, caf_b200_cfar_detection* out,
+                                 uint64_t* counts) {
+    return detect_cfar_dev_impl<float>(h, surface, p, d, n, freqs_hz, k_max, guard_doppler, guard_delay, train_doppler,
+                                       train_delay, scale, out, counts);
+}
+int caf_b200_cfar_noise_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
+                                uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler, uint32_t train_delay,
+                                double* noise_out) {
+    return cfar_noise_dev_impl<double>(h, surface, p, d, n, guard_doppler, guard_delay, train_doppler, train_delay, noise_out);
+}
+int caf_b200_cfar_noise_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n,
+                                uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler, uint32_t train_delay,
+                                double* noise_out) {
+    return cfar_noise_dev_impl<float>(h, surface, p, d, n, guard_doppler, guard_delay, train_doppler, train_delay, noise_out);
 }
 
 // ---- multi-GPU peak words: [0] = bits(value), [1] = global doppler row (UINT64_MAX if none),

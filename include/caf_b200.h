@@ -251,6 +251,59 @@ int caf_b200_detect_f32_dev(caf_b200_handle h, const float* surface, size_t p, s
                             const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
                             double min_ratio, caf_b200_detection* out, uint64_t* counts);
 
+/* ---- CFAR detection: local maxima that stand above a local noise estimate (cell-averaging CFAR) ---------------------
+ * detect() ranks candidates; this decides whether anything is there.  Surfaces and the window rule are detect's; gr, gd
+ * are guard_doppler, guard_delay (the local-maximum window and the CFAR guard region), tr, tc are train_doppler,
+ * train_delay, and R = gr + tr, C = gd + tc.
+ * Training cells of (r, k): rows r' in [r - R, r + R] clipped to [0, d), each taking cells (k + j) mod n for |j| <= C,
+ * without those with |r' - r| <= gr and |j| <= gd; NaN cells are skipped.  m = how many remain.
+ * noise, in ONE summation order (so the GPU, the dense map and any restatement agree bit for bit): each row r' sums +0.0
+ * plus its training cells in ascending j, in double (f32 values widened first); the cell sums +0.0 plus those row sums in
+ * ascending r'; noise = sum / m, correctly rounded, NaN when m = 0.  Only non-negative additions: no cancellation next to
+ * a strong peak (which a running sum, adding the entering cell and subtracting the leaving one, would suffer).
+ * Cell (r, k) of value v is a detection when it is a local maximum under detect's rule with (gr, gd), m > 0 and
+ * v > scale * noise (correctly rounded product).  Detections are ordered by value descending, then flat index ascending,
+ * and cut to k_max (no min_ratio); each is refined exactly as in detect.  Detection 0 need not be find_peak's cell, and
+ * the list may be empty: a surface that holds nothing above its noise gives count 0.
+ * Limits: 1 <= k_max <= 1024, gr + tr <= 32, gd + tc <= 256, tr + tc >= 1, 2C + 1 <= n (n > 0), scale finite and > 0, no
+ * null pointer; anything else is CAF_B200_EINVAL and writes nothing.  An empty surface gives a count of 0.
+ * Threshold: for N i.i.d. exponential training cells (|.|^2 of complex Gaussian noise) and a test cell of the same law,
+ * P(v > a * mean) = (1 + a / N)^-N, so scale = N (Pfa^(-1/N) - 1) with N = (2R+1)(2C+1) - (2gr+1)(2gd+1) gives false-alarm
+ * probability Pfa for the threshold test alone (before the local-maximum rule; edge rows have fewer training cells; the
+ * correlation between CAF cells is not modelled).  The Python package's cfar_scale / cfar_train_cells compute it.
+ * Scratch: as detect, 32 bytes per candidate slot. */
+typedef struct {
+    double value;           /* the first six fields are caf_b200_detection's, in its order */
+    double freq_hz;
+    uint64_t doppler_idx;   /* UINT64_MAX in unused slots */
+    uint64_t delay_idx;
+    double lag_samples;
+    double freq_hz_interp;
+    double noise;           /* the cell's noise estimate (0 in unused slots) */
+    uint64_t train_cells;   /* m, the training cells averaged (0 in unused slots) */
+} caf_b200_cfar_detection;
+/* a surface object; synchronous, host records; same handle rule as caf_b200_surface_detect */
+int caf_b200_surface_detect_cfar(caf_b200_surface s, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                 uint32_t train_doppler, uint32_t train_delay, double scale, caf_b200_cfar_detection* out,
+                                 size_t* count);
+/* device surfaces [p][d][n]; out [p][k_max] and counts [p] in device memory; two plain stream-ordered launches */
+int caf_b200_detect_cfar_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
+                                 const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                 uint32_t train_doppler, uint32_t train_delay, double scale, caf_b200_cfar_detection* out,
+                                 uint64_t* counts);
+int caf_b200_detect_cfar_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n,
+                                 const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                 uint32_t train_doppler, uint32_t train_delay, double scale, caf_b200_cfar_detection* out,
+                                 uint64_t* counts);
+/* the dense noise map: noise_out [p][d][n] doubles (device), NaN where m = 0, bit for bit the noise of every record above;
+ * one stream-ordered launch (none for an empty surface).  Limits as above without k_max and scale. */
+int caf_b200_cfar_noise_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
+                                uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler, uint32_t train_delay,
+                                double* noise_out);
+int caf_b200_cfar_noise_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n,
+                                uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler, uint32_t train_delay,
+                                double* noise_out);
+
 /* ---- the sibling programs' layouts of the same surface (SURVEY.md section 8(f)4) -------------------
  * The reference's Go and Python programs compute this correlation with the operands swapped and keep the
  * magnitude |xcor| (cmplx.Abs, np.abs) where the Rust crate keeps |xcor|^2 (norm_sqr):

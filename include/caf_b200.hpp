@@ -46,6 +46,7 @@ inline caf_b200_handle thread_handle() {
 }
 
 using Detection = caf_b200_detection;   // the strongest local maxima of a surface, refined below the grid (caf_b200.h)
+using CfarDetection = caf_b200_cfar_detection;   // the same, above a local noise estimate, with that estimate
 
 // One surface on the GPU, shared by its rows (caf_b200_surface_*).  The reference's CafSurfaceRow owns a Vec<f64> per row
 // (mod.rs:17-22) but keeps every field PRIVATE, so no caller of the crate can read it: here a row is (surface, row number)
@@ -87,6 +88,17 @@ public:
         std::vector<Detection> out(k_max);
         std::size_t count = 0;
         check(caf_b200_surface_detect(s_, k_max, guard_doppler, guard_delay, min_ratio, out.data(), &count));
+        out.resize(count);
+        return out;
+    }
+    // caf_b200_surface_detect_cfar: the count valid CFAR detections, best first (possibly none)
+    std::vector<CfarDetection> detect_cfar(std::size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                           uint32_t train_doppler, uint32_t train_delay, double scale) const {
+        if (std::this_thread::get_id() != owner_) throw Panic("detect_cfar: a surface is searched on the thread that created it");
+        std::vector<CfarDetection> out(k_max);
+        std::size_t count = 0;
+        check(caf_b200_surface_detect_cfar(s_, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale,
+                                           out.data(), &count));
         out.resize(count);
         return out;
     }
@@ -152,6 +164,15 @@ struct CafB200 {
         for (std::size_t i = 0; i < arr.size() && whole; ++i) whole = arr[i].surface() == arr[0].surface() && arr[i].row() == i;
         if (!whole) throw Panic("detect needs the untouched rows of one caf_surface call");
         return arr[0].surface()->detect(k_max, guard_doppler, guard_delay, min_ratio);
+    }
+    // CFAR detection on the surface behind `arr` (same rule for `arr` and the calling thread as detect)
+    static std::vector<CfarDetection> detect_cfar(const std::vector<CafSurfaceRow>& arr, std::size_t k_max,
+                                                  uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler,
+                                                  uint32_t train_delay, double scale) {
+        bool whole = !arr.empty() && arr[0].surface() && arr.size() == arr[0].surface()->rows();
+        for (std::size_t i = 0; i < arr.size() && whole; ++i) whole = arr[i].surface() == arr[0].surface() && arr[i].row() == i;
+        if (!whole) throw Panic("detect_cfar needs the untouched rows of one caf_surface call");
+        return arr[0].surface()->detect_cfar(k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale);
     }
     // caf_surface + find_peak fused on the GPU, the surface never leaves the chip
     static std::pair<double, std::size_t> caf_peak(const std::vector<Complex64>& needle, const std::vector<Complex64>& haystack,

@@ -42,6 +42,18 @@ impl DeviceSurface {
         out.truncate(count);
         out
     }
+    fn detect_cfar(&self, k_max: usize, guard_doppler: u32, guard_delay: u32, train_doppler: u32, train_delay: u32,
+                   scale: f64) -> Vec<ffi::caf_b200_cfar_detection> {
+        assert!(std::thread::current().id() == self.owner, "detect_cfar: a surface is searched on the thread that created it");
+        let mut out = vec![ffi::caf_b200_cfar_detection::default(); k_max];
+        let mut count = 0usize;
+        ffi::check(unsafe {
+            ffi::caf_b200_surface_detect_cfar(self.raw, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale,
+                                              out.as_mut_ptr(), &mut count)
+        });
+        out.truncate(count);
+        out
+    }
     fn fused_peak(&self) -> ffi::caf_b200_peak {
         let mut pk = ffi::caf_b200_peak::default();
         ffi::check(unsafe { ffi::caf_b200_surface_find_peak(self.raw, &mut pk) });
@@ -139,6 +151,17 @@ impl CafB200 {
             && arr.iter().enumerate().all(|(i, r)| r.row == i && Arc::ptr_eq(&r.surface, &first.surface));
         assert!(whole, "detect needs the untouched rows of one caf_surface call");
         first.surface.detect(k_max, guard_doppler, guard_delay, min_ratio)
+    }
+    /// The local maxima of the surface behind `arr` that exceed `scale` x their local noise estimate (cell-averaging
+    /// CFAR, include/caf_b200.h, caf_b200_surface_detect_cfar), best first, at most `k_max` and possibly none.  Same rules
+    /// for `arr` and the calling thread as `detect`.
+    pub fn detect_cfar(arr: &[CafSurfaceRow], k_max: usize, guard_doppler: u32, guard_delay: u32, train_doppler: u32,
+                       train_delay: u32, scale: f64) -> Vec<ffi::caf_b200_cfar_detection> {
+        let first = arr.first().expect("detect_cfar needs the untouched rows of one caf_surface call");
+        let whole = arr.len() == first.surface.rows
+            && arr.iter().enumerate().all(|(i, r)| r.row == i && Arc::ptr_eq(&r.surface, &first.surface));
+        assert!(whole, "detect_cfar needs the untouched rows of one caf_surface call");
+        first.surface.detect_cfar(k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale)
     }
 }
 

@@ -28,6 +28,20 @@ pub struct caf_b200_detection {
     pub freq_hz_interp: f64,
 }
 
+/// caf_b200_cfar_detection: caf_b200_detection's six fields, then the cell's local noise estimate and its training cells
+#[repr(C)]
+#[derive(Clone, Copy, Default, Debug)]
+pub struct caf_b200_cfar_detection {
+    pub value: f64,
+    pub freq_hz: f64,
+    pub doppler_idx: u64,
+    pub delay_idx: u64,
+    pub lag_samples: f64,
+    pub freq_hz_interp: f64,
+    pub noise: f64,
+    pub train_cells: u64,
+}
+
 extern "C" {
     pub fn caf_b200_create(device: c_int, out: *mut caf_b200_handle) -> c_int;
     pub fn caf_b200_destroy(h: caf_b200_handle) -> c_int;
@@ -59,6 +73,24 @@ extern "C" {
     pub fn caf_b200_detect_f32_dev(h: caf_b200_handle, surface: *const f32, p: usize, d: usize, n: usize,
                                    freqs_hz: *const f64, k_max: usize, guard_doppler: u32, guard_delay: u32, min_ratio: f64,
                                    out: *mut caf_b200_detection, counts: *mut u64) -> c_int;
+    // CFAR detection: local maxima above scale x their local noise estimate, and the dense noise map
+    pub fn caf_b200_surface_detect_cfar(s: caf_b200_surface, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                        train_doppler: u32, train_delay: u32, scale: f64,
+                                        out: *mut caf_b200_cfar_detection, count: *mut usize) -> c_int;
+    pub fn caf_b200_detect_cfar_f64_dev(h: caf_b200_handle, surface: *const f64, p: usize, d: usize, n: usize,
+                                        freqs_hz: *const f64, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                        train_doppler: u32, train_delay: u32, scale: f64,
+                                        out: *mut caf_b200_cfar_detection, counts: *mut u64) -> c_int;
+    pub fn caf_b200_detect_cfar_f32_dev(h: caf_b200_handle, surface: *const f32, p: usize, d: usize, n: usize,
+                                        freqs_hz: *const f64, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                        train_doppler: u32, train_delay: u32, scale: f64,
+                                        out: *mut caf_b200_cfar_detection, counts: *mut u64) -> c_int;
+    pub fn caf_b200_cfar_noise_f64_dev(h: caf_b200_handle, surface: *const f64, p: usize, d: usize, n: usize,
+                                       guard_doppler: u32, guard_delay: u32, train_doppler: u32, train_delay: u32,
+                                       noise_out: *mut f64) -> c_int;
+    pub fn caf_b200_cfar_noise_f32_dev(h: caf_b200_handle, surface: *const f32, p: usize, d: usize, n: usize,
+                                       guard_doppler: u32, guard_delay: u32, train_doppler: u32, train_delay: u32,
+                                       noise_out: *mut f64) -> c_int;
     // read_file_c64 straight onto the device, and device memory for callers without a CUDA runtime of their own
     pub fn caf_b200_load_c64_dev_f64(h: caf_b200_handle, path: *const c_char, first_sample: usize, max_samples: usize,
                                      dev_out: *mut *mut Complex64, n_out: *mut usize) -> c_int;

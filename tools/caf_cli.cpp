@@ -17,6 +17,9 @@
 // --detect K prints, after those two lines, one line per detection: the K strongest local maxima of the surface
 // (caf_b200_surface_detect; guards default to 1 row x 1 cell), each refined below the grid, dropping those more than X dB
 // below the first (--min-db X, min_ratio = 10^(-X/10); default: keep all K).
+// --cfar-db X (with --detect K, instead of --min-db) keeps only the local maxima more than X dB above their local noise
+// estimate (caf_b200_surface_detect_cfar, scale = 10^(X/10); training region --train-doppler A rows x --train-delay B
+// cells beyond the guards, default 2 x 16), at most K of them and possibly none; each line ends with its SNR.
 // Build: g++ -std=c++17 -O2 -Iinclude tools/caf_cli.cpp -Lcaf_cookoff_b200 -lcaf_b200 -Wl,-rpath,$PWD/caf_cookoff_b200
 #include <cmath>
 #include <cstdio>
@@ -48,7 +51,9 @@ int main(int argc, char** argv) {
     bool device_load = false;
     std::size_t detect_k = 0;
     uint32_t guard_doppler = 1, guard_delay = 1;
-    double min_db = INFINITY;
+    double min_db = INFINITY, cfar_db = NAN;
+    uint32_t train_doppler = 2, train_delay = 16;
+    bool train_given = false;
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
         auto need = [&](const char* what) -> const char* {
@@ -71,17 +76,33 @@ int main(int argc, char** argv) {
             min_db = std::strtod(v, &end);
             if (end == v || *end || !(min_db >= 0.0)) { std::fprintf(stderr, "caf_cli: --min-db needs a number >= 0, got '%s'\n", v); std::exit(2); }
         }
+        else if (a == "--cfar-db") {
+            const char* v = need("--cfar-db");
+            char* end = nullptr;
+            cfar_db = std::strtod(v, &end);
+            if (end == v || *end || !std::isfinite(cfar_db) || !std::isfinite(std::pow(10.0, cfar_db / 10.0)) ||
+                !(std::pow(10.0, cfar_db / 10.0) > 0.0)) {
+                std::fprintf(stderr, "caf_cli: --cfar-db needs a finite number of dB, got '%s'\n", v);
+                std::exit(2);
+            }
+        }
+        else if (a == "--train-doppler") { train_doppler = (uint32_t)count_arg("--train-doppler", need("--train-doppler"), 0, 32); train_given = true; }
+        else if (a == "--train-delay") { train_delay = (uint32_t)count_arg("--train-delay", need("--train-delay"), 0, 256); train_given = true; }
         else if (a == "-h" || a == "--help") {
             std::printf("usage: caf_cli NEEDLE.c64 HAYSTACK.c64 [--fmin HZ] [--fmax HZ] [--fstep HZ] [--fs HZ] "
                         "[--layout rust|go|python] [--dump FILE] [--device-load] "
-                        "[--detect K [--guard-doppler R] [--guard-delay C] [--min-db X]]\n");
+                        "[--detect K [--guard-doppler R] [--guard-delay C] "
+                        "[--min-db X | --cfar-db X [--train-doppler A] [--train-delay B]]]\n");
             return 0;
         } else if (a.rfind("--", 0) == 0) { std::fprintf(stderr, "caf_cli: unknown option %s\n", a.c_str()); return 2; }
         else pos.push_back(a);
     }
     if (pos.size() != 2) { std::fprintf(stderr, "caf_cli: expected NEEDLE.c64 HAYSTACK.c64 (see --help)\n"); return 2; }
     if (!(fstep > 0.0) || fs == 0) { std::fprintf(stderr, "caf_cli: --fstep and --fs must be positive\n"); return 2; }
-    const bool detecting = detect_k > 0;
+    const bool detecting = detect_k > 0, cfar = !std::isnan(cfar_db);
+    if (cfar && !detecting) { std::fprintf(stderr, "caf_cli: --cfar-db needs --detect K\n"); return 2; }
+    if (cfar && !std::isinf(min_db)) { std::fprintf(stderr, "caf_cli: --cfar-db and --min-db exclude each other\n"); return 2; }
+    if (train_given && !cfar) { std::fprintf(stderr, "caf_cli: --train-doppler / --train-delay need --cfar-db\n"); return 2; }
     if (detecting && (device_load || layout != "rust" || !dump.empty())) {
         std::fprintf(stderr, "caf_cli: --detect goes with the default report (no --layout / --dump / --device-load)\n");
         return 2;
@@ -105,6 +126,17 @@ int main(int argc, char** argv) {
                 const auto rows = CafB200::caf_surface(needle, haystack, shifts, fs);          // the surface stays on the GPU
                 const auto [freq, idx] = CafB200::find_peak(rows);
                 std::printf("Frequency offset: %.1fHz\nTime offset: %zu samples (%.3fms)\n", freq, idx, (double)idx / ((double)fs / 1e3));
+                if (cfar) {
+                    const auto dets = CafB200::detect_cfar(rows, detect_k, guard_doppler, guard_delay, train_doppler,
+                                                           train_delay, std::pow(10.0, cfar_db / 10.0));
+                    for (std::size_t i = 0; i < dets.size(); ++i)
+                        std::printf("Detection %zu: %.4fHz (grid %.2fHz), %.3f samples (cell %llu), %.2f dB below the first, "
+                                    "%.2f dB above the noise\n", i, dets[i].freq_hz_interp, dets[i].freq_hz,
+                                    dets[i].lag_samples, (unsigned long long)dets[i].delay_idx,
+                                    10.0 * std::log10(dets[0].value / dets[i].value),
+                                    10.0 * std::log10(dets[i].value / dets[i].noise));
+                    return 0;
+                }
                 const double min_ratio = std::isinf(min_db) ? 0.0 : std::pow(10.0, -min_db / 10.0);
                 const auto dets = CafB200::detect(rows, detect_k, guard_doppler, guard_delay, min_ratio);
                 for (std::size_t i = 0; i < dets.size(); ++i)
