@@ -1503,39 +1503,62 @@ int check_detect(size_t d, size_t n, size_t k_max, uint32_t gr, uint32_t gd, dou
     return CAF_B200_OK;
 }
 
+// Tile height: the tallest of 16 / 8 / 4 / 2 / 1 rows whose shared memory bytes(tr) leaves room for two CTAs per SM;
+// rows beyond the surface's own are not worth their halo
+template <typename Bytes>
+int det_tile_rows(size_t d, Bytes bytes) {
+    int tr = 16;
+    while (tr > 1 && (bytes(tr) > caf::kDetSmemBudget || (size_t)(tr / 2) >= d)) tr /= 2;
+    return tr;
+}
+
+// Both passes of a detector on the handle's stream, for tiles of tr rows with up to mx local maxima each: carves the
+// per-pair counters and candidate lists out of h->det, zeroes the counters, then launches
+// tiles(grid, tiles_c, tiles_per_pair, cap, entries, ctr) when the surface has cells and merge(cap, entries, ctr).
+template <typename Entry, typename Tiles, typename Merge>
+int run_detection(caf_b200_handle h, size_t p, size_t d, size_t n, size_t k_max, int tr, size_t mx, Tiles tiles_launch,
+                  Merge merge_launch) {
+    using namespace caf;
+    const bool cells = d && n;
+    const long long tiles_c = (long long)((n + kDetCols - 1) / kDetCols), tiles_r = (long long)((d + tr - 1) / tr);
+    const long long tiles = cells ? tiles_c * tiles_r : 0;
+    const long long slots = (long long)std::min(k_max, mx);   // entries one tile can append
+    const long long cap = tiles * slots;
+    if ((double)p * (double)tiles > 2147483647.0) return fail(CAF_B200_EUNSUPPORTED, "too many tiles for one launch");
+    const size_t ctr_bytes = (16 * p + 255) & ~(size_t)255;
+    CK(h->det.ensure(ctr_bytes + sizeof(Entry) * (size_t)cap * p));
+    unsigned long long* ctr = reinterpret_cast<unsigned long long*>(h->det.p);
+    Entry* entries = reinterpret_cast<Entry*>((char*)h->det.p + ctr_bytes);
+    CK(cudaMemsetAsync(ctr, 0, 16 * p, h->stream));
+    if (tiles) {
+        tiles_launch((unsigned)(p * tiles), tiles_c, tiles, cap, entries, ctr);
+        h->launches++;
+        CK(cudaGetLastError());
+    }
+    merge_launch(cap, entries, ctr);
+    h->launches++;
+    CK(cudaGetLastError());
+    return CAF_B200_OK;
+}
+
 // Both passes on the handle's stream; every pointer is device memory.  Arguments are already checked.
 template <typename T>
 int run_detect_dev(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs, size_t k_max,
                    uint32_t gr, uint32_t gd, double min_ratio, caf::DetectOut* out, unsigned long long* counts) {
     using namespace caf;
     if (p == 0) return CAF_B200_OK;
-    const bool cells = d && n;
-    // tile height: the tallest of 16 / 8 / 4 / 2 / 1 rows whose shared memory leaves room for two CTAs per SM; rows
-    // beyond the surface's own are not worth their halo
-    int tr = 16;
-    while (tr > 1 && (det_tile_smem<T>(tr, (int)gr, (int)gd) > kDetSmemBudget || (size_t)(tr / 2) >= d)) tr /= 2;
+    const int tr = det_tile_rows(d, [&](int t) { return det_tile_smem<T>(t, (int)gr, (int)gd); });
     const size_t smem = det_tile_smem<T>(tr, (int)gr, (int)gd);      // <= det_tile_smem_max<T>(), set at handle creation
-    const long long tiles_c = (long long)((n + kDetCols - 1) / kDetCols), tiles_r = (long long)((d + tr - 1) / tr);
-    const long long tiles = cells ? tiles_c * tiles_r : 0;
-    const long long slots = (long long)std::min(k_max, det_tile_max_maxima(tr, (int)gr, (int)gd));   // entries one tile can append
-    const long long cap = tiles * slots;
-    if ((double)p * (double)tiles > 2147483647.0) return fail(CAF_B200_EUNSUPPORTED, "too many tiles for one launch");
-    const size_t ctr_bytes = (16 * p + 255) & ~(size_t)255;
-    CK(h->det.ensure(ctr_bytes + sizeof(DetEntry) * (size_t)cap * p));
-    unsigned long long* ctr = reinterpret_cast<unsigned long long*>(h->det.p);
-    DetEntry* entries = reinterpret_cast<DetEntry*>((char*)h->det.p + ctr_bytes);
-    CK(cudaMemsetAsync(ctr, 0, 16 * p, h->stream));
-    if (tiles) {
-        caf_detect_tiles_kernel<T><<<(unsigned)(p * tiles), kDetCols, smem, h->stream>>>(
-            surface, (long long)d, (long long)n, (int)gr, (int)gd, tr, tiles_c, tiles, (unsigned)k_max, cap, entries, ctr);
-        h->launches++;
-        CK(cudaGetLastError());
-    }
-    caf_detect_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
-        surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, min_ratio, out, counts);
-    h->launches++;
-    CK(cudaGetLastError());
-    return CAF_B200_OK;
+    return run_detection<DetEntry>(
+        h, p, d, n, k_max, tr, det_tile_max_maxima(tr, (int)gr, (int)gd),
+        [&](unsigned grid, long long tiles_c, long long tiles, long long cap, DetEntry* entries, unsigned long long* ctr) {
+            caf_detect_tiles_kernel<T><<<grid, kDetCols, smem, h->stream>>>(
+                surface, (long long)d, (long long)n, (int)gr, (int)gd, tr, tiles_c, tiles, (unsigned)k_max, cap, entries, ctr);
+        },
+        [&](long long cap, const DetEntry* entries, const unsigned long long* ctr) {
+            caf_detect_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
+                surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, min_ratio, out, counts);
+        });
 }
 
 template <typename T>
@@ -1552,6 +1575,36 @@ int detect_dev_impl(caf_b200_handle h, const T* surface, size_t p, size_t d, siz
     return run_detect_dev<T>(h, surface, p, d, n, freqs, k_max, gr, gd, min_ratio, (caf::DetectOut*)out,
                              (unsigned long long*)counts);
 }
+
+// A detector on a stored surface whose arguments are checked: uploads its grid, runs run(freqs, records, count) on the
+// handle's stream with device pointers, copies the k_max records (Out on the device, Rec here) and the count back,
+// synchronises.
+template <typename Out, typename Rec, typename Run>
+int surface_detect_io(caf_b200_surface s, size_t k_max, Rec* out, size_t* count, Run run) {
+    {
+        std::lock_guard<std::mutex> lk(g_live_mu);
+        if (!g_live_handles.count(s->h)) return fail(CAF_B200_EINVAL, "the surface's handle was destroyed");
+    }
+    caf_b200_handle h = s->h;
+    CK(cudaSetDevice(h->device));
+    // device block: grid | records | count
+    const size_t fr_bytes = (sizeof(double) * s->d + 255) & ~(size_t)255, rec_bytes = sizeof(Rec) * k_max;
+    CK(h->det_io.ensure(fr_bytes + rec_bytes + 8));
+    double* d_freqs = (double*)h->det_io.p;
+    Out* d_out = (Out*)((char*)h->det_io.p + fr_bytes);
+    unsigned long long* d_count = (unsigned long long*)((char*)d_out + rec_bytes);
+    if (s->d) CK(cudaMemcpyAsync(d_freqs, s->freqs.data(), sizeof(double) * s->d, cudaMemcpyHostToDevice, h->stream));
+    int rc = run(d_freqs, d_out, d_count);
+    if (rc) return rc;
+    std::vector<Rec> rec(k_max);
+    unsigned long long cnt = 0;
+    CK(cudaMemcpyAsync(rec.data(), d_out, rec_bytes, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(&cnt, d_count, 8, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    std::memcpy(out, rec.data(), rec_bytes);
+    *count = (size_t)cnt;
+    return CAF_B200_OK;
+}
 }  // namespace
 }  // extern "C++"
 
@@ -1560,30 +1613,11 @@ int caf_b200_surface_detect(caf_b200_surface s, size_t k_max, uint32_t guard_dop
     if (!s || !out || !count) return fail(CAF_B200_EINVAL, "null argument");
     int rc = check_detect(s->d, s->n, k_max, guard_doppler, guard_delay, min_ratio);
     if (rc) return rc;
-    {
-        std::lock_guard<std::mutex> lk(g_live_mu);
-        if (!g_live_handles.count(s->h)) return fail(CAF_B200_EINVAL, "the surface's handle was destroyed");
-    }
-    caf_b200_handle h = s->h;
-    CK(cudaSetDevice(h->device));
-    // device block: grid | records | count
-    const size_t fr_bytes = (sizeof(double) * s->d + 255) & ~(size_t)255, rec_bytes = sizeof(caf_b200_detection) * k_max;
-    CK(h->det_io.ensure(fr_bytes + rec_bytes + 8));
-    double* d_freqs = (double*)h->det_io.p;
-    caf::DetectOut* d_out = (caf::DetectOut*)((char*)h->det_io.p + fr_bytes);
-    unsigned long long* d_count = (unsigned long long*)((char*)d_out + rec_bytes);
-    if (s->d) CK(cudaMemcpyAsync(d_freqs, s->freqs.data(), sizeof(double) * s->d, cudaMemcpyHostToDevice, h->stream));
-    if (s->f32) rc = run_detect_dev<float>(h, (const float*)s->dev, 1, s->d, s->n, d_freqs, k_max, guard_doppler, guard_delay, min_ratio, d_out, d_count);
-    else rc = run_detect_dev<double>(h, (const double*)s->dev, 1, s->d, s->n, d_freqs, k_max, guard_doppler, guard_delay, min_ratio, d_out, d_count);
-    if (rc) return rc;
-    std::vector<caf_b200_detection> rec(k_max);
-    unsigned long long cnt = 0;
-    CK(cudaMemcpyAsync(rec.data(), d_out, rec_bytes, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(&cnt, d_count, 8, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    std::memcpy(out, rec.data(), rec_bytes);
-    *count = (size_t)cnt;
-    return CAF_B200_OK;
+    return surface_detect_io<caf::DetectOut>(
+        s, k_max, out, count, [&](const double* freqs, caf::DetectOut* d_out, unsigned long long* d_count) {
+            if (s->f32) return run_detect_dev<float>(s->h, (const float*)s->dev, 1, s->d, s->n, freqs, k_max, guard_doppler, guard_delay, min_ratio, d_out, d_count);
+            return run_detect_dev<double>(s->h, (const double*)s->dev, 1, s->d, s->n, freqs, k_max, guard_doppler, guard_delay, min_ratio, d_out, d_count);
+        });
 }
 int caf_b200_detect_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n, const double* freqs_hz,
                             size_t k_max, uint32_t guard_doppler, uint32_t guard_delay, double min_ratio,
@@ -1622,46 +1656,28 @@ int run_cfar_dev(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t
                  unsigned long long* counts) {
     using namespace caf;
     if (p == 0) return CAF_B200_OK;
-    const bool cells = d && n;
     const int R = (int)(gr + trd), C = (int)(gd + tcd);
-    // tile height: the tallest of 16 / 8 / 4 / 2 / 1 rows that stages its training region and leaves room for two CTAs
-    // per SM; else one row staging up to kCfarSmemMax; else (the largest windows) the tallest tile that reads its
-    // training cells from the surface
+    // tile height: the tallest tile that stages its training region; else one row staging up to kCfarSmemMax; else (the
+    // largest windows) the tallest tile that reads its training cells from the surface
     auto smem = [&](int tr, bool staged) {
         return cfar_tile_layout<T>(tr, (int)gr, (int)gd, R, C, staged, (int)det_tile_max_maxima(tr, (int)gr, (int)gd)).total;
     };
-    int tr = 16;
-    bool staged = true;
-    while (tr > 1 && (smem(tr, true) > kDetSmemBudget || (size_t)(tr / 2) >= d)) tr /= 2;
-    if (smem(tr, true) > kCfarSmemMax) {
-        staged = false;
-        tr = 16;
-        while (tr > 1 && (smem(tr, false) > kDetSmemBudget || (size_t)(tr / 2) >= d)) tr /= 2;
-    }
+    int tr = det_tile_rows(d, [&](int t) { return smem(t, true); });
+    const bool staged = smem(tr, true) <= kCfarSmemMax;
+    if (!staged) tr = det_tile_rows(d, [&](int t) { return smem(t, false); });
     const size_t bytes = smem(tr, staged);                       // <= kCfarSmemMax, set at handle creation
     const int mx = (int)det_tile_max_maxima(tr, (int)gr, (int)gd);
-    const long long tiles_c = (long long)((n + kDetCols - 1) / kDetCols), tiles_r = (long long)((d + tr - 1) / tr);
-    const long long tiles = cells ? tiles_c * tiles_r : 0;
-    const long long slots = (long long)std::min(k_max, (size_t)mx);   // entries one tile can append
-    const long long cap = tiles * slots;
-    if ((double)p * (double)tiles > 2147483647.0) return fail(CAF_B200_EUNSUPPORTED, "too many tiles for one launch");
-    const size_t ctr_bytes = (16 * p + 255) & ~(size_t)255;
-    CK(h->det.ensure(ctr_bytes + sizeof(CfarEntry) * (size_t)cap * p));
-    unsigned long long* ctr = reinterpret_cast<unsigned long long*>(h->det.p);
-    CfarEntry* entries = reinterpret_cast<CfarEntry*>((char*)h->det.p + ctr_bytes);
-    CK(cudaMemsetAsync(ctr, 0, 16 * p, h->stream));
-    if (tiles) {
-        caf_cfar_tiles_kernel<T><<<(unsigned)(p * tiles), kDetCols, bytes, h->stream>>>(
-            surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, scale, tiles_c, tiles,
-            (unsigned)k_max, cap, entries, ctr);
-        h->launches++;
-        CK(cudaGetLastError());
-    }
-    caf_cfar_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
-        surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, out, counts);
-    h->launches++;
-    CK(cudaGetLastError());
-    return CAF_B200_OK;
+    return run_detection<CfarEntry>(
+        h, p, d, n, k_max, tr, (size_t)mx,
+        [&](unsigned grid, long long tiles_c, long long tiles, long long cap, CfarEntry* entries, unsigned long long* ctr) {
+            caf_cfar_tiles_kernel<T><<<grid, kDetCols, bytes, h->stream>>>(
+                surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, scale, tiles_c, tiles,
+                (unsigned)k_max, cap, entries, ctr);
+        },
+        [&](long long cap, const CfarEntry* entries, const unsigned long long* ctr) {
+            caf_cfar_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
+                surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, out, counts);
+        });
 }
 
 template <typename T>
@@ -1707,30 +1723,11 @@ int caf_b200_surface_detect_cfar(caf_b200_surface s, size_t k_max, uint32_t guar
     if (!s || !out || !count) return fail(CAF_B200_EINVAL, "null argument");
     int rc = check_cfar(s->d, s->n, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale);
     if (rc) return rc;
-    {
-        std::lock_guard<std::mutex> lk(g_live_mu);
-        if (!g_live_handles.count(s->h)) return fail(CAF_B200_EINVAL, "the surface's handle was destroyed");
-    }
-    caf_b200_handle h = s->h;
-    CK(cudaSetDevice(h->device));
-    // device block: grid | records | count
-    const size_t fr_bytes = (sizeof(double) * s->d + 255) & ~(size_t)255, rec_bytes = sizeof(caf_b200_cfar_detection) * k_max;
-    CK(h->det_io.ensure(fr_bytes + rec_bytes + 8));
-    double* d_freqs = (double*)h->det_io.p;
-    caf::CfarOut* d_out = (caf::CfarOut*)((char*)h->det_io.p + fr_bytes);
-    unsigned long long* d_count = (unsigned long long*)((char*)d_out + rec_bytes);
-    if (s->d) CK(cudaMemcpyAsync(d_freqs, s->freqs.data(), sizeof(double) * s->d, cudaMemcpyHostToDevice, h->stream));
-    if (s->f32) rc = run_cfar_dev<float>(h, (const float*)s->dev, 1, s->d, s->n, d_freqs, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale, d_out, d_count);
-    else rc = run_cfar_dev<double>(h, (const double*)s->dev, 1, s->d, s->n, d_freqs, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale, d_out, d_count);
-    if (rc) return rc;
-    std::vector<caf_b200_cfar_detection> rec(k_max);
-    unsigned long long cnt = 0;
-    CK(cudaMemcpyAsync(rec.data(), d_out, rec_bytes, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemcpyAsync(&cnt, d_count, 8, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    std::memcpy(out, rec.data(), rec_bytes);
-    *count = (size_t)cnt;
-    return CAF_B200_OK;
+    return surface_detect_io<caf::CfarOut>(
+        s, k_max, out, count, [&](const double* freqs, caf::CfarOut* d_out, unsigned long long* d_count) {
+            if (s->f32) return run_cfar_dev<float>(s->h, (const float*)s->dev, 1, s->d, s->n, freqs, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale, d_out, d_count);
+            return run_cfar_dev<double>(s->h, (const double*)s->dev, 1, s->d, s->n, freqs, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale, d_out, d_count);
+        });
 }
 int caf_b200_detect_cfar_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
                                  const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,

@@ -9,15 +9,16 @@
 //   gives the same bits.  (r, k) is a detection when it is a local maximum under detect's rule with (gr, gd), m > 0 and
 //   v > scale * noise (the correctly rounded product).
 //
-// Pass 1 (caf_cfar_tiles_kernel): the tiles, staging and local-maximum rule of caf_detect_tiles_kernel (restated here,
-//   not factored out of it, so that detect's kernel and its code generation stay exactly as they are).  Only the local
-//   maxima that pass the pair's floor then sum their training cells: one warp takes 32 / (2R + 1) candidates, a lane one
-//   training row of one candidate, and the lanes' row sums are added in ascending row by shuffles.  The cells come from a
-//   copy of the tile's training region in shared memory (its row pitch is odd, so the lanes of a warp, on different rows
-//   of one column, hit different banks) or, when the region does not fit even in a one-row tile, from the surface.  The
-//   tile's qualifying cells are cut to its best k_max and raise the pair's floor as in detect; every entry carries its
-//   noise and m, so pass 2 never sums again.
-// Pass 2 (caf_cfar_merge_kernel): detect's merge without min_ratio, writing the 64-byte records.
+// Pass 1 (caf_cfar_tiles_kernel): the tiles, staging and local-maximum rule of caf_detect_tiles_kernel, restated here.
+//   Calling shared inline steps instead changes both tile kernels' code generation, and made this kernel 2.4 % slower
+//   on config-1 f64 surfaces (NVIDIA B200, 1000 W; DESIGN.md section 10).  Only the local maxima that pass the pair's
+//   floor then sum their training cells: one warp takes 32 / (2R + 1) candidates, a lane one training row of one
+//   candidate, and the lanes' row sums are added in ascending row by shuffles.  The cells come from a copy of the tile's
+//   training region in shared memory (its row pitch is odd, so the lanes of a warp, on different rows of one column, hit
+//   different banks) or, when the region does not fit even in a one-row tile, from the surface.  The tile's qualifying
+//   cells are cut to its best k_max and raise the pair's floor as in detect; every entry carries its noise and m, so
+//   pass 2 never sums again.
+// Pass 2 (caf_cfar_merge_kernel): detect's det_merge without min_ratio, writing the 64-byte records.
 // Map (caf_cfar_noise_kernel): one thread per cell, the same row-sum code, reading the surface.
 #pragma once
 #include <cstdint>
@@ -37,16 +38,16 @@ constexpr int kCfarMaxTrainDoppler = 32;      // limits of gr + tr and gd + tc: 
 constexpr int kCfarMaxTrainDelay = 256;
 constexpr size_t kCfarSmemMax = 200 * 1024;   // one-row tiles may stage a region this large (B200: 227 KB per CTA)
 
-// Dynamic shared memory of pass 1, in bytes from the start: detect's buffers (window maxima, output-row values, one staged
-// row per warp), the training region [tr + 2R][pitch] when staged, then per candidate slot (mx of them) its noise, its
-// m, its tile-local index and its place in the qualifying list, and the radix-select histogram.
+// Dynamic shared memory of pass 1, in bytes from the start: detect's staged buffers (det_stage_smem), the training region
+// [tr + 2R][pitch] when staged, then per candidate slot (mx of them) its noise, its m, its tile-local index and its place
+// in the qualifying list, and the radix-select histogram.
 struct CfarTileLayout { size_t region, noise, mcnt, cand, qual, hist, total; int pitch; };
 
 template <typename T>
 __host__ __device__ inline CfarTileLayout cfar_tile_layout(int tr, int gr, int gd, int R, int C, bool staged, int mx) {
     CfarTileLayout L;
     L.pitch = (kDetCols + 2 * C) | 1;
-    size_t o = sizeof(T) * ((size_t)(tr + 2 * gr) * kDetCols + (size_t)tr * kDetCols + (size_t)kDetWarps * (kDetCols + 2 * gd));
+    size_t o = det_stage_smem<T>(tr, gr, gd);
     L.region = o;
     if (staged) o += sizeof(T) * (size_t)(tr + 2 * R) * (size_t)L.pitch;
     o = (o + 7) & ~(size_t)7;
@@ -290,72 +291,11 @@ __global__ void __launch_bounds__(kDetMergeThreads) caf_cfar_merge_kernel(
         const T* __restrict__ surf, long long d, long long n, const double* __restrict__ freqs,
         const CfarEntry* __restrict__ entries, long long cap, const unsigned long long* __restrict__ ctr, unsigned kmax,
         CfarOut* __restrict__ out, unsigned long long* __restrict__ counts) {
-    __shared__ CfarEntry win[kDetMaxK];
-    __shared__ unsigned hist[256];
-    __shared__ DetSelState sel;
-    __shared__ unsigned nwin;
-    const int tid = threadIdx.x;
-    const long long pair = blockIdx.x;
-    const T* S = surf + pair * d * n;
-    const CfarEntry* E = entries + pair * cap;
-    const long long N = (long long)ctr[2 * pair];
-    if (tid == 0) nwin = 0u;
-    auto key = [&](long long i, unsigned long long& h, unsigned long long& l) { h = E[i].vbits; l = ~E[i].flat; };
-    unsigned long long th = 0ull, tl = 0ull;
-    if (N > (long long)kmax) { det_select_kth(key, N, kmax, hist, &sel); th = sel.oh; tl = sel.ol; }
-    __syncthreads();
-    for (long long i = tid; i < N; i += blockDim.x) {
-        unsigned long long h, l;
-        key(i, h, l);
-        if (det_key_ge(h, l, th, tl)) win[atomicAdd(&nwin, 1u)] = E[i];
-    }
-    __syncthreads();
-    const unsigned m = nwin;
-    unsigned P = 1;
-    while (P < m) P <<= 1;
-    for (unsigned i = m + tid; i < P; i += blockDim.x) win[i] = CfarEntry{0ull, ~0ull, 0ull, 0ull};   // sorts last
-    __syncthreads();
-    // bitonic sort, best key first
-    for (unsigned kk = 2; kk <= P; kk <<= 1)
-        for (unsigned j = kk >> 1; j > 0; j >>= 1) {
-            for (unsigned i = tid; i < P; i += blockDim.x) {
-                const unsigned x = i ^ j;
-                if (x > i) {
-                    const CfarEntry a = win[i], b = win[x];
-                    const bool a_first = a.vbits > b.vbits || (a.vbits == b.vbits && a.flat < b.flat);
-                    if (((i & kk) == 0) != a_first) { win[i] = b; win[x] = a; }
-                }
-            }
-            __syncthreads();
-        }
-    CfarOut* O = out + pair * (long long)kmax;
-    for (unsigned i = tid; i < kmax; i += blockDim.x) {
-        CfarOut o;
-        DetectOut& e = o.det;
-        if (i < m) {
-            const unsigned long long flat = win[i].flat;
-            const long long r = (long long)(flat / (unsigned long long)n), k = (long long)(flat % (unsigned long long)n);
-            const T* row = S + r * n;
-            const double v = (double)row[k];
-            double dk = 0.0, df = 0.0;
-            if (n >= 3) dk = det_fit((double)row[k == 0 ? n - 1 : k - 1], v, (double)row[k + 1 == n ? 0 : k + 1]);
-            if (r > 0 && r + 1 < d) df = det_fit((double)row[k - n], v, (double)row[k + n]);
-            const double fr = freqs[r];
-            double fi = fr;
-            if (df > 0.0) fi = __dadd_rn(fr, __dmul_rn(df, __dsub_rn(freqs[r + 1], fr)));
-            else if (df < 0.0) fi = __dadd_rn(fr, __dmul_rn(df, __dsub_rn(fr, freqs[r - 1])));
-            e.value = v; e.freq_hz = fr; e.doppler_idx = (unsigned long long)r; e.delay_idx = (unsigned long long)k;
-            e.lag_samples = __dadd_rn((double)(2 * k < n ? k : k - n), dk);
-            e.freq_hz_interp = fi;
-            o.noise = __longlong_as_double((long long)win[i].noise_bits);
-            o.train_cells = win[i].m;
-        } else {
-            e.value = 0.0; e.freq_hz = 0.0; e.doppler_idx = ~0ull; e.delay_idx = 0ull; e.lag_samples = 0.0; e.freq_hz_interp = 0.0;
-            o.noise = 0.0; o.train_cells = 0ull;
-        }
-        O[i] = o;
-    }
-    if (tid == 0) counts[pair] = m;
+    det_merge<T, false>(surf, d, n, freqs, entries, cap, ctr, kmax, 0.0, out, counts,
+                        [](CfarOut& o, const CfarEntry& w, bool used) {
+                            o.noise = used ? __longlong_as_double((long long)w.noise_bits) : 0.0;
+                            o.train_cells = used ? w.m : 0ull;
+                        });
 }
 
 // ---- the dense noise map ---------------------------------------------------------------------------------------------

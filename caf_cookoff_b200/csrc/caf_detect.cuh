@@ -12,13 +12,17 @@
 //   of the tile plus the halo (wrapped in delay) in shared memory and writes the row's sliding maximum over +-gd cells;
 //   the column maximum of those over +-gr rows is the window maximum.  Only a cell equal to its window maximum runs the
 //   equal-value rule, from shared memory except where a staged row maximum shows an equal cell in an earlier row (then
-//   that row is read from the surface) and for halo or wrapped cells of its own row.  The tile's local maxima are cut to its top k_max by the 128-bit key
-//   (value bits, ~flat index) -- values are >= 0, so the bit pattern of the double orders them -- and appended to the
-//   pair's candidate list.  A tile with k_max or more local maxima also raises the pair's floor to its k_max-th value:
-//   that many entries reach it, so nothing below it can be in the answer, and later tiles drop such entries at once.
+//   that row is read from the surface) and for halo or wrapped cells of its own row.  The tile's local maxima are cut to
+//   its top k_max by the 128-bit key (value bits, ~flat index) -- values are >= 0, so the bit pattern of the double
+//   orders them -- and appended to the pair's candidate list.  A tile with k_max or more local maxima also raises the
+//   pair's floor to its k_max-th value: that many entries reach it, so nothing below it can be in the answer, and later
+//   tiles drop such entries at once.
 // Pass 2 (caf_detect_merge_kernel): one CTA per pair selects the k_max best keys of the candidate list, sorts them,
 //   refines each from its neighbours and writes the records.  Keys are unique (the flat index is), so the answer does not
 //   depend on the order in which tiles appended their lists: it is the same for any grid and on every call.
+//
+// CFAR detection (caf_cfar.cuh) runs the same passes.  Its merge kernel is det_merge with its own entry and record
+// types, and its tile kernel's shared memory starts with the buffers of det_stage_smem.
 #pragma once
 #include <cstdint>
 
@@ -42,12 +46,18 @@ constexpr int kDetMaxK = 1024;
 constexpr int kDetMaxGuardDoppler = 32;
 constexpr int kDetMaxGuardDelay = 256;
 
-// dynamic shared memory of pass 1: window maxima of tr + 2 gr rows, values of the tr output rows, one staged row per warp,
-// the candidate list (tile-local indices) and the radix-select histogram
+// The buffers at the start of both tile kernels' dynamic shared memory, in bytes: window maxima of tr + 2 gr rows, values
+// of the tr output rows, one staged row per warp
+template <typename T>
+__host__ __device__ constexpr size_t det_stage_smem(int tr, int gr, int gd) {
+    return sizeof(T) * ((size_t)(tr + 2 * gr) * kDetCols + (size_t)tr * kDetCols + (size_t)kDetWarps * (kDetCols + 2 * gd));
+}
+
+// dynamic shared memory of pass 1: the staged buffers, the candidate list (tile-local indices) and the radix-select
+// histogram
 template <typename T>
 __host__ __device__ constexpr size_t det_tile_smem(int tr, int gr, int gd) {
-    return sizeof(T) * ((size_t)(tr + 2 * gr) * kDetCols + (size_t)tr * kDetCols + (size_t)kDetWarps * (kDetCols + 2 * gd)) +
-           sizeof(unsigned) * ((size_t)tr * kDetCols + 256);
+    return det_stage_smem<T>(tr, gr, gd) + sizeof(unsigned) * ((size_t)tr * kDetCols + 256);
 }
 
 constexpr size_t kDetSmemBudget = 100 * 1024;     // tiles taller than one row stay under this: two CTAs per SM
@@ -278,19 +288,26 @@ __device__ __forceinline__ double det_fit(double a, double v, double b) {   // p
     return dl < -0.5 ? -0.5 : (dl > 0.5 ? 0.5 : dl);
 }
 
-template <typename T>
-__global__ void __launch_bounds__(kDetMergeThreads) caf_detect_merge_kernel(
+__device__ __forceinline__ DetectOut& det_rec(DetectOut& o) { return o; }
+template <typename Out> __device__ __forceinline__ DetectOut& det_rec(Out& o) { return o.det; }
+
+// The merge of both detectors (this one and caf_cfar_merge_kernel).  Entry starts with (vbits, flat) and Out holds a
+// DetectOut, the whole record or its member det; fill(o, entry, used) writes the rest of the record.  With RATIO the
+// entries below min_ratio x the first are dropped.  Its shared arrays are declared here, in this order, not passed in
+// from the kernels: passing them in changes the merge kernels' generated code.
+template <typename T, bool RATIO, typename Entry, typename Out, typename Fill>
+__device__ __forceinline__ void det_merge(
         const T* __restrict__ surf, long long d, long long n, const double* __restrict__ freqs,
-        const DetEntry* __restrict__ entries, long long cap, const unsigned long long* __restrict__ ctr, unsigned kmax,
-        double min_ratio, DetectOut* __restrict__ out, unsigned long long* __restrict__ counts) {
-    __shared__ DetEntry win[kDetMaxK];
+        const Entry* __restrict__ entries, long long cap, const unsigned long long* __restrict__ ctr, unsigned kmax,
+        double min_ratio, Out* __restrict__ out, unsigned long long* __restrict__ counts, Fill fill) {
+    __shared__ Entry win[kDetMaxK];
     __shared__ unsigned hist[256];
     __shared__ DetSelState sel;
     __shared__ unsigned nwin, nkept;
     const int tid = threadIdx.x;
     const long long pair = blockIdx.x;
     const T* S = surf + pair * d * n;
-    const DetEntry* E = entries + pair * cap;
+    const Entry* E = entries + pair * cap;
     const long long N = (long long)ctr[2 * pair];
     if (tid == 0) { nwin = 0u; nkept = 0u; }
     auto key = [&](long long i, unsigned long long& h, unsigned long long& l) { h = E[i].vbits; l = ~E[i].flat; };
@@ -306,7 +323,7 @@ __global__ void __launch_bounds__(kDetMergeThreads) caf_detect_merge_kernel(
     const unsigned m = nwin;
     unsigned P = 1;
     while (P < m) P <<= 1;
-    for (unsigned i = m + tid; i < P; i += blockDim.x) win[i] = DetEntry{0ull, ~0ull};   // sorts after every candidate
+    for (unsigned i = m + tid; i < P; i += blockDim.x) win[i] = Entry{0ull, ~0ull};   // sorts after every candidate
     __syncthreads();
     // bitonic sort, best key first
     for (unsigned kk = 2; kk <= P; kk <<= 1)
@@ -314,24 +331,28 @@ __global__ void __launch_bounds__(kDetMergeThreads) caf_detect_merge_kernel(
             for (unsigned i = tid; i < P; i += blockDim.x) {
                 const unsigned x = i ^ j;
                 if (x > i) {
-                    const DetEntry a = win[i], b = win[x];
+                    const Entry a = win[i], b = win[x];
                     const bool a_first = a.vbits > b.vbits || (a.vbits == b.vbits && a.flat < b.flat);
                     if (((i & kk) == 0) != a_first) { win[i] = b; win[x] = a; }
                 }
             }
             __syncthreads();
         }
-    const double v0 = m ? __longlong_as_double((long long)win[0].vbits) : 0.0;
-    const double bar = min_ratio * v0;
-    unsigned mine = 0;
-    for (unsigned i = tid; i < m; i += blockDim.x)
-        if (!(__longlong_as_double((long long)win[i].vbits) < bar)) ++mine;
-    if (mine) atomicAdd(&nkept, mine);
-    __syncthreads();
-    const unsigned kept = nkept;        // values descend, so the kept entries are a prefix
-    DetectOut* O = out + pair * (long long)kmax;
+    unsigned kept = m;
+    if (RATIO) {
+        const double v0 = m ? __longlong_as_double((long long)win[0].vbits) : 0.0;
+        const double bar = min_ratio * v0;
+        unsigned mine = 0;
+        for (unsigned i = tid; i < m; i += blockDim.x)
+            if (!(__longlong_as_double((long long)win[i].vbits) < bar)) ++mine;
+        if (mine) atomicAdd(&nkept, mine);
+        __syncthreads();
+        kept = nkept;        // values descend, so the kept entries are a prefix
+    }
+    Out* O = out + pair * (long long)kmax;
     for (unsigned i = tid; i < kmax; i += blockDim.x) {
-        DetectOut o;
+        Out o;
+        DetectOut& e = det_rec(o);
         if (i < kept) {
             const unsigned long long flat = win[i].flat;
             const long long r = (long long)(flat / (unsigned long long)n), k = (long long)(flat % (unsigned long long)n);
@@ -344,15 +365,26 @@ __global__ void __launch_bounds__(kDetMergeThreads) caf_detect_merge_kernel(
             double fi = fr;
             if (df > 0.0) fi = __dadd_rn(fr, __dmul_rn(df, __dsub_rn(freqs[r + 1], fr)));
             else if (df < 0.0) fi = __dadd_rn(fr, __dmul_rn(df, __dsub_rn(fr, freqs[r - 1])));
-            o.value = v; o.freq_hz = fr; o.doppler_idx = (unsigned long long)r; o.delay_idx = (unsigned long long)k;
-            o.lag_samples = __dadd_rn((double)(2 * k < n ? k : k - n), dk);
-            o.freq_hz_interp = fi;
+            e.value = v; e.freq_hz = fr; e.doppler_idx = (unsigned long long)r; e.delay_idx = (unsigned long long)k;
+            e.lag_samples = __dadd_rn((double)(2 * k < n ? k : k - n), dk);
+            e.freq_hz_interp = fi;
+            fill(o, win[i], true);
         } else {
-            o.value = 0.0; o.freq_hz = 0.0; o.doppler_idx = ~0ull; o.delay_idx = 0ull; o.lag_samples = 0.0; o.freq_hz_interp = 0.0;
+            e.value = 0.0; e.freq_hz = 0.0; e.doppler_idx = ~0ull; e.delay_idx = 0ull; e.lag_samples = 0.0; e.freq_hz_interp = 0.0;
+            fill(o, win[i], false);
         }
         O[i] = o;
     }
     if (tid == 0) counts[pair] = kept;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kDetMergeThreads) caf_detect_merge_kernel(
+        const T* __restrict__ surf, long long d, long long n, const double* __restrict__ freqs,
+        const DetEntry* __restrict__ entries, long long cap, const unsigned long long* __restrict__ ctr, unsigned kmax,
+        double min_ratio, DetectOut* __restrict__ out, unsigned long long* __restrict__ counts) {
+    det_merge<T, true>(surf, d, n, freqs, entries, cap, ctr, kmax, min_ratio, out, counts,
+                       [](DetectOut&, const DetEntry&, bool) {});
 }
 
 }  // namespace caf
