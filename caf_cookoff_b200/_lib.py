@@ -85,6 +85,8 @@ _xcor = [_vp, _vp, _vp, _sz, _vp]
 _detect_dev = [_vp, _vp, _sz, _sz, _sz, _vp, _sz, _u32, _u32, _dbl, _vp, _vp]
 _cfar_dev = [_vp, _vp, _sz, _sz, _sz, _vp, _sz, _u32, _u32, _u32, _u32, _dbl, _vp, _vp]
 _cfar_noise = [_vp, _vp, _sz, _sz, _sz, _u32, _u32, _u32, _u32, _vp]
+_cfar_os_dev = [_vp, _vp, _sz, _sz, _sz, _vp, _sz, _u32, _u32, _u32, _u32, _u32, _dbl, _vp, _vp]
+_cfar_os_noise = [_vp, _vp, _sz, _sz, _sz, _u32, _u32, _u32, _u32, _u32, _vp]
 SYMBOLS = {
     "caf_b200_create": (_int, [_int, C.POINTER(_vp)]),
     "caf_b200_create_on_stream": (_int, [_int, _vp, C.POINTER(_vp)]),
@@ -148,6 +150,12 @@ SYMBOLS = {
     "caf_b200_detect_cfar_f32_dev": (_int, _cfar_dev),
     "caf_b200_cfar_noise_f64_dev": (_int, _cfar_noise),
     "caf_b200_cfar_noise_f32_dev": (_int, _cfar_noise),
+    "caf_b200_surface_detect_cfar_os": (_int, [_vp, _sz, _u32, _u32, _u32, _u32, _u32, _dbl, C.POINTER(CfarDetection),
+                                               C.POINTER(_sz)]),
+    "caf_b200_detect_cfar_os_f64_dev": (_int, _cfar_os_dev),
+    "caf_b200_detect_cfar_os_f32_dev": (_int, _cfar_os_dev),
+    "caf_b200_cfar_os_noise_f64_dev": (_int, _cfar_os_noise),
+    "caf_b200_cfar_os_noise_f32_dev": (_int, _cfar_os_noise),
     "caf_b200_peak_resolve_status": (_int, [C.POINTER(C.c_uint64), _sz, _PK]),
     "caf_b200_peak_allgather_async": (_int, [_vp, _vp, _vp, C.c_uint64, _vp]),
     "caf_b200_comm_remote_error": (_int, [_vp, C.POINTER(_int)]),

@@ -321,6 +321,24 @@ class DeviceSurface:
                                                       C.byref(count)))
         return list(out)[:count.value]
 
+    def detect_cfar_os(self, k_max: int, guard_doppler: int = 1, guard_delay: int = 1, train_doppler: int = 2,
+                       train_delay: int = 16, rank: Optional[int] = None,
+                       scale: Optional[float] = None) -> List[_lib.CfarDetection]:
+        """caf_b200_surface_detect_cfar_os: as detect_cfar, against the rank-th smallest training cell (scaled to the
+        cell's training cells) instead of their mean.  rank defaults to ceil(3N / 4) and scale to
+        cfar_os_scale(1e-6, N, rank), N = cfar_train_cells(...).  Same handle rule as detect()."""
+        N = cfar_train_cells(guard_doppler, guard_delay, train_doppler, train_delay)
+        if rank is None:
+            rank = (3 * N + 3) // 4
+        if scale is None:
+            scale = cfar_os_scale(1e-6, N, rank)
+        out = (_lib.CfarDetection * max(int(k_max), 1))()
+        count = C.c_size_t()
+        _check(self._lib.caf_b200_surface_detect_cfar_os(self._s, int(k_max), int(guard_doppler), int(guard_delay),
+                                                         int(train_doppler), int(train_delay), int(rank), float(scale),
+                                                         out, C.byref(count)))
+        return list(out)[:count.value]
+
     def close(self):
         if getattr(self, "_s", None) is not None and self._s:
             self._lib.caf_b200_surface_destroy(self._s)
@@ -387,6 +405,61 @@ def cfar_noise_dev(surface_ptr: int, p: int, d: int, n: int, noise_ptr: int, *, 
     fn = getattr(_lib.load(), "caf_b200_cfar_noise_f32_dev" if f32 else "caf_b200_cfar_noise_f64_dev")
     _check(fn(h.raw, C.c_void_p(surface_ptr), int(p), int(d), int(n), int(guard_doppler), int(guard_delay),
               int(train_doppler), int(train_delay), C.c_void_p(noise_ptr)))
+
+
+def cfar_os_scale(pfa: float, train_cells: int, rank: int) -> float:
+    """The OS-CFAR threshold factor alpha for the rank-th smallest of N training cells.
+
+    For N i.i.d. exponential training cells and a test cell of the same law, P(v > alpha * X_(k)) =
+    prod_{i=0}^{k-1} (N - i) / (N - i + alpha).  That decreases in alpha; it is solved here by bisection on the log of both
+    sides.  rank = 1 gives N (1 / Pfa - 1).  The caveats of cfar_scale apply, and more so: order statistics of the
+    correlated cells of a CAF stray further from the model, so a CAF surface of noise gives more crossings than Pfa.
+    Pure host arithmetic."""
+    pfa, n, k = float(pfa), int(train_cells), int(rank)
+    if not 0.0 < pfa < 1.0:
+        raise ValueError("pfa must be in (0, 1)")
+    if n < 1:
+        raise ValueError("train_cells must be >= 1")
+    if not 1 <= k <= n:
+        raise ValueError("rank must be in [1, train_cells]")
+    den = n - np.arange(k, dtype=np.float64)
+    target = -np.log(pfa)
+
+    def log_inv_p(alpha):                      # -log P(v > alpha X_(k)), increasing in alpha
+        return float(np.sum(np.log1p(alpha / den)))
+
+    lo, hi = 0.0, n / pfa                      # log_inv_p(hi) >= log1p(1 / pfa) > target
+    while True:
+        mid = 0.5 * (lo + hi)
+        if mid <= lo or mid >= hi:
+            return hi
+        if log_inv_p(mid) < target:
+            lo = mid
+        else:
+            hi = mid
+
+
+def detect_cfar_os_dev(surface_ptr: int, p: int, d: int, n: int, freqs_ptr: int, k_max: int, out_ptr: int,
+                       counts_ptr: int, *, rank: int, scale: float, guard_doppler: int = 1, guard_delay: int = 1,
+                       train_doppler: int = 2, train_delay: int = 16, f32: bool = False, handle: Optional[Handle] = None):
+    """caf_b200_detect_cfar_os_{f64,f32}_dev on device pointers: surface [p][d][n], freqs [d], out [p][k_max]
+    caf_b200_cfar_detection records (64 bytes each), counts [p] uint64.  Asynchronous on the handle's stream."""
+    h = handle or default_handle()
+    fn = getattr(_lib.load(), "caf_b200_detect_cfar_os_f32_dev" if f32 else "caf_b200_detect_cfar_os_f64_dev")
+    _check(fn(h.raw, C.c_void_p(surface_ptr), int(p), int(d), int(n), C.c_void_p(freqs_ptr), int(k_max),
+              int(guard_doppler), int(guard_delay), int(train_doppler), int(train_delay), int(rank), float(scale),
+              C.c_void_p(out_ptr), C.c_void_p(counts_ptr)))
+
+
+def cfar_os_noise_dev(surface_ptr: int, p: int, d: int, n: int, noise_ptr: int, *, rank: int, guard_doppler: int = 1,
+                      guard_delay: int = 1, train_doppler: int = 2, train_delay: int = 16, f32: bool = False,
+                      handle: Optional[Handle] = None):
+    """caf_b200_cfar_os_noise_{f64,f32}_dev: noise [p][d][n] doubles (NaN where a cell has no training cell), the same
+    bits as the `noise` of detect_cfar_os's records.  Asynchronous on the handle's stream."""
+    h = handle or default_handle()
+    fn = getattr(_lib.load(), "caf_b200_cfar_os_noise_f32_dev" if f32 else "caf_b200_cfar_os_noise_f64_dev")
+    _check(fn(h.raw, C.c_void_p(surface_ptr), int(p), int(d), int(n), int(guard_doppler), int(guard_delay),
+              int(train_doppler), int(train_delay), int(rank), C.c_void_p(noise_ptr)))
 
 
 def peak_pack(pk: _lib.Peak, global_row_offset: int) -> np.ndarray:

@@ -26,6 +26,7 @@
 #include "caf_large.cuh"
 #include "caf_detect.cuh"
 #include "caf_cfar.cuh"
+#include "caf_cfar_os.cuh"
 #include "overlap_policy.hpp"
 
 namespace {
@@ -322,6 +323,13 @@ cudaError_t configure_detect() {
 template <typename T>
 cudaError_t configure_cfar() {
     return cudaFuncSetAttribute(caf::caf_cfar_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)caf::kCfarSmemMax);
+}
+
+// OS-CFAR tiles: the same, at the most run_cfar_os_dev can ask for
+template <typename T>
+cudaError_t configure_cfar_os() {
+    return cudaFuncSetAttribute(caf::caf_cfar_os_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)caf::kCfarSmemMax);
 }
 
@@ -1122,7 +1130,9 @@ static int create_impl(int device, bool own_stream, void* cuda_stream, caf_b200_
         (e = configure_detect<double>()) != cudaSuccess ||
         (e = configure_detect<float>()) != cudaSuccess ||
         (e = configure_cfar<double>()) != cudaSuccess ||
-        (e = configure_cfar<float>()) != cudaSuccess) {
+        (e = configure_cfar<float>()) != cudaSuccess ||
+        (e = configure_cfar_os<double>()) != cudaSuccess ||
+        (e = configure_cfar_os<float>()) != cudaSuccess) {
         std::string m = std::string("handle setup failed: ") + cudaGetErrorString(e);
         caf_b200_destroy(h);
         return fail(CAF_B200_ECUDA, m);
@@ -1752,6 +1762,137 @@ int caf_b200_cfar_noise_f32_dev(caf_b200_handle h, const float* surface, size_t 
                                 uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler, uint32_t train_delay,
                                 double* noise_out) {
     return cfar_noise_dev_impl<float>(h, surface, p, d, n, guard_doppler, guard_delay, train_doppler, train_delay, noise_out);
+}
+
+// ---- OS-CFAR detection and its noise map (caf_cfar_os.cuh) ---------------------------------------------------------
+extern "C++" {
+namespace {
+uint64_t cfar_train_cells(uint32_t gr, uint32_t gd, uint32_t tr, uint32_t tc) {
+    const uint64_t R = (uint64_t)gr + tr, C = (uint64_t)gd + tc;
+    return (2 * R + 1) * (2 * C + 1) - (2 * (uint64_t)gr + 1) * (2 * (uint64_t)gd + 1);
+}
+// CA's window limits, then 1 <= rank <= N
+int check_cfar_os_window(size_t d, size_t n, uint32_t gr, uint32_t gd, uint32_t tr, uint32_t tc, uint32_t rank) {
+    int rc = check_cfar_window(d, n, gr, gd, tr, tc);
+    if (rc) return rc;
+    if (rank < 1 || (uint64_t)rank > cfar_train_cells(gr, gd, tr, tc))
+        return fail(CAF_B200_EINVAL, "rank must be 1 ... the training cells N = (2R+1)(2C+1) - (2gr+1)(2gd+1)");
+    return CAF_B200_OK;
+}
+int check_cfar_os(size_t d, size_t n, size_t k_max, uint32_t gr, uint32_t gd, uint32_t tr, uint32_t tc, uint32_t rank,
+                  double scale) {
+    int rc = check_cfar(d, n, k_max, gr, gd, tr, tc, scale);
+    if (rc) return rc;
+    return check_cfar_os_window(d, n, gr, gd, tr, tc, rank);
+}
+
+// Both passes on the handle's stream; every pointer is device memory.  Arguments are already checked.  Tile height as in
+// run_cfar_dev, with the OS layout.
+template <typename T>
+int run_cfar_os_dev(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs, size_t k_max,
+                    uint32_t gr, uint32_t gd, uint32_t trd, uint32_t tcd, uint32_t rank, double scale, caf::CfarOut* out,
+                    unsigned long long* counts) {
+    using namespace caf;
+    if (p == 0) return CAF_B200_OK;
+    const int R = (int)(gr + trd), C = (int)(gd + tcd);
+    auto smem = [&](int tr, bool staged) {
+        return cfar_os_tile_layout<T>(tr, (int)gr, (int)gd, R, C, staged, (int)det_tile_max_maxima(tr, (int)gr, (int)gd)).total;
+    };
+    int tr = det_tile_rows(d, [&](int t) { return smem(t, true); });
+    const bool staged = smem(tr, true) <= kCfarSmemMax;
+    if (!staged) tr = det_tile_rows(d, [&](int t) { return smem(t, false); });
+    const size_t bytes = smem(tr, staged);                       // <= kCfarSmemMax, set at handle creation
+    const int mx = (int)det_tile_max_maxima(tr, (int)gr, (int)gd);
+    const unsigned long long ntrain = cfar_train_cells(gr, gd, trd, tcd);
+    return run_detection<CfarEntry>(
+        h, p, d, n, k_max, tr, (size_t)mx,
+        [&](unsigned grid, long long tiles_c, long long tiles, long long cap, CfarEntry* entries, unsigned long long* ctr) {
+            caf_cfar_os_tiles_kernel<T><<<grid, kDetCols, bytes, h->stream>>>(
+                surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, rank, ntrain, scale, tiles_c,
+                tiles, (unsigned)k_max, cap, entries, ctr);
+        },
+        [&](long long cap, const CfarEntry* entries, const unsigned long long* ctr) {
+            caf_cfar_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
+                surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, out, counts);
+        });
+}
+
+template <typename T>
+int detect_cfar_os_dev_impl(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs,
+                            size_t k_max, uint32_t gr, uint32_t gd, uint32_t tr, uint32_t tc, uint32_t rank, double scale,
+                            caf_b200_cfar_detection* out, uint64_t* counts) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_cfar_os(d, n, k_max, gr, gd, tr, tc, rank, scale);
+    if (rc) return rc;
+    if (!out || !counts) return fail(CAF_B200_EINVAL, "null out / counts");
+    if (!surface) return fail(CAF_B200_EINVAL, "null surface");
+    if (!freqs) return fail(CAF_B200_EINVAL, "null freqs_hz");
+    if ((double)p * (double)d * (double)n > 9.0e18) return fail(CAF_B200_EUNSUPPORTED, "surface too large");
+    CK(cudaSetDevice(h->device));
+    return run_cfar_os_dev<T>(h, surface, p, d, n, freqs, k_max, gr, gd, tr, tc, rank, scale, (caf::CfarOut*)out,
+                              (unsigned long long*)counts);
+}
+
+template <typename T>
+int cfar_os_noise_dev_impl(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, uint32_t gr, uint32_t gd,
+                           uint32_t tr, uint32_t tc, uint32_t rank, double* noise_out) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_cfar_os_window(d, n, gr, gd, tr, tc, rank);
+    if (rc) return rc;
+    if (!surface || !noise_out) return fail(CAF_B200_EINVAL, "null surface / noise_out");
+    if ((double)p * (double)d * (double)n > 9.0e18) return fail(CAF_B200_EUNSUPPORTED, "surface too large");
+    const long long cells = (long long)(p * d * n);
+    if (cells == 0) return CAF_B200_OK;
+    CK(cudaSetDevice(h->device));
+    constexpr int wpb = caf::kCfarOsMapThreads / 32;                // one warp per cell
+    const long long blocks = std::min<long long>((cells + wpb - 1) / wpb, (long long)h->sm_count * 64);
+    caf::caf_cfar_os_noise_kernel<T><<<(unsigned)blocks, caf::kCfarOsMapThreads, 0, h->stream>>>(
+        surface, (long long)p, (long long)d, (long long)n, (int)gr, (int)gd, (int)(gr + tr), (int)(gd + tc), rank,
+        cfar_train_cells(gr, gd, tr, tc), noise_out);
+    h->launches++;
+    CK(cudaGetLastError());
+    return CAF_B200_OK;
+}
+}  // namespace
+}  // extern "C++"
+
+int caf_b200_surface_detect_cfar_os(caf_b200_surface s, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                    uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                    caf_b200_cfar_detection* out, size_t* count) {
+    if (!s || !out || !count) return fail(CAF_B200_EINVAL, "null argument");
+    int rc = check_cfar_os(s->d, s->n, k_max, guard_doppler, guard_delay, train_doppler, train_delay, rank, scale);
+    if (rc) return rc;
+    return surface_detect_io<caf::CfarOut>(
+        s, k_max, out, count, [&](const double* freqs, caf::CfarOut* d_out, unsigned long long* d_count) {
+            if (s->f32) return run_cfar_os_dev<float>(s->h, (const float*)s->dev, 1, s->d, s->n, freqs, k_max, guard_doppler, guard_delay, train_doppler, train_delay, rank, scale, d_out, d_count);
+            return run_cfar_os_dev<double>(s->h, (const double*)s->dev, 1, s->d, s->n, freqs, k_max, guard_doppler, guard_delay, train_doppler, train_delay, rank, scale, d_out, d_count);
+        });
+}
+int caf_b200_detect_cfar_os_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
+                                    const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                    uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                    caf_b200_cfar_detection* out, uint64_t* counts) {
+    return detect_cfar_os_dev_impl<double>(h, surface, p, d, n, freqs_hz, k_max, guard_doppler, guard_delay, train_doppler,
+                                           train_delay, rank, scale, out, counts);
+}
+int caf_b200_detect_cfar_os_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n,
+                                    const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                    uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                    caf_b200_cfar_detection* out, uint64_t* counts) {
+    return detect_cfar_os_dev_impl<float>(h, surface, p, d, n, freqs_hz, k_max, guard_doppler, guard_delay, train_doppler,
+                                          train_delay, rank, scale, out, counts);
+}
+int caf_b200_cfar_os_noise_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
+                                   uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler,
+                                   uint32_t train_delay, uint32_t rank, double* noise_out) {
+    return cfar_os_noise_dev_impl<double>(h, surface, p, d, n, guard_doppler, guard_delay, train_doppler, train_delay, rank,
+                                          noise_out);
+}
+int caf_b200_cfar_os_noise_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n,
+                                   uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler,
+                                   uint32_t train_delay, uint32_t rank, double* noise_out) {
+    return cfar_os_noise_dev_impl<float>(h, surface, p, d, n, guard_doppler, guard_delay, train_doppler, train_delay, rank,
+                                         noise_out);
 }
 
 // ---- multi-GPU peak words: [0] = bits(value), [1] = global doppler row (UINT64_MAX if none),

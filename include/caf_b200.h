@@ -304,6 +304,42 @@ int caf_b200_cfar_noise_f32_dev(caf_b200_handle h, const float* surface, size_t 
                                 uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler, uint32_t train_delay,
                                 double* noise_out);
 
+/* ---- OS-CFAR detection: the same, against an order statistic of the training cells (ordered-statistic CFAR) ---------
+ * CA-CFAR's mean moves with every strong cell in the training region: an emitter's own Doppler main lobe raises its
+ * threshold, and a weak emitter inside a strong one's region is masked.  Here the noise estimate is the rank-th smallest of
+ * N training cells instead, which a few strong cells do not move.  Surfaces, windows, training cells, m, N, the detection
+ * rule, records and refinement are CA-CFAR's above; only noise differs:
+ * each training value is widened to double and +0.0 is added (-0.0 counts as +0.0); with k_m = ceil(rank * m / N) in
+ * 64-bit integers, noise is the k_m-th smallest of those m values, NaN when m = 0.  It is one of the values, not a rounded
+ * sum, so every path (records, the dense map, any restatement) agrees bit for bit.  A record's train_cells is m.
+ * Limits: CA-CFAR's, plus 1 <= rank <= N; anything else is CAF_B200_EINVAL and writes nothing.
+ * Threshold: for N i.i.d. exponential cells and a test cell of the same law, P(v > a * X_(k)) = prod_{i<k} (N-i)/(N-i+a);
+ * the Python package's cfar_os_scale solves it for a.  The caveats of cfar_scale apply (the threshold test alone, edge rows
+ * with fewer cells, correlated CAF cells), and order statistics of correlated cells stray further from the model: expect
+ * more crossings on noise than the nominal Pfa.
+ * Scratch: as CA-CFAR. */
+/* a surface object; synchronous, host records; same handle rule as caf_b200_surface_detect */
+int caf_b200_surface_detect_cfar_os(caf_b200_surface s, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                    uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                    caf_b200_cfar_detection* out, size_t* count);
+/* device surfaces [p][d][n]; out [p][k_max] and counts [p] in device memory; two plain stream-ordered launches */
+int caf_b200_detect_cfar_os_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
+                                    const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                    uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                    caf_b200_cfar_detection* out, uint64_t* counts);
+int caf_b200_detect_cfar_os_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n,
+                                    const double* freqs_hz, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                    uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                    caf_b200_cfar_detection* out, uint64_t* counts);
+/* the dense map: noise_out [p][d][n] doubles (device), NaN where m = 0, bit for bit the noise of every record above; one
+ * stream-ordered launch (none for an empty surface).  Limits as above without k_max and scale. */
+int caf_b200_cfar_os_noise_f64_dev(caf_b200_handle h, const double* surface, size_t p, size_t d, size_t n,
+                                   uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler,
+                                   uint32_t train_delay, uint32_t rank, double* noise_out);
+int caf_b200_cfar_os_noise_f32_dev(caf_b200_handle h, const float* surface, size_t p, size_t d, size_t n,
+                                   uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler,
+                                   uint32_t train_delay, uint32_t rank, double* noise_out);
+
 /* ---- the sibling programs' layouts of the same surface (SURVEY.md section 8(f)4) -------------------
  * The reference's Go and Python programs compute this correlation with the operands swapped and keep the
  * magnitude |xcor| (cmplx.Abs, np.abs) where the Rust crate keeps |xcor|^2 (norm_sqr):

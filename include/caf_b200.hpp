@@ -102,6 +102,18 @@ public:
         out.resize(count);
         return out;
     }
+    // caf_b200_surface_detect_cfar_os: the same against the rank-th smallest training cell (OS-CFAR)
+    std::vector<CfarDetection> detect_cfar_os(std::size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                              uint32_t train_doppler, uint32_t train_delay, uint32_t rank,
+                                              double scale) const {
+        if (std::this_thread::get_id() != owner_) throw Panic("detect_cfar_os: a surface is searched on the thread that created it");
+        std::vector<CfarDetection> out(k_max);
+        std::size_t count = 0;
+        check(caf_b200_surface_detect_cfar_os(s_, k_max, guard_doppler, guard_delay, train_doppler, train_delay, rank,
+                                              scale, out.data(), &count));
+        out.resize(count);
+        return out;
+    }
 };
 
 // mod.rs:17-22 (fields are private in the reference; accessors added so results can be inspected)
@@ -173,6 +185,15 @@ struct CafB200 {
         for (std::size_t i = 0; i < arr.size() && whole; ++i) whole = arr[i].surface() == arr[0].surface() && arr[i].row() == i;
         if (!whole) throw Panic("detect_cfar needs the untouched rows of one caf_surface call");
         return arr[0].surface()->detect_cfar(k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale);
+    }
+    // OS-CFAR detection on the surface behind `arr` (same rule for `arr` and the calling thread as detect)
+    static std::vector<CfarDetection> detect_cfar_os(const std::vector<CafSurfaceRow>& arr, std::size_t k_max,
+                                                     uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler,
+                                                     uint32_t train_delay, uint32_t rank, double scale) {
+        bool whole = !arr.empty() && arr[0].surface() && arr.size() == arr[0].surface()->rows();
+        for (std::size_t i = 0; i < arr.size() && whole; ++i) whole = arr[i].surface() == arr[0].surface() && arr[i].row() == i;
+        if (!whole) throw Panic("detect_cfar_os needs the untouched rows of one caf_surface call");
+        return arr[0].surface()->detect_cfar_os(k_max, guard_doppler, guard_delay, train_doppler, train_delay, rank, scale);
     }
     // caf_surface + find_peak fused on the GPU, the surface never leaves the chip
     static std::pair<double, std::size_t> caf_peak(const std::vector<Complex64>& needle, const std::vector<Complex64>& haystack,

@@ -5,7 +5,8 @@
 //
 //   caf_cli NEEDLE.c64 HAYSTACK.c64 [--fmin HZ] [--fmax HZ] [--fstep HZ] [--fs HZ]
 //           [--layout rust|go|python] [--dump FILE] [--device-load]
-//           [--detect K [--guard-doppler R] [--guard-delay C] [--min-db X]]
+//           [--detect K [--guard-doppler R] [--guard-delay C] [--min-db X |
+//                        --cfar-db X [--train-doppler A] [--train-delay B] [--cfar-rank K]]]
 //
 // With no options it prints exactly what main.rs prints for the same two files:
 //     Frequency offset: 69.0Hz
@@ -20,6 +21,8 @@
 // --cfar-db X (with --detect K, instead of --min-db) keeps only the local maxima more than X dB above their local noise
 // estimate (caf_b200_surface_detect_cfar, scale = 10^(X/10); training region --train-doppler A rows x --train-delay B
 // cells beyond the guards, default 2 x 16), at most K of them and possibly none; each line ends with its SNR.
+// --cfar-rank K (with --cfar-db) estimates the noise as the K-th smallest training cell instead of their mean
+// (ordered-statistic CFAR, caf_b200_surface_detect_cfar_os; 1 <= K <= the training cells); the lines are the same.
 // Build: g++ -std=c++17 -O2 -Iinclude tools/caf_cli.cpp -Lcaf_cookoff_b200 -lcaf_b200 -Wl,-rpath,$PWD/caf_cookoff_b200
 #include <cmath>
 #include <cstdio>
@@ -54,6 +57,7 @@ int main(int argc, char** argv) {
     double min_db = INFINITY, cfar_db = NAN;
     uint32_t train_doppler = 2, train_delay = 16;
     bool train_given = false;
+    uint32_t cfar_rank = 0;                                     // 0: cell-averaging CFAR
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
         auto need = [&](const char* what) -> const char* {
@@ -88,11 +92,12 @@ int main(int argc, char** argv) {
         }
         else if (a == "--train-doppler") { train_doppler = (uint32_t)count_arg("--train-doppler", need("--train-doppler"), 0, 32); train_given = true; }
         else if (a == "--train-delay") { train_delay = (uint32_t)count_arg("--train-delay", need("--train-delay"), 0, 256); train_given = true; }
+        else if (a == "--cfar-rank") cfar_rank = (uint32_t)count_arg("--cfar-rank", need("--cfar-rank"), 1, 65 * 513);
         else if (a == "-h" || a == "--help") {
             std::printf("usage: caf_cli NEEDLE.c64 HAYSTACK.c64 [--fmin HZ] [--fmax HZ] [--fstep HZ] [--fs HZ] "
                         "[--layout rust|go|python] [--dump FILE] [--device-load] "
                         "[--detect K [--guard-doppler R] [--guard-delay C] "
-                        "[--min-db X | --cfar-db X [--train-doppler A] [--train-delay B]]]\n");
+                        "[--min-db X | --cfar-db X [--train-doppler A] [--train-delay B] [--cfar-rank K]]]\n");
             return 0;
         } else if (a.rfind("--", 0) == 0) { std::fprintf(stderr, "caf_cli: unknown option %s\n", a.c_str()); return 2; }
         else pos.push_back(a);
@@ -103,6 +108,7 @@ int main(int argc, char** argv) {
     if (cfar && !detecting) { std::fprintf(stderr, "caf_cli: --cfar-db needs --detect K\n"); return 2; }
     if (cfar && !std::isinf(min_db)) { std::fprintf(stderr, "caf_cli: --cfar-db and --min-db exclude each other\n"); return 2; }
     if (train_given && !cfar) { std::fprintf(stderr, "caf_cli: --train-doppler / --train-delay need --cfar-db\n"); return 2; }
+    if (cfar_rank && !cfar) { std::fprintf(stderr, "caf_cli: --cfar-rank needs --cfar-db\n"); return 2; }
     if (detecting && (device_load || layout != "rust" || !dump.empty())) {
         std::fprintf(stderr, "caf_cli: --detect goes with the default report (no --layout / --dump / --device-load)\n");
         return 2;
@@ -127,8 +133,11 @@ int main(int argc, char** argv) {
                 const auto [freq, idx] = CafB200::find_peak(rows);
                 std::printf("Frequency offset: %.1fHz\nTime offset: %zu samples (%.3fms)\n", freq, idx, (double)idx / ((double)fs / 1e3));
                 if (cfar) {
-                    const auto dets = CafB200::detect_cfar(rows, detect_k, guard_doppler, guard_delay, train_doppler,
-                                                           train_delay, std::pow(10.0, cfar_db / 10.0));
+                    const double scale = std::pow(10.0, cfar_db / 10.0);
+                    const auto dets = cfar_rank ? CafB200::detect_cfar_os(rows, detect_k, guard_doppler, guard_delay,
+                                                                          train_doppler, train_delay, cfar_rank, scale)
+                                                : CafB200::detect_cfar(rows, detect_k, guard_doppler, guard_delay,
+                                                                       train_doppler, train_delay, scale);
                     for (std::size_t i = 0; i < dets.size(); ++i)
                         std::printf("Detection %zu: %.4fHz (grid %.2fHz), %.3f samples (cell %llu), %.2f dB below the first, "
                                     "%.2f dB above the noise\n", i, dets[i].freq_hz_interp, dets[i].freq_hz,
