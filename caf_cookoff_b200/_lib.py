@@ -87,6 +87,10 @@ _cfar_dev = [_vp, _vp, _sz, _sz, _sz, _vp, _sz, _u32, _u32, _u32, _u32, _dbl, _v
 _cfar_noise = [_vp, _vp, _sz, _sz, _sz, _u32, _u32, _u32, _u32, _vp]
 _cfar_os_dev = [_vp, _vp, _sz, _sz, _sz, _vp, _sz, _u32, _u32, _u32, _u32, _u32, _dbl, _vp, _vp]
 _cfar_os_noise = [_vp, _vp, _sz, _sz, _sz, _u32, _u32, _u32, _u32, _u32, _vp]
+_rows = [_vp, _vp, _sz, _sz, _vp, _sz, _sz, C.c_uint64, _sz, _sz]    # handle ... k_max: what every block detector starts with
+_detect_rows = _rows + [_u32, _u32, _dbl, _vp, _vp]
+_cfar_rows = _rows + [_u32, _u32, _u32, _u32, _dbl, _vp, _vp]
+_cfar_os_rows = _rows + [_u32, _u32, _u32, _u32, _u32, _dbl, _vp, _vp]
 SYMBOLS = {
     "caf_b200_create": (_int, [_int, C.POINTER(_vp)]),
     "caf_b200_create_on_stream": (_int, [_int, _vp, C.POINTER(_vp)]),
@@ -162,6 +166,16 @@ SYMBOLS = {
     "caf_b200_comm_uses_p2p": (_int, [_vp, C.POINTER(_int)]),
     "caf_b200_sharded_f64_dev": (_int, [_vp, _vp, _vp, _vp, _sz, _vp, _sz, C.c_uint64, _u32, _vp, _vp, _vp, _vp]),
     "caf_b200_sharded_f32_dev": (_int, [_vp, _vp, _vp, _vp, _sz, _vp, _sz, C.c_uint64, _u32, _vp, _vp, _vp, _vp]),
+    "caf_b200_detect_rows_f64_dev": (_int, _detect_rows),
+    "caf_b200_detect_rows_f32_dev": (_int, _detect_rows),
+    "caf_b200_detect_cfar_rows_f64_dev": (_int, _cfar_rows),
+    "caf_b200_detect_cfar_rows_f32_dev": (_int, _cfar_rows),
+    "caf_b200_detect_cfar_os_rows_f64_dev": (_int, _cfar_os_rows),
+    "caf_b200_detect_cfar_os_rows_f32_dev": (_int, _cfar_os_rows),
+    "caf_b200_detect_merge_dev": (_int, [_vp, _vp, _vp, _sz, _sz, _dbl, _vp, _vp]),
+    "caf_b200_cfar_merge_dev": (_int, [_vp, _vp, _vp, _sz, _sz, _vp, _vp]),
+    "caf_b200_detect_allgather_dev": (_int, [_vp, _vp, _vp, _vp, _sz, _dbl, _vp, _vp]),
+    "caf_b200_cfar_allgather_dev": (_int, [_vp, _vp, _vp, _vp, _sz, _vp, _vp]),
 }
 
 _lib = None

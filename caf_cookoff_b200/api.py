@@ -462,6 +462,75 @@ def cfar_os_noise_dev(surface_ptr: int, p: int, d: int, n: int, noise_ptr: int, 
               int(train_doppler), int(train_delay), int(rank), C.c_void_p(noise_ptr)))
 
 
+def halo_rows(detector: str, guard_doppler: int, train_doppler: int = 0) -> int:
+    """H, the rows on each side of a rank's owned rows that its block must hold for *_rows_dev to give the whole-surface
+    answer (include/caf_b200.h, DESIGN.md section 12): max(guard_doppler, 1) for "detect", max(guard_doppler +
+    train_doppler, 1) for "cfar" and "cfar_os"."""
+    if detector == "detect":
+        return max(int(guard_doppler), 1)
+    if detector in ("cfar", "cfar_os"):
+        return max(int(guard_doppler) + int(train_doppler), 1)
+    raise ValueError("detector must be 'detect', 'cfar' or 'cfar_os'")
+
+
+def _rows_args(surface_ptr, d_buf, n, freqs_ptr, row_lo, row_hi, row_offset, d_global, k_max):
+    return [C.c_void_p(surface_ptr), int(d_buf), int(n), C.c_void_p(freqs_ptr), int(row_lo), int(row_hi),
+            int(row_offset), int(d_global), int(k_max)]
+
+
+def detect_rows_dev(surface_ptr: int, d_buf: int, n: int, freqs_ptr: int, row_lo: int, row_hi: int, row_offset: int,
+                    d_global: int, k_max: int, out_ptr: int, count_ptr: int, *, guard_doppler: int = 1,
+                    guard_delay: int = 1, min_ratio: float = 0.0, f32: bool = False, handle: Optional[Handle] = None):
+    """caf_b200_detect_rows_{f64,f32}_dev: detect over owned rows [row_lo, row_hi) of a block [d_buf][n] whose row 0 is
+    global row row_offset of a d_global-row surface; freqs [d_buf] is the block's grid; out [k_max] records carry global
+    rows, count is one uint64.  Asynchronous on the handle's stream."""
+    h = handle or default_handle()
+    fn = getattr(_lib.load(), "caf_b200_detect_rows_f32_dev" if f32 else "caf_b200_detect_rows_f64_dev")
+    _check(fn(h.raw, *_rows_args(surface_ptr, d_buf, n, freqs_ptr, row_lo, row_hi, row_offset, d_global, k_max),
+              int(guard_doppler), int(guard_delay), float(min_ratio), C.c_void_p(out_ptr), C.c_void_p(count_ptr)))
+
+
+def detect_cfar_rows_dev(surface_ptr: int, d_buf: int, n: int, freqs_ptr: int, row_lo: int, row_hi: int,
+                         row_offset: int, d_global: int, k_max: int, out_ptr: int, count_ptr: int, *, scale: float,
+                         guard_doppler: int = 1, guard_delay: int = 1, train_doppler: int = 2, train_delay: int = 16,
+                         f32: bool = False, handle: Optional[Handle] = None):
+    """caf_b200_detect_cfar_rows_{f64,f32}_dev: detect_cfar over a block's owned rows, as detect_rows_dev."""
+    h = handle or default_handle()
+    fn = getattr(_lib.load(), "caf_b200_detect_cfar_rows_f32_dev" if f32 else "caf_b200_detect_cfar_rows_f64_dev")
+    _check(fn(h.raw, *_rows_args(surface_ptr, d_buf, n, freqs_ptr, row_lo, row_hi, row_offset, d_global, k_max),
+              int(guard_doppler), int(guard_delay), int(train_doppler), int(train_delay), float(scale),
+              C.c_void_p(out_ptr), C.c_void_p(count_ptr)))
+
+
+def detect_cfar_os_rows_dev(surface_ptr: int, d_buf: int, n: int, freqs_ptr: int, row_lo: int, row_hi: int,
+                            row_offset: int, d_global: int, k_max: int, out_ptr: int, count_ptr: int, *, rank: int,
+                            scale: float, guard_doppler: int = 1, guard_delay: int = 1, train_doppler: int = 2,
+                            train_delay: int = 16, f32: bool = False, handle: Optional[Handle] = None):
+    """caf_b200_detect_cfar_os_rows_{f64,f32}_dev: detect_cfar_os over a block's owned rows, as detect_rows_dev."""
+    h = handle or default_handle()
+    fn = getattr(_lib.load(), "caf_b200_detect_cfar_os_rows_f32_dev" if f32 else "caf_b200_detect_cfar_os_rows_f64_dev")
+    _check(fn(h.raw, *_rows_args(surface_ptr, d_buf, n, freqs_ptr, row_lo, row_hi, row_offset, d_global, k_max),
+              int(guard_doppler), int(guard_delay), int(train_doppler), int(train_delay), int(rank), float(scale),
+              C.c_void_p(out_ptr), C.c_void_p(count_ptr)))
+
+
+def detect_merge_dev(lists_ptr: int, counts_ptr: int, world: int, k_max: int, out_ptr: int, count_ptr: int, *,
+                     min_ratio: float = 0.0, handle: Optional[Handle] = None):
+    """caf_b200_detect_merge_dev: the ranks' detect_rows_dev lists [world][k_max] and counts [world] (device) -> the
+    whole-surface records out [k_max] and count.  Asynchronous on the handle's stream."""
+    h = handle or default_handle()
+    _check(_lib.load().caf_b200_detect_merge_dev(h.raw, C.c_void_p(lists_ptr), C.c_void_p(counts_ptr), int(world),
+                                                 int(k_max), float(min_ratio), C.c_void_p(out_ptr), C.c_void_p(count_ptr)))
+
+
+def cfar_merge_dev(lists_ptr: int, counts_ptr: int, world: int, k_max: int, out_ptr: int, count_ptr: int, *,
+                   handle: Optional[Handle] = None):
+    """caf_b200_cfar_merge_dev: detect_merge_dev for the 64-byte records of both CFAR detectors (no min_ratio)."""
+    h = handle or default_handle()
+    _check(_lib.load().caf_b200_cfar_merge_dev(h.raw, C.c_void_p(lists_ptr), C.c_void_p(counts_ptr), int(world),
+                                               int(k_max), C.c_void_p(out_ptr), C.c_void_p(count_ptr)))
+
+
 def peak_pack(pk: _lib.Peak, global_row_offset: int) -> np.ndarray:
     """caf_b200_peak_pack -> 4 uint64 words for the NCCL exchange."""
     words = (C.c_uint64 * 4)()

@@ -127,6 +127,7 @@ struct caf_b200_comm_s {
     unsigned long long** peer_mail = nullptr;     // device: [world] pointers (own entry = mail)
     std::vector<void*> opened;                    // IPC mappings to close
     unsigned long long p2p_epoch = 0;
+    DevBuf det_x;                                 // detection exchange: this rank's block, then the world's
 };
 
 struct caf_b200_handle_s {
@@ -315,21 +316,30 @@ cudaError_t configure_fused() {
 // belongs to the device, so every handle sets the same value and no handle can lower it under another)
 template <typename T>
 cudaError_t configure_detect() {
-    return cudaFuncSetAttribute(caf::caf_detect_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(caf::caf_detect_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)caf::det_tile_smem_max<T>());
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(caf::caf_detect_tiles_rows_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)caf::det_tile_smem_max<T>());
 }
 
 // CFAR tiles: the same rule, at the most run_cfar_dev can ask for (a one-row tile staging its training region)
 template <typename T>
 cudaError_t configure_cfar() {
-    return cudaFuncSetAttribute(caf::caf_cfar_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(caf::caf_cfar_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)caf::kCfarSmemMax);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(caf::caf_cfar_tiles_rows_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)caf::kCfarSmemMax);
 }
 
 // OS-CFAR tiles: the same, at the most run_cfar_os_dev can ask for
 template <typename T>
 cudaError_t configure_cfar_os() {
-    return cudaFuncSetAttribute(caf::caf_cfar_os_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(caf::caf_cfar_os_tiles_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)caf::kCfarSmemMax);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(caf::caf_cfar_os_tiles_rows_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)caf::kCfarSmemMax);
 }
 
@@ -1551,23 +1561,41 @@ int run_detection(caf_b200_handle h, size_t p, size_t d, size_t n, size_t k_max,
     return CAF_B200_OK;
 }
 
-// Both passes on the handle's stream; every pointer is device memory.  Arguments are already checked.
+// Owned rows [lo, hi) of a block of rows whose row 0 is global row offset (DESIGN.md section 12): the tiles cover those
+// rows only and the records carry global rows.
+struct RowBlock { size_t lo, hi; uint64_t offset; };
+
+// Both passes on the handle's stream; every pointer is device memory.  Arguments are already checked.  With blk (p = 1),
+// detection over the block's owned rows.
 template <typename T>
 int run_detect_dev(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs, size_t k_max,
-                   uint32_t gr, uint32_t gd, double min_ratio, caf::DetectOut* out, unsigned long long* counts) {
+                   uint32_t gr, uint32_t gd, double min_ratio, caf::DetectOut* out, unsigned long long* counts,
+                   const RowBlock* blk = nullptr) {
     using namespace caf;
     if (p == 0) return CAF_B200_OK;
-    const int tr = det_tile_rows(d, [&](int t) { return det_tile_smem<T>(t, (int)gr, (int)gd); });
+    const size_t rows = blk ? blk->hi - blk->lo : d;                 // the rows the tiles cover
+    const int tr = det_tile_rows(rows, [&](int t) { return det_tile_smem<T>(t, (int)gr, (int)gd); });
     const size_t smem = det_tile_smem<T>(tr, (int)gr, (int)gd);      // <= det_tile_smem_max<T>(), set at handle creation
     return run_detection<DetEntry>(
-        h, p, d, n, k_max, tr, det_tile_max_maxima(tr, (int)gr, (int)gd),
+        h, p, rows, n, k_max, tr, det_tile_max_maxima(tr, (int)gr, (int)gd),
         [&](unsigned grid, long long tiles_c, long long tiles, long long cap, DetEntry* entries, unsigned long long* ctr) {
-            caf_detect_tiles_kernel<T><<<grid, kDetCols, smem, h->stream>>>(
-                surface, (long long)d, (long long)n, (int)gr, (int)gd, tr, tiles_c, tiles, (unsigned)k_max, cap, entries, ctr);
+            if (blk)
+                caf_detect_tiles_rows_kernel<T><<<grid, kDetCols, smem, h->stream>>>(
+                    surface, (long long)d, (long long)n, (int)gr, (int)gd, tr, tiles_c, tiles, (unsigned)k_max, cap, entries,
+                    ctr, (long long)blk->lo, (long long)blk->hi);
+            else
+                caf_detect_tiles_kernel<T><<<grid, kDetCols, smem, h->stream>>>(
+                    surface, (long long)d, (long long)n, (int)gr, (int)gd, tr, tiles_c, tiles, (unsigned)k_max, cap, entries,
+                    ctr);
         },
         [&](long long cap, const DetEntry* entries, const unsigned long long* ctr) {
-            caf_detect_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
-                surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, min_ratio, out, counts);
+            if (blk)
+                caf_detect_merge_rows_kernel<T><<<1, kDetMergeThreads, 0, h->stream>>>(
+                    surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, min_ratio, out, counts,
+                    (long long)blk->offset);
+            else
+                caf_detect_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
+                    surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, min_ratio, out, counts);
         });
 }
 
@@ -1659,34 +1687,55 @@ int check_cfar(size_t d, size_t n, size_t k_max, uint32_t gr, uint32_t gd, uint3
     return check_cfar_window(d, n, gr, gd, tr, tc);
 }
 
-// Both passes on the handle's stream; every pointer is device memory.  Arguments are already checked.
+// pass 2 of both CFAR detectors, over p surfaces or (blk, p = 1) a block's owned rows
+template <typename T>
+void cfar_merge_launch(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs, long long cap,
+                       const caf::CfarEntry* entries, const unsigned long long* ctr, size_t k_max, caf::CfarOut* out,
+                       unsigned long long* counts, const RowBlock* blk) {
+    using namespace caf;
+    if (blk)
+        caf_cfar_merge_rows_kernel<T><<<1, kDetMergeThreads, 0, h->stream>>>(
+            surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, out, counts,
+            (long long)blk->offset);
+    else
+        caf_cfar_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
+            surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, out, counts);
+}
+
+// Both passes on the handle's stream; every pointer is device memory.  Arguments are already checked.  blk as in
+// run_detect_dev.
 template <typename T>
 int run_cfar_dev(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs, size_t k_max,
                  uint32_t gr, uint32_t gd, uint32_t trd, uint32_t tcd, double scale, caf::CfarOut* out,
-                 unsigned long long* counts) {
+                 unsigned long long* counts, const RowBlock* blk = nullptr) {
     using namespace caf;
     if (p == 0) return CAF_B200_OK;
+    const size_t rows = blk ? blk->hi - blk->lo : d;
     const int R = (int)(gr + trd), C = (int)(gd + tcd);
     // tile height: the tallest tile that stages its training region; else one row staging up to kCfarSmemMax; else (the
     // largest windows) the tallest tile that reads its training cells from the surface
     auto smem = [&](int tr, bool staged) {
         return cfar_tile_layout<T>(tr, (int)gr, (int)gd, R, C, staged, (int)det_tile_max_maxima(tr, (int)gr, (int)gd)).total;
     };
-    int tr = det_tile_rows(d, [&](int t) { return smem(t, true); });
+    int tr = det_tile_rows(rows, [&](int t) { return smem(t, true); });
     const bool staged = smem(tr, true) <= kCfarSmemMax;
-    if (!staged) tr = det_tile_rows(d, [&](int t) { return smem(t, false); });
+    if (!staged) tr = det_tile_rows(rows, [&](int t) { return smem(t, false); });
     const size_t bytes = smem(tr, staged);                       // <= kCfarSmemMax, set at handle creation
     const int mx = (int)det_tile_max_maxima(tr, (int)gr, (int)gd);
     return run_detection<CfarEntry>(
-        h, p, d, n, k_max, tr, (size_t)mx,
+        h, p, rows, n, k_max, tr, (size_t)mx,
         [&](unsigned grid, long long tiles_c, long long tiles, long long cap, CfarEntry* entries, unsigned long long* ctr) {
-            caf_cfar_tiles_kernel<T><<<grid, kDetCols, bytes, h->stream>>>(
-                surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, scale, tiles_c, tiles,
-                (unsigned)k_max, cap, entries, ctr);
+            if (blk)
+                caf_cfar_tiles_rows_kernel<T><<<grid, kDetCols, bytes, h->stream>>>(
+                    surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, scale, tiles_c, tiles,
+                    (unsigned)k_max, cap, entries, ctr, (long long)blk->lo, (long long)blk->hi);
+            else
+                caf_cfar_tiles_kernel<T><<<grid, kDetCols, bytes, h->stream>>>(
+                    surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, scale, tiles_c, tiles,
+                    (unsigned)k_max, cap, entries, ctr);
         },
         [&](long long cap, const CfarEntry* entries, const unsigned long long* ctr) {
-            caf_cfar_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
-                surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, out, counts);
+            cfar_merge_launch<T>(h, surface, p, d, n, freqs, cap, entries, ctr, k_max, out, counts, blk);
         });
 }
 
@@ -1791,29 +1840,34 @@ int check_cfar_os(size_t d, size_t n, size_t k_max, uint32_t gr, uint32_t gd, ui
 template <typename T>
 int run_cfar_os_dev(caf_b200_handle h, const T* surface, size_t p, size_t d, size_t n, const double* freqs, size_t k_max,
                     uint32_t gr, uint32_t gd, uint32_t trd, uint32_t tcd, uint32_t rank, double scale, caf::CfarOut* out,
-                    unsigned long long* counts) {
+                    unsigned long long* counts, const RowBlock* blk = nullptr) {
     using namespace caf;
     if (p == 0) return CAF_B200_OK;
+    const size_t rows = blk ? blk->hi - blk->lo : d;
     const int R = (int)(gr + trd), C = (int)(gd + tcd);
     auto smem = [&](int tr, bool staged) {
         return cfar_os_tile_layout<T>(tr, (int)gr, (int)gd, R, C, staged, (int)det_tile_max_maxima(tr, (int)gr, (int)gd)).total;
     };
-    int tr = det_tile_rows(d, [&](int t) { return smem(t, true); });
+    int tr = det_tile_rows(rows, [&](int t) { return smem(t, true); });
     const bool staged = smem(tr, true) <= kCfarSmemMax;
-    if (!staged) tr = det_tile_rows(d, [&](int t) { return smem(t, false); });
+    if (!staged) tr = det_tile_rows(rows, [&](int t) { return smem(t, false); });
     const size_t bytes = smem(tr, staged);                       // <= kCfarSmemMax, set at handle creation
     const int mx = (int)det_tile_max_maxima(tr, (int)gr, (int)gd);
     const unsigned long long ntrain = cfar_train_cells(gr, gd, trd, tcd);
     return run_detection<CfarEntry>(
-        h, p, d, n, k_max, tr, (size_t)mx,
+        h, p, rows, n, k_max, tr, (size_t)mx,
         [&](unsigned grid, long long tiles_c, long long tiles, long long cap, CfarEntry* entries, unsigned long long* ctr) {
-            caf_cfar_os_tiles_kernel<T><<<grid, kDetCols, bytes, h->stream>>>(
-                surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, rank, ntrain, scale, tiles_c,
-                tiles, (unsigned)k_max, cap, entries, ctr);
+            if (blk)
+                caf_cfar_os_tiles_rows_kernel<T><<<grid, kDetCols, bytes, h->stream>>>(
+                    surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, rank, ntrain, scale,
+                    tiles_c, tiles, (unsigned)k_max, cap, entries, ctr, (long long)blk->lo, (long long)blk->hi);
+            else
+                caf_cfar_os_tiles_kernel<T><<<grid, kDetCols, bytes, h->stream>>>(
+                    surface, (long long)d, (long long)n, (int)gr, (int)gd, R, C, tr, staged, mx, rank, ntrain, scale,
+                    tiles_c, tiles, (unsigned)k_max, cap, entries, ctr);
         },
         [&](long long cap, const CfarEntry* entries, const unsigned long long* ctr) {
-            caf_cfar_merge_kernel<T><<<(unsigned)p, kDetMergeThreads, 0, h->stream>>>(
-                surface, (long long)d, (long long)n, freqs, entries, cap, ctr, (unsigned)k_max, out, counts);
+            cfar_merge_launch<T>(h, surface, p, d, n, freqs, cap, entries, ctr, k_max, out, counts, blk);
         });
 }
 
@@ -1893,6 +1947,168 @@ int caf_b200_cfar_os_noise_f32_dev(caf_b200_handle h, const float* surface, size
                                    uint32_t train_delay, uint32_t rank, double* noise_out) {
     return cfar_os_noise_dev_impl<float>(h, surface, p, d, n, guard_doppler, guard_delay, train_doppler, train_delay, rank,
                                          noise_out);
+}
+
+// ---- detection on the owned rows of a row block, and the merge of the ranks' lists (DESIGN.md section 12) -----------
+extern "C++" {
+namespace {
+// Owned rows [row_lo, row_hi) of a block of d_buf rows whose row 0 is global row row_offset, on a surface of d_global
+// rows, read with a neighbourhood of H rows: on each side the block holds H rows past the owned ones or ends where the
+// surface does (there the block's edge clips windows exactly as the surface's).  An empty owned range needs no halo.
+int check_rows(size_t d_buf, size_t row_lo, size_t row_hi, uint64_t row_offset, size_t d_global, size_t H) {
+    if (row_lo > row_hi || row_hi > d_buf) return fail(CAF_B200_EINVAL, "owned rows must satisfy row_lo <= row_hi <= d_buf");
+    if (row_offset > d_global || d_buf > d_global - row_offset)
+        return fail(CAF_B200_EINVAL, "row_offset + d_buf exceeds d_global");
+    if (d_global > (1ull << 31)) return fail(CAF_B200_EUNSUPPORTED, "more than 2^31 rows");
+    if (row_lo == row_hi) return CAF_B200_OK;
+    if (row_lo < H && row_offset != 0)
+        return fail(CAF_B200_EINVAL, "the block holds fewer than H halo rows above the owned rows");
+    if (d_buf - row_hi < H && row_offset + d_buf != d_global)
+        return fail(CAF_B200_EINVAL, "the block holds fewer than H halo rows below the owned rows");
+    return CAF_B200_OK;
+}
+
+// the checks every block detector shares after its own limits: handle, rows, pointers, size
+int check_rows_call(caf_b200_handle h, const void* surface, size_t d_buf, size_t n, const double* freqs, size_t row_lo,
+                    size_t row_hi, uint64_t row_offset, size_t d_global, size_t H, const void* out, const void* count) {
+    int rc = check_rows(d_buf, row_lo, row_hi, row_offset, d_global, H);
+    if (rc) return rc;
+    if (!out || !count) return fail(CAF_B200_EINVAL, "null out / count");
+    if (row_lo < row_hi && n && !surface) return fail(CAF_B200_EINVAL, "null surface");
+    if (row_lo < row_hi && !freqs) return fail(CAF_B200_EINVAL, "null freqs_hz");
+    if ((double)d_buf * (double)n > 9.0e18) return fail(CAF_B200_EUNSUPPORTED, "surface too large");
+    if (cudaSetDevice(h->device) != cudaSuccess) return fail(CAF_B200_ECUDA, "cudaSetDevice failed");
+    return CAF_B200_OK;
+}
+
+size_t halo_of(uint32_t rows) { return rows > 1 ? rows : 1; }
+
+template <typename T>
+int detect_rows_impl(caf_b200_handle h, const T* surface, size_t d_buf, size_t n, const double* freqs, size_t row_lo,
+                     size_t row_hi, uint64_t row_offset, size_t d_global, size_t k_max, uint32_t gr, uint32_t gd,
+                     double min_ratio, caf_b200_detection* out, uint64_t* count) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_detect(d_buf, n, k_max, gr, gd, min_ratio);
+    if (!rc) rc = check_rows_call(h, surface, d_buf, n, freqs, row_lo, row_hi, row_offset, d_global, halo_of(gr), out, count);
+    if (rc) return rc;
+    const RowBlock blk{row_lo, row_hi, row_offset};
+    return run_detect_dev<T>(h, surface, 1, d_buf, n, freqs, k_max, gr, gd, min_ratio, (caf::DetectOut*)out,
+                             (unsigned long long*)count, &blk);
+}
+
+template <typename T>
+int detect_cfar_rows_impl(caf_b200_handle h, const T* surface, size_t d_buf, size_t n, const double* freqs, size_t row_lo,
+                          size_t row_hi, uint64_t row_offset, size_t d_global, size_t k_max, uint32_t gr, uint32_t gd,
+                          uint32_t tr, uint32_t tc, double scale, caf_b200_cfar_detection* out, uint64_t* count) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_cfar(d_buf, n, k_max, gr, gd, tr, tc, scale);
+    if (!rc) rc = check_rows_call(h, surface, d_buf, n, freqs, row_lo, row_hi, row_offset, d_global, halo_of(gr + tr), out, count);
+    if (rc) return rc;
+    const RowBlock blk{row_lo, row_hi, row_offset};
+    return run_cfar_dev<T>(h, surface, 1, d_buf, n, freqs, k_max, gr, gd, tr, tc, scale, (caf::CfarOut*)out,
+                           (unsigned long long*)count, &blk);
+}
+
+template <typename T>
+int detect_cfar_os_rows_impl(caf_b200_handle h, const T* surface, size_t d_buf, size_t n, const double* freqs,
+                             size_t row_lo, size_t row_hi, uint64_t row_offset, size_t d_global, size_t k_max, uint32_t gr,
+                             uint32_t gd, uint32_t tr, uint32_t tc, uint32_t rank, double scale,
+                             caf_b200_cfar_detection* out, uint64_t* count) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_cfar_os(d_buf, n, k_max, gr, gd, tr, tc, rank, scale);
+    if (!rc) rc = check_rows_call(h, surface, d_buf, n, freqs, row_lo, row_hi, row_offset, d_global, halo_of(gr + tr), out, count);
+    if (rc) return rc;
+    const RowBlock blk{row_lo, row_hi, row_offset};
+    return run_cfar_os_dev<T>(h, surface, 1, d_buf, n, freqs, k_max, gr, gd, tr, tc, rank, scale, (caf::CfarOut*)out,
+                              (unsigned long long*)count, &blk);
+}
+
+constexpr size_t kMaxWorld = 1u << 16;
+
+int check_merge(size_t world, size_t k_max, const void* lists, const void* counts, const void* out, const void* count) {
+    if (k_max < 1 || k_max > (size_t)caf::kDetMaxK) return fail(CAF_B200_EINVAL, "k_max must be 1 ... 1024");
+    if (world < 1 || world > kMaxWorld) return fail(CAF_B200_EINVAL, "world must be 1 ... 65536");
+    if (!lists || !counts || !out || !count) return fail(CAF_B200_EINVAL, "null lists / counts / out / count");
+    return CAF_B200_OK;
+}
+}  // namespace
+}  // extern "C++"
+
+int caf_b200_detect_rows_f64_dev(caf_b200_handle h, const double* surface, size_t d_buf, size_t n, const double* freqs_hz,
+                                 size_t row_lo, size_t row_hi, uint64_t row_offset, size_t d_global, size_t k_max,
+                                 uint32_t guard_doppler, uint32_t guard_delay, double min_ratio, caf_b200_detection* out,
+                                 uint64_t* count) {
+    return detect_rows_impl<double>(h, surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset, d_global, k_max,
+                                    guard_doppler, guard_delay, min_ratio, out, count);
+}
+int caf_b200_detect_rows_f32_dev(caf_b200_handle h, const float* surface, size_t d_buf, size_t n, const double* freqs_hz,
+                                 size_t row_lo, size_t row_hi, uint64_t row_offset, size_t d_global, size_t k_max,
+                                 uint32_t guard_doppler, uint32_t guard_delay, double min_ratio, caf_b200_detection* out,
+                                 uint64_t* count) {
+    return detect_rows_impl<float>(h, surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset, d_global, k_max,
+                                   guard_doppler, guard_delay, min_ratio, out, count);
+}
+int caf_b200_detect_cfar_rows_f64_dev(caf_b200_handle h, const double* surface, size_t d_buf, size_t n,
+                                      const double* freqs_hz, size_t row_lo, size_t row_hi, uint64_t row_offset,
+                                      size_t d_global, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                      uint32_t train_doppler, uint32_t train_delay, double scale,
+                                      caf_b200_cfar_detection* out, uint64_t* count) {
+    return detect_cfar_rows_impl<double>(h, surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset, d_global, k_max,
+                                         guard_doppler, guard_delay, train_doppler, train_delay, scale, out, count);
+}
+int caf_b200_detect_cfar_rows_f32_dev(caf_b200_handle h, const float* surface, size_t d_buf, size_t n,
+                                      const double* freqs_hz, size_t row_lo, size_t row_hi, uint64_t row_offset,
+                                      size_t d_global, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                      uint32_t train_doppler, uint32_t train_delay, double scale,
+                                      caf_b200_cfar_detection* out, uint64_t* count) {
+    return detect_cfar_rows_impl<float>(h, surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset, d_global, k_max,
+                                        guard_doppler, guard_delay, train_doppler, train_delay, scale, out, count);
+}
+int caf_b200_detect_cfar_os_rows_f64_dev(caf_b200_handle h, const double* surface, size_t d_buf, size_t n,
+                                         const double* freqs_hz, size_t row_lo, size_t row_hi, uint64_t row_offset,
+                                         size_t d_global, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                         uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                         caf_b200_cfar_detection* out, uint64_t* count) {
+    return detect_cfar_os_rows_impl<double>(h, surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset, d_global, k_max,
+                                            guard_doppler, guard_delay, train_doppler, train_delay, rank, scale, out,
+                                            count);
+}
+int caf_b200_detect_cfar_os_rows_f32_dev(caf_b200_handle h, const float* surface, size_t d_buf, size_t n,
+                                         const double* freqs_hz, size_t row_lo, size_t row_hi, uint64_t row_offset,
+                                         size_t d_global, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                         uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                         caf_b200_cfar_detection* out, uint64_t* count) {
+    return detect_cfar_os_rows_impl<float>(h, surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset, d_global, k_max,
+                                           guard_doppler, guard_delay, train_doppler, train_delay, rank, scale, out,
+                                           count);
+}
+
+int caf_b200_detect_merge_dev(caf_b200_handle h, const caf_b200_detection* lists, const uint64_t* counts, size_t world,
+                              size_t k_max, double min_ratio, caf_b200_detection* out, uint64_t* count) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_merge(world, k_max, lists, counts, out, count);
+    if (rc) return rc;
+    if (!(min_ratio >= 0.0 && min_ratio <= 1.0)) return fail(CAF_B200_EINVAL, "min_ratio must be in [0, 1]");
+    CK(cudaSetDevice(h->device));
+    caf::caf_detect_rank_merge_kernel<<<1, caf::kDetMergeThreads, 0, h->stream>>>(
+        (const caf::DetectOut*)lists, (long long)k_max, (const unsigned long long*)counts, 1, (int)world, (unsigned)k_max,
+        min_ratio, (caf::DetectOut*)out, (unsigned long long*)count, nullptr);
+    h->launches++;
+    CK(cudaGetLastError());
+    return CAF_B200_OK;
+}
+int caf_b200_cfar_merge_dev(caf_b200_handle h, const caf_b200_cfar_detection* lists, const uint64_t* counts, size_t world,
+                            size_t k_max, caf_b200_cfar_detection* out, uint64_t* count) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_merge(world, k_max, lists, counts, out, count);
+    if (rc) return rc;
+    CK(cudaSetDevice(h->device));
+    caf::caf_cfar_rank_merge_kernel<<<1, caf::kDetMergeThreads, 0, h->stream>>>(
+        (const caf::CfarOut*)lists, (long long)k_max, (const unsigned long long*)counts, 1, (int)world, (unsigned)k_max,
+        (caf::CfarOut*)out, (unsigned long long*)count, nullptr);
+    h->launches++;
+    CK(cudaGetLastError());
+    return CAF_B200_OK;
 }
 
 // ---- multi-GPU peak words: [0] = bits(value), [1] = global doppler row (UINT64_MAX if none),
@@ -2019,6 +2235,7 @@ int caf_b200_comm_destroy(caf_b200_comm c) {
     if (c->recv) cudaFree(c->recv);
     if (c->host) cudaFreeHost(c->host);
     if (c->status) cudaFreeHost(c->status);
+    c->det_x.release();
     if (c->own && c->comm && nccl_api().ok()) nccl_api().CommDestroy(c->comm);
     delete c;
     return CAF_B200_OK;
@@ -2109,6 +2326,72 @@ int caf_b200_peak_allgather_dev(caf_b200_handle h, caf_b200_comm c, const caf_b2
     h->launches++;
     CK(cudaGetLastError());
     return exchange_sync(h, c, out);
+}
+
+extern "C++" {
+namespace {
+// The detection exchange: this rank's k_max records and count go out as one block of k_max + 1 records (the count in the
+// last slot), ONE ncclAllGather gives every rank the world's blocks, and merge(lists, list_stride, counts, count_stride,
+// status) launches the merge across ranks over them.  A rank whose inputs are missing still enters the collective, with
+// the failure mark as its count; its peers' merges skip its list and report it through c->status.  Synchronous.
+template <typename Rec, typename Merge>
+int detection_allgather(caf_b200_handle h, caf_b200_comm c, const Rec* local, const uint64_t* local_count, size_t k_max,
+                        Rec* out, uint64_t* count, Merge merge) {
+    int rc = check_comm(h, c);
+    if (rc) return rc;
+    // k_max sizes the collective, so every rank passes the same one: a bad value fails on every rank before it
+    if (k_max < 1 || k_max > (size_t)caf::kDetMaxK) return fail(CAF_B200_EINVAL, "k_max must be 1 ... 1024");
+    CK(cudaSetDevice(h->device));
+    const size_t blk = (k_max + 1) * sizeof(Rec);
+    CK(c->det_x.ensure(blk * ((size_t)c->world + 1)));
+    char* send = (char*)c->det_x.p;
+    char* recv = send + blk;
+    unsigned long long* send_count = (unsigned long long*)(send + k_max * sizeof(Rec));
+    const bool ok = local && local_count && out && count;
+    if (ok) {
+        CK(cudaMemcpyAsync(send, local, k_max * sizeof(Rec), cudaMemcpyDeviceToDevice, h->stream));
+        CK(cudaMemcpyAsync(send_count, local_count, 8, cudaMemcpyDeviceToDevice, h->stream));
+    } else {
+        const unsigned long long mark = caf::kPeakRemoteError;
+        CK(cudaMemcpyAsync(send_count, &mark, 8, cudaMemcpyHostToDevice, h->stream));
+    }
+    CKN(nccl_api().AllGather(send, recv, blk / 8, kNcclUint64, c->comm, h->stream));
+    if (!ok) {
+        cudaStreamSynchronize(h->stream);
+        return fail(CAF_B200_EINVAL, "null local records / local count / out / count");
+    }
+    merge((const Rec*)recv, (long long)(k_max + 1), (const unsigned long long*)(recv + k_max * sizeof(Rec)),
+          (long long)(blk / 8), c->status);
+    h->launches++;
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(h->stream));
+    if (*c->status) return fail(CAF_B200_EREMOTE, "a peer rank failed before the detection exchange");
+    return CAF_B200_OK;
+}
+}  // namespace
+}  // extern "C++"
+
+int caf_b200_detect_allgather_dev(caf_b200_handle h, caf_b200_comm c, const caf_b200_detection* local,
+                                  const uint64_t* local_count, size_t k_max, double min_ratio, caf_b200_detection* out,
+                                  uint64_t* count) {
+    // like k_max, the same on every rank: a bad value fails on every rank before the collective
+    if (!(min_ratio >= 0.0 && min_ratio <= 1.0)) return fail(CAF_B200_EINVAL, "min_ratio must be in [0, 1]");
+    return detection_allgather<caf::DetectOut>(
+        h, c, (const caf::DetectOut*)local, local_count, k_max, (caf::DetectOut*)out, count,
+        [&](const caf::DetectOut* lists, long long ls, const unsigned long long* counts, long long cs, int* status) {
+            caf::caf_detect_rank_merge_kernel<<<1, caf::kDetMergeThreads, 0, h->stream>>>(
+                lists, ls, counts, cs, c->world, (unsigned)k_max, min_ratio, (caf::DetectOut*)out,
+                (unsigned long long*)count, status);
+        });
+}
+int caf_b200_cfar_allgather_dev(caf_b200_handle h, caf_b200_comm c, const caf_b200_cfar_detection* local,
+                                const uint64_t* local_count, size_t k_max, caf_b200_cfar_detection* out, uint64_t* count) {
+    return detection_allgather<caf::CfarOut>(
+        h, c, (const caf::CfarOut*)local, local_count, k_max, (caf::CfarOut*)out, count,
+        [&](const caf::CfarOut* lists, long long ls, const unsigned long long* counts, long long cs, int* status) {
+            caf::caf_cfar_rank_merge_kernel<<<1, caf::kDetMergeThreads, 0, h->stream>>>(
+                lists, ls, counts, cs, c->world, (unsigned)k_max, (caf::CfarOut*)out, (unsigned long long*)count, status);
+        });
 }
 
 extern "C++" {

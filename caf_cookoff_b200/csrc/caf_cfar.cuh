@@ -85,11 +85,12 @@ __device__ __forceinline__ double cfar_noise_of(double sum, unsigned m) {
 // ---- pass 1 --------------------------------------------------------------------------------------------------------
 // surf [p][d][n]; grid = p * tiles_per_pair CTAs of kDetCols threads.  ctr [p][2] = (entries appended, floor value bits),
 // zeroed before the launch; entries [p][cap].  mx = det_tile_max_maxima(tr, gr, gd), the candidate slots of a tile.
-template <typename T>
-__global__ void __launch_bounds__(kDetCols) caf_cfar_tiles_kernel(
+// BLOCK, row_lo, row_hi: as in det_tiles.
+template <typename T, bool BLOCK>
+__device__ __forceinline__ void cfar_tiles(
         const T* __restrict__ surf, long long d, long long n, int gr, int gd, int R, int C, int tr, bool staged, int mx,
         double scale, long long tiles_c, long long tiles_per_pair, unsigned kmax, long long cap,
-        CfarEntry* __restrict__ entries, unsigned long long* __restrict__ ctr) {
+        CfarEntry* __restrict__ entries, unsigned long long* __restrict__ ctr, long long row_lo, long long row_hi) {
     extern __shared__ __align__(16) unsigned char cfar_smem[];
     const CfarTileLayout L = cfar_tile_layout<T>(tr, gr, gd, R, C, staged, mx);
     T* hbuf = reinterpret_cast<T*>(cfar_smem);                            // [tr + 2 gr][kDetCols]
@@ -109,7 +110,8 @@ __global__ void __launch_bounds__(kDetCols) caf_cfar_tiles_kernel(
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const long long pair = (long long)blockIdx.x / tiles_per_pair;
     const long long t = (long long)blockIdx.x - pair * tiles_per_pair;
-    const long long r0 = (t / tiles_c) * tr, c0 = (t % tiles_c) * kDetCols;
+    const long long r0 = (BLOCK ? row_lo : 0ll) + (t / tiles_c) * tr, c0 = (t % tiles_c) * kDetCols;
+    const long long rend = BLOCK ? row_hi : d;           // candidates stop here
     const T* S = surf + pair * d * n;
     unsigned long long* my_ctr = ctr + 2 * pair;
     if (tid == 0) { ncand = 0u; nqual = 0u; nkeep = 0u; wpos = 0u; }
@@ -167,7 +169,7 @@ __global__ void __launch_bounds__(kDetCols) caf_cfar_tiles_kernel(
     const unsigned long long floor0 = *reinterpret_cast<volatile unsigned long long*>(my_ctr + 1);
     const long long c = c0 + tid;
     if (c < n) {
-        for (int q = 0; q < tr && r0 + q < d; ++q) {
+        for (int q = 0; q < tr && r0 + q < rend; ++q) {
             const long long r = r0 + q;
             const T v = vbuf[(size_t)q * kDetCols + tid];
             if (!(v > (T)0)) continue;
@@ -284,6 +286,25 @@ __global__ void __launch_bounds__(kDetCols) caf_cfar_tiles_kernel(
     }
 }
 
+template <typename T>
+__global__ void __launch_bounds__(kDetCols) caf_cfar_tiles_kernel(
+        const T* __restrict__ surf, long long d, long long n, int gr, int gd, int R, int C, int tr, bool staged, int mx,
+        double scale, long long tiles_c, long long tiles_per_pair, unsigned kmax, long long cap,
+        CfarEntry* __restrict__ entries, unsigned long long* __restrict__ ctr) {
+    cfar_tiles<T, false>(surf, d, n, gr, gd, R, C, tr, staged, mx, scale, tiles_c, tiles_per_pair, kmax, cap, entries, ctr,
+                         0, 0);
+}
+
+// rows [row_lo, row_hi) of a block of d rows
+template <typename T>
+__global__ void __launch_bounds__(kDetCols) caf_cfar_tiles_rows_kernel(
+        const T* __restrict__ surf, long long d, long long n, int gr, int gd, int R, int C, int tr, bool staged, int mx,
+        double scale, long long tiles_c, long long tiles_per_pair, unsigned kmax, long long cap,
+        CfarEntry* __restrict__ entries, unsigned long long* __restrict__ ctr, long long row_lo, long long row_hi) {
+    cfar_tiles<T, true>(surf, d, n, gr, gd, R, C, tr, staged, mx, scale, tiles_c, tiles_per_pair, kmax, cap, entries, ctr,
+                        row_lo, row_hi);
+}
+
 // ---- pass 2 --------------------------------------------------------------------------------------------------------
 // one CTA per pair: out [p][kmax], counts [p]
 template <typename T>
@@ -296,6 +317,28 @@ __global__ void __launch_bounds__(kDetMergeThreads) caf_cfar_merge_kernel(
                             o.noise = used ? __longlong_as_double((long long)w.noise_bits) : 0.0;
                             o.train_cells = used ? w.m : 0ull;
                         });
+}
+
+// one pair: a block of d rows whose row 0 is global row row_offset (both CFAR detectors)
+template <typename T>
+__global__ void __launch_bounds__(kDetMergeThreads) caf_cfar_merge_rows_kernel(
+        const T* __restrict__ surf, long long d, long long n, const double* __restrict__ freqs,
+        const CfarEntry* __restrict__ entries, long long cap, const unsigned long long* __restrict__ ctr, unsigned kmax,
+        CfarOut* __restrict__ out, unsigned long long* __restrict__ counts, long long row_offset) {
+    det_merge<T, false, true>(surf, d, n, freqs, entries, cap, ctr, kmax, 0.0, out, counts,
+                              [](CfarOut& o, const CfarEntry& w, bool used) {
+                                  o.noise = used ? __longlong_as_double((long long)w.noise_bits) : 0.0;
+                                  o.train_cells = used ? w.m : 0ull;
+                              },
+                              row_offset);
+}
+
+// the merge across ranks of CFAR records (both detectors): det_rank_merge without min_ratio
+__global__ void __launch_bounds__(kDetMergeThreads) caf_cfar_rank_merge_kernel(
+        const CfarOut* __restrict__ lists, long long list_stride, const unsigned long long* __restrict__ counts,
+        long long count_stride, int world, unsigned kmax, CfarOut* __restrict__ out, unsigned long long* __restrict__ count,
+        int* __restrict__ status) {
+    det_rank_merge<false>(lists, list_stride, counts, count_stride, world, kmax, 0.0, out, count, status);
 }
 
 // ---- the dense noise map ---------------------------------------------------------------------------------------------

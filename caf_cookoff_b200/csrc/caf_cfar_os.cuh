@@ -123,11 +123,13 @@ __device__ __forceinline__ unsigned os_rank_of(unsigned rank, unsigned m, unsign
 // ---- pass 1 --------------------------------------------------------------------------------------------------------
 // surf [p][d][n]; grid = p * tiles_per_pair CTAs of kDetCols threads.  ctr [p][2] = (entries appended, floor value bits),
 // zeroed before the launch; entries [p][cap].  mx = det_tile_max_maxima(tr, gr, gd), the candidate slots of a tile.
-template <typename T>
-__global__ void __launch_bounds__(kDetCols) caf_cfar_os_tiles_kernel(
+// BLOCK, row_lo, row_hi: as in det_tiles.
+template <typename T, bool BLOCK>
+__device__ __forceinline__ void cfar_os_tiles(
         const T* __restrict__ surf, long long d, long long n, int gr, int gd, int R, int C, int tr, bool staged, int mx,
         unsigned rank, unsigned long long ntrain, double scale, long long tiles_c, long long tiles_per_pair, unsigned kmax,
-        long long cap, CfarEntry* __restrict__ entries, unsigned long long* __restrict__ ctr) {
+        long long cap, CfarEntry* __restrict__ entries, unsigned long long* __restrict__ ctr, long long row_lo,
+        long long row_hi) {
     extern __shared__ __align__(16) unsigned char cfar_os_smem[];
     const CfarTileLayout L = cfar_os_tile_layout<T>(tr, gr, gd, R, C, staged, mx);
     T* hbuf = reinterpret_cast<T*>(cfar_os_smem);                         // [tr + 2 gr][kDetCols]
@@ -148,7 +150,8 @@ __global__ void __launch_bounds__(kDetCols) caf_cfar_os_tiles_kernel(
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const long long pair = (long long)blockIdx.x / tiles_per_pair;
     const long long t = (long long)blockIdx.x - pair * tiles_per_pair;
-    const long long r0 = (t / tiles_c) * tr, c0 = (t % tiles_c) * kDetCols;
+    const long long r0 = (BLOCK ? row_lo : 0ll) + (t / tiles_c) * tr, c0 = (t % tiles_c) * kDetCols;
+    const long long rend = BLOCK ? row_hi : d;           // candidates stop here
     const T* S = surf + pair * d * n;
     unsigned long long* my_ctr = ctr + 2 * pair;
     if (tid == 0) { ncand = 0u; nqual = 0u; nkeep = 0u; wpos = 0u; }
@@ -206,7 +209,7 @@ __global__ void __launch_bounds__(kDetCols) caf_cfar_os_tiles_kernel(
     const unsigned long long floor0 = *reinterpret_cast<volatile unsigned long long*>(my_ctr + 1);
     const long long c = c0 + tid;
     if (c < n) {
-        for (int q = 0; q < tr && r0 + q < d; ++q) {
+        for (int q = 0; q < tr && r0 + q < rend; ++q) {
             const long long r = r0 + q;
             const T v = vbuf[(size_t)q * kDetCols + tid];
             if (!(v > (T)0)) continue;
@@ -297,6 +300,26 @@ __global__ void __launch_bounds__(kDetCols) caf_cfar_os_tiles_kernel(
                                                 (unsigned long long)mcnt[ci]};
         }
     }
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kDetCols) caf_cfar_os_tiles_kernel(
+        const T* __restrict__ surf, long long d, long long n, int gr, int gd, int R, int C, int tr, bool staged, int mx,
+        unsigned rank, unsigned long long ntrain, double scale, long long tiles_c, long long tiles_per_pair, unsigned kmax,
+        long long cap, CfarEntry* __restrict__ entries, unsigned long long* __restrict__ ctr) {
+    cfar_os_tiles<T, false>(surf, d, n, gr, gd, R, C, tr, staged, mx, rank, ntrain, scale, tiles_c, tiles_per_pair, kmax,
+                            cap, entries, ctr, 0, 0);
+}
+
+// rows [row_lo, row_hi) of a block of d rows
+template <typename T>
+__global__ void __launch_bounds__(kDetCols) caf_cfar_os_tiles_rows_kernel(
+        const T* __restrict__ surf, long long d, long long n, int gr, int gd, int R, int C, int tr, bool staged, int mx,
+        unsigned rank, unsigned long long ntrain, double scale, long long tiles_c, long long tiles_per_pair, unsigned kmax,
+        long long cap, CfarEntry* __restrict__ entries, unsigned long long* __restrict__ ctr, long long row_lo,
+        long long row_hi) {
+    cfar_os_tiles<T, true>(surf, d, n, gr, gd, R, C, tr, staged, mx, rank, ntrain, scale, tiles_c, tiles_per_pair, kmax,
+                           cap, entries, ctr, row_lo, row_hi);
 }
 
 // ---- the dense noise map ---------------------------------------------------------------------------------------------

@@ -158,12 +158,14 @@ __device__ __forceinline__ bool det_key_ge(unsigned long long h, unsigned long l
 
 // ---- pass 1 --------------------------------------------------------------------------------------------------------
 // surf [p][d][n]; grid = p * tiles_per_pair CTAs of kDetCols threads.  ctr [p][2] = (entries appended, floor value bits),
-// zeroed before the launch; entries [p][cap].
-template <typename T>
-__global__ void __launch_bounds__(kDetCols) caf_detect_tiles_kernel(
+// zeroed before the launch; entries [p][cap].  With BLOCK the tiles cover only rows [row_lo, row_hi) of the d rows (a
+// rank's owned rows inside its halo'd block, DESIGN.md section 12): the rows around them are read as neighbourhood only.
+// Without it the tiles cover [0, d) and row_lo, row_hi are not read.
+template <typename T, bool BLOCK>
+__device__ __forceinline__ void det_tiles(
         const T* __restrict__ surf, long long d, long long n, int gr, int gd, int tr, long long tiles_c,
         long long tiles_per_pair, unsigned kmax, long long cap, DetEntry* __restrict__ entries,
-        unsigned long long* __restrict__ ctr) {
+        unsigned long long* __restrict__ ctr, long long row_lo, long long row_hi) {
     extern __shared__ __align__(16) unsigned char det_smem[];
     T* hbuf = reinterpret_cast<T*>(det_smem);                             // [tr + 2 gr][kDetCols]
     T* vbuf = hbuf + (size_t)(tr + 2 * gr) * kDetCols;                   // [tr][kDetCols]
@@ -178,7 +180,8 @@ __global__ void __launch_bounds__(kDetCols) caf_detect_tiles_kernel(
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const long long pair = (long long)blockIdx.x / tiles_per_pair;
     const long long t = (long long)blockIdx.x - pair * tiles_per_pair;
-    const long long r0 = (t / tiles_c) * tr, c0 = (t % tiles_c) * kDetCols;
+    const long long r0 = (BLOCK ? row_lo : 0ll) + (t / tiles_c) * tr, c0 = (t % tiles_c) * kDetCols;
+    const long long rend = BLOCK ? row_hi : d;           // candidates stop here
     const T* S = surf + pair * d * n;
     unsigned long long* my_ctr = ctr + 2 * pair;
     if (tid == 0) { ncand = 0u; nkeep = 0u; wpos = 0u; }
@@ -216,7 +219,7 @@ __global__ void __launch_bounds__(kDetCols) caf_detect_tiles_kernel(
     const unsigned long long floor0 = *reinterpret_cast<volatile unsigned long long*>(my_ctr + 1);
     const long long c = c0 + tid;
     if (c < n) {
-        for (int q = 0; q < tr && r0 + q < d; ++q) {
+        for (int q = 0; q < tr && r0 + q < rend; ++q) {
             const long long r = r0 + q;
             const T v = vbuf[(size_t)q * kDetCols + tid];
             if (!(v > (T)0)) continue;
@@ -279,6 +282,23 @@ __global__ void __launch_bounds__(kDetCols) caf_detect_tiles_kernel(
     }
 }
 
+template <typename T>
+__global__ void __launch_bounds__(kDetCols) caf_detect_tiles_kernel(
+        const T* __restrict__ surf, long long d, long long n, int gr, int gd, int tr, long long tiles_c,
+        long long tiles_per_pair, unsigned kmax, long long cap, DetEntry* __restrict__ entries,
+        unsigned long long* __restrict__ ctr) {
+    det_tiles<T, false>(surf, d, n, gr, gd, tr, tiles_c, tiles_per_pair, kmax, cap, entries, ctr, 0, 0);
+}
+
+// rows [row_lo, row_hi) of a block of d rows
+template <typename T>
+__global__ void __launch_bounds__(kDetCols) caf_detect_tiles_rows_kernel(
+        const T* __restrict__ surf, long long d, long long n, int gr, int gd, int tr, long long tiles_c,
+        long long tiles_per_pair, unsigned kmax, long long cap, DetEntry* __restrict__ entries,
+        unsigned long long* __restrict__ ctr, long long row_lo, long long row_hi) {
+    det_tiles<T, true>(surf, d, n, gr, gd, tr, tiles_c, tiles_per_pair, kmax, cap, entries, ctr, row_lo, row_hi);
+}
+
 // ---- pass 2 --------------------------------------------------------------------------------------------------------
 // one CTA per pair: out [p][kmax], counts [p]
 __device__ __forceinline__ double det_fit(double a, double v, double b) {   // parabola vertex offset, in cells
@@ -290,16 +310,38 @@ __device__ __forceinline__ double det_fit(double a, double v, double b) {   // p
 
 __device__ __forceinline__ DetectOut& det_rec(DetectOut& o) { return o; }
 template <typename Out> __device__ __forceinline__ DetectOut& det_rec(Out& o) { return o.det; }
+__device__ __forceinline__ const DetectOut& det_rec_c(const DetectOut& o) { return o; }
+template <typename Out> __device__ __forceinline__ const DetectOut& det_rec_c(const Out& o) { return o.det; }
+
+// Bitonic sort of win[0, P) (P a power of two), best key first: value bits descending, then flat ascending.  Every
+// thread of the block calls it.
+template <typename Entry>
+__device__ __forceinline__ void det_sort(Entry* win, unsigned P) {
+    for (unsigned kk = 2; kk <= P; kk <<= 1)
+        for (unsigned j = kk >> 1; j > 0; j >>= 1) {
+            for (unsigned i = threadIdx.x; i < P; i += blockDim.x) {
+                const unsigned x = i ^ j;
+                if (x > i) {
+                    const Entry a = win[i], b = win[x];
+                    const bool a_first = a.vbits > b.vbits || (a.vbits == b.vbits && a.flat < b.flat);
+                    if (((i & kk) == 0) != a_first) { win[i] = b; win[x] = a; }
+                }
+            }
+            __syncthreads();
+        }
+}
 
 // The merge of both detectors (this one and caf_cfar_merge_kernel).  Entry starts with (vbits, flat) and Out holds a
 // DetectOut, the whole record or its member det; fill(o, entry, used) writes the rest of the record.  With RATIO the
-// entries below min_ratio x the first are dropped.  Its shared arrays are declared here, in this order, not passed in
-// from the kernels: passing them in changes the merge kernels' generated code.
-template <typename T, bool RATIO, typename Entry, typename Out, typename Fill>
+// entries below min_ratio x the first are dropped.  With BLOCK the surface is a block whose row 0 is global row
+// row_offset, and doppler_idx is written as the global row.  Its shared arrays are declared here, in this order, not
+// passed in from the kernels: passing them in changes the merge kernels' generated code.
+template <typename T, bool RATIO, bool BLOCK = false, typename Entry, typename Out, typename Fill>
 __device__ __forceinline__ void det_merge(
         const T* __restrict__ surf, long long d, long long n, const double* __restrict__ freqs,
         const Entry* __restrict__ entries, long long cap, const unsigned long long* __restrict__ ctr, unsigned kmax,
-        double min_ratio, Out* __restrict__ out, unsigned long long* __restrict__ counts, Fill fill) {
+        double min_ratio, Out* __restrict__ out, unsigned long long* __restrict__ counts, Fill fill,
+        long long row_offset = 0) {
     __shared__ Entry win[kDetMaxK];
     __shared__ unsigned hist[256];
     __shared__ DetSelState sel;
@@ -325,19 +367,7 @@ __device__ __forceinline__ void det_merge(
     while (P < m) P <<= 1;
     for (unsigned i = m + tid; i < P; i += blockDim.x) win[i] = Entry{0ull, ~0ull};   // sorts after every candidate
     __syncthreads();
-    // bitonic sort, best key first
-    for (unsigned kk = 2; kk <= P; kk <<= 1)
-        for (unsigned j = kk >> 1; j > 0; j >>= 1) {
-            for (unsigned i = tid; i < P; i += blockDim.x) {
-                const unsigned x = i ^ j;
-                if (x > i) {
-                    const Entry a = win[i], b = win[x];
-                    const bool a_first = a.vbits > b.vbits || (a.vbits == b.vbits && a.flat < b.flat);
-                    if (((i & kk) == 0) != a_first) { win[i] = b; win[x] = a; }
-                }
-            }
-            __syncthreads();
-        }
+    det_sort(win, P);
     unsigned kept = m;
     if (RATIO) {
         const double v0 = m ? __longlong_as_double((long long)win[0].vbits) : 0.0;
@@ -365,7 +395,7 @@ __device__ __forceinline__ void det_merge(
             double fi = fr;
             if (df > 0.0) fi = __dadd_rn(fr, __dmul_rn(df, __dsub_rn(freqs[r + 1], fr)));
             else if (df < 0.0) fi = __dadd_rn(fr, __dmul_rn(df, __dsub_rn(fr, freqs[r - 1])));
-            e.value = v; e.freq_hz = fr; e.doppler_idx = (unsigned long long)r; e.delay_idx = (unsigned long long)k;
+            e.value = v; e.freq_hz = fr; e.doppler_idx = (unsigned long long)(BLOCK ? row_offset + r : r); e.delay_idx = (unsigned long long)k;
             e.lag_samples = __dadd_rn((double)(2 * k < n ? k : k - n), dk);
             e.freq_hz_interp = fi;
             fill(o, win[i], true);
@@ -385,6 +415,111 @@ __global__ void __launch_bounds__(kDetMergeThreads) caf_detect_merge_kernel(
         double min_ratio, DetectOut* __restrict__ out, unsigned long long* __restrict__ counts) {
     det_merge<T, true>(surf, d, n, freqs, entries, cap, ctr, kmax, min_ratio, out, counts,
                        [](DetectOut&, const DetEntry&, bool) {});
+}
+
+// one pair: a block of d rows whose row 0 is global row row_offset
+template <typename T>
+__global__ void __launch_bounds__(kDetMergeThreads) caf_detect_merge_rows_kernel(
+        const T* __restrict__ surf, long long d, long long n, const double* __restrict__ freqs,
+        const DetEntry* __restrict__ entries, long long cap, const unsigned long long* __restrict__ ctr, unsigned kmax,
+        double min_ratio, DetectOut* __restrict__ out, unsigned long long* __restrict__ counts, long long row_offset) {
+    det_merge<T, true, true>(surf, d, n, freqs, entries, cap, ctr, kmax, min_ratio, out, counts,
+                             [](DetectOut&, const DetEntry&, bool) {}, row_offset);
+}
+
+// ---- the merge across ranks ------------------------------------------------------------------------------------------
+// Each of `world` ranks detected on its own rows and holds its first counts[r] records, best first, with global
+// doppler_idx: lists[r * list_stride + i].  The global best kmax are among them, because a rank's list holds every one of
+// its local maxima that can be in the answer.  One CTA of kDetMergeThreads selects them by the key (value bits,
+// ~global flat index) -- the flat index as doppler_idx << 32 | delay_idx, which orders as doppler_idx * n + delay_idx
+// since both are below 2^31 -- sorts them, copies the whole records (no refit: they are already refined), applies
+// min_ratio against the global first when RATIO, and writes out[kmax] (unused slots: zero, doppler_idx ~0) and *count.
+// counts[r * count_stride] above kmax marks a rank that failed: its list is skipped.  *status (when given) is set to 1
+// when some rank failed, else 0.
+struct DetRankEntry { unsigned long long vbits, flat; unsigned pos; };
+
+template <bool RATIO, typename Rec>
+__device__ __forceinline__ void det_rank_merge(
+        const Rec* __restrict__ lists, long long list_stride, const unsigned long long* __restrict__ counts,
+        long long count_stride, int world, unsigned kmax, double min_ratio, Rec* __restrict__ out,
+        unsigned long long* __restrict__ count, int* __restrict__ status) {
+    __shared__ DetRankEntry win[kDetMaxK];
+    __shared__ unsigned hist[256];
+    __shared__ DetSelState sel;
+    __shared__ unsigned nwin, nkept, nvalid, nfailed;
+    const int tid = threadIdx.x;
+    if (tid == 0) { nwin = 0u; nkept = 0u; nvalid = 0u; nfailed = 0u; }
+    __syncthreads();
+    const long long N = (long long)world * kmax;
+    auto cnt_of = [&](long long r) {
+        const unsigned long long c = counts[r * count_stride];
+        return c > kmax ? 0ull : c;
+    };
+    // a slot past its rank's count gets key (0, 0): below every record (values are > 0) and never selected
+    auto key = [&](long long i, unsigned long long& h, unsigned long long& l) {
+        const long long r = i / kmax, k = i - r * kmax;
+        h = 0ull; l = 0ull;
+        if ((unsigned long long)k < cnt_of(r)) {
+            const DetectOut& e = det_rec_c(lists[r * list_stride + k]);
+            h = (unsigned long long)__double_as_longlong(e.value);
+            l = ~((e.doppler_idx << 32) | e.delay_idx);
+        }
+    };
+    for (int r = tid; r < world; r += blockDim.x) {
+        const unsigned long long c = counts[(long long)r * count_stride];
+        if (c > kmax) atomicAdd(&nfailed, 1u);
+        atomicAdd(&nvalid, (unsigned)cnt_of(r));
+    }
+    __syncthreads();
+    if (tid == 0 && status) *status = nfailed ? 1 : 0;
+    unsigned long long th = 0ull, tl = 0ull;
+    if (nvalid > kmax) { det_select_kth(key, N, kmax, hist, &sel); th = sel.oh; tl = sel.ol; }
+    __syncthreads();
+    for (long long i = tid; i < N; i += blockDim.x) {
+        unsigned long long h, l;
+        key(i, h, l);
+        if (h && det_key_ge(h, l, th, tl)) {
+            const long long r = i / kmax;
+            const unsigned s = atomicAdd(&nwin, 1u);
+            // only lists of overlapping rows (equal keys) could bring more than kmax
+            if (s < kmax) win[s] = DetRankEntry{h, ~l, (unsigned)(r * list_stride + (i - r * kmax))};
+        }
+    }
+    __syncthreads();
+    const unsigned m = nwin < kmax ? nwin : kmax;
+    unsigned P = 1;
+    while (P < m) P <<= 1;
+    for (unsigned i = m + tid; i < P; i += blockDim.x) win[i] = DetRankEntry{0ull, ~0ull, 0u};
+    __syncthreads();
+    det_sort(win, P);
+    unsigned kept = m;
+    if (RATIO) {
+        const double v0 = m ? __longlong_as_double((long long)win[0].vbits) : 0.0;
+        const double bar = min_ratio * v0;
+        unsigned mine = 0;
+        for (unsigned i = tid; i < m; i += blockDim.x)
+            if (!(__longlong_as_double((long long)win[i].vbits) < bar)) ++mine;
+        if (mine) atomicAdd(&nkept, mine);
+        __syncthreads();
+        kept = nkept;
+    }
+    for (unsigned i = tid; i < kmax; i += blockDim.x) {
+        if (i < kept) {
+            out[i] = lists[win[i].pos];
+        } else {
+            Rec o{};
+            det_rec(o).doppler_idx = ~0ull;
+            out[i] = o;
+        }
+    }
+    if (tid == 0) *count = kept;
+}
+
+__global__ void __launch_bounds__(kDetMergeThreads) caf_detect_rank_merge_kernel(
+        const DetectOut* __restrict__ lists, long long list_stride, const unsigned long long* __restrict__ counts,
+        long long count_stride, int world, unsigned kmax, double min_ratio, DetectOut* __restrict__ out,
+        unsigned long long* __restrict__ count, int* __restrict__ status) {
+    det_rank_merge<true>(lists, list_stride, counts, count_stride, world, kmax, min_ratio, out, count, status);
 }
 
 }  // namespace caf

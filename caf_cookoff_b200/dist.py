@@ -12,7 +12,7 @@ from typing import Tuple
 
 import numpy as np
 
-from . import _lib
+from . import _lib, api
 from .api import _check, peak_pack, peak_resolve
 
 
@@ -141,6 +141,114 @@ def peaks_as_tuples(words: np.ndarray):
     return [(float(w[i, 1:2].view(np.float64)[0]), int(w[i, 3])) for i in range(w.shape[0])]
 
 
+_FAILED = -2        # UINT64_MAX - 1 as int64: the failure mark of a rank's count (above any k_max), as in the library
+
+
+def _block_detect(detector: str, needle, haystack, freqs, fs: int, k_max: int, world: int, rank: int, *,
+                  guard_doppler: int, guard_delay: int, train_doppler: int, train_delay: int, os_rank, scale,
+                  min_ratio: float, handle):
+    """One rank's half of sharded detection: the halo'd block of its rows shard_bounds(d, world, rank) computed with
+    caf_b200_batch_*_dev from the same inputs every rank holds, then the block detector over the owned rows.  Returns
+    (records [k_max, 6 or 8] float64 tensor, count int64 tensor [1]) on the handle's device, complete.  The handle's
+    stream and torch's are not ordered with each other, so torch's is synchronised before the first launch (the inputs
+    as torch last wrote them, and buffers from torch's allocator that torch's pending work may still use) and the
+    handle's before the return (the block is freed on return)."""
+    import torch
+    if detector not in ("detect", "cfar", "cfar_os"):
+        raise ValueError("detector must be 'detect', 'cfar' or 'cfar_os'")
+    h = handle or api.default_handle()
+    f32 = needle.dtype == torch.complex64
+    l, d = int(needle.numel()), int(freqs.numel())
+    n = 2 * l
+    lo, hi = shard_bounds(d, world, rank)
+    H = api.halo_rows(detector, guard_doppler, 0 if detector == "detect" else train_doppler)
+    b_lo, b_hi = max(lo - H, 0), min(hi + H, d)
+    dev = needle.device
+    surf = torch.empty((b_hi - b_lo, n), dtype=torch.float32 if f32 else torch.float64, device=dev)
+    peak = torch.empty(4, dtype=torch.float64, device=dev)
+    out = torch.empty((k_max, 6 if detector == "detect" else 8), dtype=torch.float64, device=dev)
+    cnt = torch.empty(1, dtype=torch.int64, device=dev)
+    torch.cuda.current_stream(dev).synchronize()
+    try:
+        f_ptr = freqs.data_ptr() + 8 * b_lo
+        if b_hi > b_lo:
+            fn = getattr(_lib.load(), "caf_b200_batch_f32_dev" if f32 else "caf_b200_batch_f64_dev")
+            _check(fn(h.raw, needle.data_ptr(), haystack.data_ptr(), 1, l, f_ptr, b_hi - b_lo, int(fs), surf.data_ptr(),
+                      None, None, peak.data_ptr()))
+        args = (surf.data_ptr(), b_hi - b_lo, n, f_ptr, lo - b_lo, hi - b_lo, b_lo, d, k_max, out.data_ptr(),
+                cnt.data_ptr())
+        win = dict(guard_doppler=guard_doppler, guard_delay=guard_delay, f32=f32, handle=h)
+        if detector == "detect":
+            api.detect_rows_dev(*args, min_ratio=min_ratio, **win)
+        else:
+            N = api.cfar_train_cells(guard_doppler, guard_delay, train_doppler, train_delay)
+            win.update(train_doppler=train_doppler, train_delay=train_delay)
+            if detector == "cfar":
+                api.detect_cfar_rows_dev(*args, scale=api.cfar_scale(1e-6, N) if scale is None else scale, **win)
+            else:
+                os_rank = (3 * N + 3) // 4 if os_rank is None else os_rank
+                api.detect_cfar_os_rows_dev(*args, rank=os_rank,
+                                            scale=api.cfar_os_scale(1e-6, N, os_rank) if scale is None else scale, **win)
+    finally:
+        h.sync()                      # also when a call raised after the batch launch: surf dies here
+    return out, cnt
+
+
+def detect_sharded(detector: str, needle, haystack, freqs, fs: int, k_max: int, *, guard_doppler: int = 1,
+                   guard_delay: int = 1, train_doppler: int = 2, train_delay: int = 16, rank=None, scale=None,
+                   min_ratio: float = 0.0, handle=None, group=None):
+    """Detection on a row-sharded surface over torch.distributed (DESIGN.md section 12).  detector is "detect", "cfar" or
+    "cfar_os"; every rank passes the same CUDA tensors needle, haystack [l] (complex128, or complex64 for f32 surfaces)
+    and freqs [d] (float64, the whole grid).  Rank r computes rows shard_bounds(d, world, r) plus a halo of
+    api.halo_rows(...) rows, detects over its own rows, and ONE all_gather_into_tensor of the records and count feeds
+    the merge.  Every rank returns (records [k_max, 6] (detect) or [k_max, 8] float64 tensor, count int64 tensor [1])
+    equal bit for bit to the same detector on the whole surface.  rank and scale of the CFAR detectors default as in
+    DeviceSurface.detect_cfar / detect_cfar_os; min_ratio is detect's.  k_max and the window must be the same on every
+    rank.  A rank whose block detection raises still takes part in the gather, with a count above k_max as its failure
+    mark, and then re-raises; its peers skip its list and raise CafError with CAF_B200_EREMOTE (-7), as the library's
+    exchange does."""
+    import torch
+    import torch.distributed as dist
+    on = dist.is_available() and dist.is_initialized()
+    world, me = (dist.get_world_size(group), dist.get_rank(group)) if on else (1, 0)
+    h = handle or api.default_handle()
+    width = 6 if detector == "detect" else 8
+    failed = None
+    try:
+        out, cnt = _block_detect(detector, needle, haystack, freqs, fs, k_max, world, me, guard_doppler=guard_doppler,
+                                 guard_delay=guard_delay, train_doppler=train_doppler, train_delay=train_delay,
+                                 os_rank=rank, scale=scale, min_ratio=min_ratio, handle=h)
+        mine = torch.cat([out.view(torch.int64).reshape(-1), cnt])
+    except Exception as e:
+        if world == 1:
+            raise
+        failed = e                    # never leave the peers alone in the collective
+        mine = torch.zeros(k_max * width + 1, dtype=torch.int64, device=needle.device)
+        mine[-1] = _FAILED
+    if world > 1:
+        allw = torch.empty((world, mine.numel()), dtype=torch.int64, device=mine.device)
+        dist.all_gather_into_tensor(allw, mine, group=group)
+    else:
+        allw = mine.reshape(1, -1)
+    if failed is not None:
+        raise failed
+    lists = allw[:, :-1].contiguous()
+    counts = allw[:, -1].contiguous()
+    res = torch.empty((k_max, width), dtype=torch.float64, device=mine.device)
+    count = torch.empty(1, dtype=torch.int64, device=mine.device)
+    torch.cuda.current_stream(mine.device).synchronize()  # the gathered lists, before the library's stream reads them
+    if detector == "detect":
+        api.detect_merge_dev(lists.data_ptr(), counts.data_ptr(), world, k_max, res.data_ptr(), count.data_ptr(),
+                             min_ratio=min_ratio, handle=h)
+    else:
+        api.cfar_merge_dev(lists.data_ptr(), counts.data_ptr(), world, k_max, res.data_ptr(), count.data_ptr(), handle=h)
+    h.sync()
+    c = counts.cpu()
+    if bool(((c < 0) | (c > k_max)).any()):
+        raise api.CafError(-7, "a peer rank failed before the detection exchange")
+    return res, count
+
+
 class Comm:
     """The library's own NCCL communicator (caf_b200_comm_*): what a caller without torch.distributed (the Rust
     shim) uses.  The 128-byte NCCL id travels out of band; here through a small file any rank can read.
@@ -226,6 +334,38 @@ class Comm:
         vp = lambda x: C.c_void_p(x or None)
         _check(fn(self.handle.raw, self._c, vp(needle_dev), vp(hay_dev), int(l), vp(freqs_local_dev), int(d_local),
                   int(row_offset), int(fs), vp(surface_local_dev), vp(row_val_dev), vp(row_idx_dev), vp(peak_out_dev)))
+
+    def detect_sharded(self, detector: str, needle, haystack, freqs, fs: int, k_max: int, *, guard_doppler: int = 1,
+                       guard_delay: int = 1, train_doppler: int = 2, train_delay: int = 16, rank=None, scale=None,
+                       min_ratio: float = 0.0):
+        """dist.detect_sharded over this communicator: the halo'd block and the block detector on this rank, then
+        caf_b200_detect_allgather_dev / caf_b200_cfar_allgather_dev.  If this rank's block cannot be computed it still
+        enters the exchange with the failure mark (its peers raise CafError EREMOTE) and raises the local error."""
+        import ctypes as C
+        import torch
+        try:
+            out, cnt = _block_detect(detector, needle, haystack, freqs, fs, k_max, self.world, self.rank,
+                                     guard_doppler=guard_doppler, guard_delay=guard_delay, train_doppler=train_doppler,
+                                     train_delay=train_delay, os_rank=rank, scale=scale, min_ratio=min_ratio,
+                                     handle=self.handle)
+        except Exception:
+            if detector == "detect":
+                self._lib.caf_b200_detect_allgather_dev(self.handle.raw, self._c, None, None, int(k_max),
+                                                        float(min_ratio), None, None)
+            else:
+                self._lib.caf_b200_cfar_allgather_dev(self.handle.raw, self._c, None, None, int(k_max), None, None)
+            raise
+        res = torch.empty_like(out)
+        count = torch.empty(1, dtype=torch.int64, device=out.device)
+        torch.cuda.current_stream(out.device).synchronize()   # res / count from torch's allocator, as in _block_detect
+        vp = lambda t: C.c_void_p(t.data_ptr())
+        if detector == "detect":
+            _check(self._lib.caf_b200_detect_allgather_dev(self.handle.raw, self._c, vp(out), vp(cnt), int(k_max),
+                                                           float(min_ratio), vp(res), vp(count)))
+        else:
+            _check(self._lib.caf_b200_cfar_allgather_dev(self.handle.raw, self._c, vp(out), vp(cnt), int(k_max), vp(res),
+                                                         vp(count)))
+        return res, count
 
     def uses_p2p(self) -> bool:
         """True when the exchange is the one-kernel peer-memory mailbox (NVLink), False when it is ncclAllGather."""

@@ -340,6 +340,61 @@ int caf_b200_cfar_os_noise_f32_dev(caf_b200_handle h, const float* surface, size
                                    uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler,
                                    uint32_t train_delay, uint32_t rank, double* noise_out);
 
+/* ---- detection on row-sharded surfaces: each rank searches its rows with a halo, one merge gives the one-GPU answer --
+ * A rank owns global rows [lo, hi) of a surface of d_global rows (e.g. from caf_b200_comm_shard).  It computes a BLOCK of
+ * d_buf rows whose row 0 is global row row_offset and that covers its owned rows plus H rows on each side, clipped to the
+ * surface (the surface calls give bit-identical rows for any sub-grid, so nothing is exchanged for the halo).  In the
+ * block the owned rows are [row_lo, row_hi) = [lo - row_offset, hi - row_offset).  H is the depth of a detector's
+ * neighbourhood: max(guard_doppler, 1) for detect (window, equal-value rule, Doppler parabola) and
+ * max(guard_doppler + train_doppler, 1) for both CFAR detectors (their training rows).
+ * The *_rows_* calls run a detector over the owned rows only, reading the rest of the block as neighbourhood: every owned
+ * cell sees exactly what it sees on the whole surface, so its decision, refinement, noise and m are the whole-surface
+ * ones.  Records carry the GLOBAL row in doppler_idx; freq_hz and freq_hz_interp come from freqs_hz, the block's own grid
+ * (d_buf values).  The list is the rank's best k_max (detect: also cut at min_ratio x the rank's first, which never drops
+ * a record the global cut keeps).  p = 1; out [k_max] and count in device memory; two stream-ordered launches.
+ * Limits: each detector's own (with d = d_buf), and row_lo <= row_hi <= d_buf, row_offset + d_buf <= d_global <= 2^31,
+ * and at least H block rows above row_lo unless the block starts the surface (row_offset == 0), and below row_hi unless
+ * it ends the surface (row_offset + d_buf == d_global); anything else is CAF_B200_EINVAL and writes nothing.  An empty owned range
+ * (row_lo == row_hi: a rank may own no rows) needs no halo and gives count 0. */
+int caf_b200_detect_rows_f64_dev(caf_b200_handle h, const double* surface, size_t d_buf, size_t n, const double* freqs_hz,
+                                 size_t row_lo, size_t row_hi, uint64_t row_offset, size_t d_global, size_t k_max,
+                                 uint32_t guard_doppler, uint32_t guard_delay, double min_ratio, caf_b200_detection* out,
+                                 uint64_t* count);
+int caf_b200_detect_rows_f32_dev(caf_b200_handle h, const float* surface, size_t d_buf, size_t n, const double* freqs_hz,
+                                 size_t row_lo, size_t row_hi, uint64_t row_offset, size_t d_global, size_t k_max,
+                                 uint32_t guard_doppler, uint32_t guard_delay, double min_ratio, caf_b200_detection* out,
+                                 uint64_t* count);
+int caf_b200_detect_cfar_rows_f64_dev(caf_b200_handle h, const double* surface, size_t d_buf, size_t n,
+                                      const double* freqs_hz, size_t row_lo, size_t row_hi, uint64_t row_offset,
+                                      size_t d_global, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                      uint32_t train_doppler, uint32_t train_delay, double scale,
+                                      caf_b200_cfar_detection* out, uint64_t* count);
+int caf_b200_detect_cfar_rows_f32_dev(caf_b200_handle h, const float* surface, size_t d_buf, size_t n,
+                                      const double* freqs_hz, size_t row_lo, size_t row_hi, uint64_t row_offset,
+                                      size_t d_global, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                      uint32_t train_doppler, uint32_t train_delay, double scale,
+                                      caf_b200_cfar_detection* out, uint64_t* count);
+int caf_b200_detect_cfar_os_rows_f64_dev(caf_b200_handle h, const double* surface, size_t d_buf, size_t n,
+                                         const double* freqs_hz, size_t row_lo, size_t row_hi, uint64_t row_offset,
+                                         size_t d_global, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                         uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                         caf_b200_cfar_detection* out, uint64_t* count);
+int caf_b200_detect_cfar_os_rows_f32_dev(caf_b200_handle h, const float* surface, size_t d_buf, size_t n,
+                                         const double* freqs_hz, size_t row_lo, size_t row_hi, uint64_t row_offset,
+                                         size_t d_global, size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                         uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                         caf_b200_cfar_detection* out, uint64_t* count);
+/* The merge: lists [world][k_max] and counts [world] (device memory) hold each rank's block records and count, from
+ * DISJOINT owned rows.  The global best k_max are among them.  One stream-ordered launch (one CTA) selects them by value
+ * descending, then global flat index doppler_idx * n + delay_idx ascending, copies the whole records (no refit), applies
+ * min_ratio against the global first (detect only) and writes out [k_max] (device; unused slots as above) and *count
+ * (device): the records and count of the same detector run on the whole surface, bit for bit.  A count above k_max marks
+ * a rank that failed: its list is skipped.  For callers with their own collective layer (torch.distributed).
+ * Limits: 1 <= k_max <= 1024, 1 <= world <= 65536, 0 <= min_ratio <= 1, no null pointer; else CAF_B200_EINVAL. */
+int caf_b200_detect_merge_dev(caf_b200_handle h, const caf_b200_detection* lists, const uint64_t* counts, size_t world,
+                              size_t k_max, double min_ratio, caf_b200_detection* out, uint64_t* count);
+int caf_b200_cfar_merge_dev(caf_b200_handle h, const caf_b200_cfar_detection* lists, const uint64_t* counts, size_t world,
+                            size_t k_max, caf_b200_cfar_detection* out, uint64_t* count);
 /* ---- the sibling programs' layouts of the same surface (SURVEY.md section 8(f)4) -------------------
  * The reference's Go and Python programs compute this correlation with the operands swapped and keep the
  * magnitude |xcor| (cmplx.Abs, np.abs) where the Rust crate keeps |xcor|^2 (norm_sqr):
@@ -425,6 +480,17 @@ int caf_b200_surface_sharded_f64(caf_b200_handle h, caf_b200_comm c, const caf_c
 int caf_b200_surface_sharded_f32(caf_b200_handle h, caf_b200_comm c, const caf_c64* needle, const caf_c64* haystack,
                                  size_t l, const double* freqs_hz, size_t d, uint32_t fs,
                                  float* surface_local, caf_b200_peak* peak);
+/* Detection on row-sharded surfaces (caf_b200_detect_rows_* and the merge, above) across this communicator's ranks. */
+/* The exchange over the library's communicator (caf_b200_comm): ONE ncclAllGather of this rank's k_max records and
+ * count (local, local_count: device memory) on the handle's stream, then the merge into out / count (device memory) on
+ * every rank; synchronous.  k_max (and min_ratio) must be the same on every rank; a bad one fails on every rank before
+ * the collective.  A rank that passes a null pointer still enters the collective with a failure mark and returns
+ * CAF_B200_EINVAL; its peers skip its list and return CAF_B200_EREMOTE. */
+int caf_b200_detect_allgather_dev(caf_b200_handle h, caf_b200_comm c, const caf_b200_detection* local,
+                                  const uint64_t* local_count, size_t k_max, double min_ratio, caf_b200_detection* out,
+                                  uint64_t* count);
+int caf_b200_cfar_allgather_dev(caf_b200_handle h, caf_b200_comm c, const caf_b200_cfar_detection* local,
+                                const uint64_t* local_count, size_t k_max, caf_b200_cfar_detection* out, uint64_t* count);
 
 #ifdef __cplusplus
 }

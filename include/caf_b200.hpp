@@ -273,6 +273,66 @@ struct GoSibling {
     }
 };
 
+// Detection on the owned rows [row_lo, row_hi) of a device block of d_buf rows whose row 0 is global row row_offset of a
+// d_global-row surface, and the merge of the ranks' lists (caf_b200.h: caf_b200_detect_rows_* ... caf_b200_cfar_merge_dev).
+// Device pointers, asynchronous on the calling thread's handle.
+inline void detect_rows_dev(const double* surface, std::size_t d_buf, std::size_t n, const double* freqs_hz,
+                            std::size_t row_lo, std::size_t row_hi, uint64_t row_offset, std::size_t d_global,
+                            std::size_t k_max, uint32_t guard_doppler, uint32_t guard_delay, double min_ratio,
+                            Detection* out, uint64_t* count) {
+    check(caf_b200_detect_rows_f64_dev(thread_handle(), surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset, d_global,
+                                       k_max, guard_doppler, guard_delay, min_ratio, out, count));
+}
+inline void detect_rows_dev(const float* surface, std::size_t d_buf, std::size_t n, const double* freqs_hz,
+                            std::size_t row_lo, std::size_t row_hi, uint64_t row_offset, std::size_t d_global,
+                            std::size_t k_max, uint32_t guard_doppler, uint32_t guard_delay, double min_ratio,
+                            Detection* out, uint64_t* count) {
+    check(caf_b200_detect_rows_f32_dev(thread_handle(), surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset, d_global,
+                                       k_max, guard_doppler, guard_delay, min_ratio, out, count));
+}
+inline void detect_cfar_rows_dev(const double* surface, std::size_t d_buf, std::size_t n, const double* freqs_hz,
+                                 std::size_t row_lo, std::size_t row_hi, uint64_t row_offset, std::size_t d_global,
+                                 std::size_t k_max, uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler,
+                                 uint32_t train_delay, double scale, CfarDetection* out, uint64_t* count) {
+    check(caf_b200_detect_cfar_rows_f64_dev(thread_handle(), surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset,
+                                            d_global, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale,
+                                            out, count));
+}
+inline void detect_cfar_rows_dev(const float* surface, std::size_t d_buf, std::size_t n, const double* freqs_hz,
+                                 std::size_t row_lo, std::size_t row_hi, uint64_t row_offset, std::size_t d_global,
+                                 std::size_t k_max, uint32_t guard_doppler, uint32_t guard_delay, uint32_t train_doppler,
+                                 uint32_t train_delay, double scale, CfarDetection* out, uint64_t* count) {
+    check(caf_b200_detect_cfar_rows_f32_dev(thread_handle(), surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset,
+                                            d_global, k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale,
+                                            out, count));
+}
+inline void detect_cfar_os_rows_dev(const double* surface, std::size_t d_buf, std::size_t n, const double* freqs_hz,
+                                    std::size_t row_lo, std::size_t row_hi, uint64_t row_offset, std::size_t d_global,
+                                    std::size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                    uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                    CfarDetection* out, uint64_t* count) {
+    check(caf_b200_detect_cfar_os_rows_f64_dev(thread_handle(), surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset,
+                                               d_global, k_max, guard_doppler, guard_delay, train_doppler, train_delay,
+                                               rank, scale, out, count));
+}
+inline void detect_cfar_os_rows_dev(const float* surface, std::size_t d_buf, std::size_t n, const double* freqs_hz,
+                                    std::size_t row_lo, std::size_t row_hi, uint64_t row_offset, std::size_t d_global,
+                                    std::size_t k_max, uint32_t guard_doppler, uint32_t guard_delay,
+                                    uint32_t train_doppler, uint32_t train_delay, uint32_t rank, double scale,
+                                    CfarDetection* out, uint64_t* count) {
+    check(caf_b200_detect_cfar_os_rows_f32_dev(thread_handle(), surface, d_buf, n, freqs_hz, row_lo, row_hi, row_offset,
+                                               d_global, k_max, guard_doppler, guard_delay, train_doppler, train_delay,
+                                               rank, scale, out, count));
+}
+inline void detect_merge_dev(const Detection* lists, const uint64_t* counts, std::size_t world, std::size_t k_max,
+                             double min_ratio, Detection* out, uint64_t* count) {
+    check(caf_b200_detect_merge_dev(thread_handle(), lists, counts, world, k_max, min_ratio, out, count));
+}
+inline void cfar_merge_dev(const CfarDetection* lists, const uint64_t* counts, std::size_t world, std::size_t k_max,
+                           CfarDetection* out, uint64_t* count) {
+    check(caf_b200_cfar_merge_dev(thread_handle(), lists, counts, world, k_max, out, count));
+}
+
 // Doppler rows sharded over one process per GPU (mod.rs:185's par_iter with GPUs for workers): the library's own NCCL
 // communicator.  Rank 0 makes the 128-byte id (ShardedCaf::unique_id) and hands it to the other ranks out of band.
 class ShardedCaf {
@@ -306,6 +366,15 @@ public:
                                            reinterpret_cast<const caf_c128*>(haystack.data()), needle.size(), freqs_hz.data(),
                                            freqs_hz.size(), fs, rows.data(), &pk));
         return {std::move(rows), {pk.freq_hz, (std::size_t)pk.delay_idx}};
+    }
+    // the exchange of the ranks' block detections (device records and counts; caf_b200_*_allgather_dev)
+    void detect_allgather_dev(const Detection* local, const uint64_t* local_count, std::size_t k_max, double min_ratio,
+                              Detection* out, uint64_t* count) const {
+        check(caf_b200_detect_allgather_dev(thread_handle(), comm_, local, local_count, k_max, min_ratio, out, count));
+    }
+    void cfar_allgather_dev(const CfarDetection* local, const uint64_t* local_count, std::size_t k_max,
+                            CfarDetection* out, uint64_t* count) const {
+        check(caf_b200_cfar_allgather_dev(thread_handle(), comm_, local, local_count, k_max, out, count));
     }
 };
 

@@ -54,6 +54,18 @@ impl DeviceSurface {
         out.truncate(count);
         out
     }
+    fn detect_cfar_os(&self, k_max: usize, guard_doppler: u32, guard_delay: u32, train_doppler: u32, train_delay: u32,
+                      rank: u32, scale: f64) -> Vec<ffi::caf_b200_cfar_detection> {
+        assert!(std::thread::current().id() == self.owner, "detect_cfar_os: a surface is searched on the thread that created it");
+        let mut out = vec![ffi::caf_b200_cfar_detection::default(); k_max];
+        let mut count = 0usize;
+        ffi::check(unsafe {
+            ffi::caf_b200_surface_detect_cfar_os(self.raw, k_max, guard_doppler, guard_delay, train_doppler, train_delay,
+                                                 rank, scale, out.as_mut_ptr(), &mut count)
+        });
+        out.truncate(count);
+        out
+    }
     fn fused_peak(&self) -> ffi::caf_b200_peak {
         let mut pk = ffi::caf_b200_peak::default();
         ffi::check(unsafe { ffi::caf_b200_surface_find_peak(self.raw, &mut pk) });
@@ -162,6 +174,15 @@ impl CafB200 {
             && arr.iter().enumerate().all(|(i, r)| r.row == i && Arc::ptr_eq(&r.surface, &first.surface));
         assert!(whole, "detect_cfar needs the untouched rows of one caf_surface call");
         first.surface.detect_cfar(k_max, guard_doppler, guard_delay, train_doppler, train_delay, scale)
+    }
+    /// OS-CFAR detection on the surface behind `arr`: as detect_cfar, against the rank-th smallest training cell
+    pub fn detect_cfar_os(arr: &[CafSurfaceRow], k_max: usize, guard_doppler: u32, guard_delay: u32, train_doppler: u32,
+                          train_delay: u32, rank: u32, scale: f64) -> Vec<ffi::caf_b200_cfar_detection> {
+        let first = arr.first().expect("detect_cfar_os needs the untouched rows of one caf_surface call");
+        let whole = arr.len() == first.surface.rows
+            && arr.iter().enumerate().all(|(i, r)| r.row == i && Arc::ptr_eq(&r.surface, &first.surface));
+        assert!(whole, "detect_cfar_os needs the untouched rows of one caf_surface call");
+        first.surface.detect_cfar_os(k_max, guard_doppler, guard_delay, train_doppler, train_delay, rank, scale)
     }
 }
 

@@ -91,6 +91,59 @@ extern "C" {
     pub fn caf_b200_cfar_noise_f32_dev(h: caf_b200_handle, surface: *const f32, p: usize, d: usize, n: usize,
                                        guard_doppler: u32, guard_delay: u32, train_doppler: u32, train_delay: u32,
                                        noise_out: *mut f64) -> c_int;
+    // OS-CFAR detection: the same against the rank-th smallest training cell, and its dense noise map
+    pub fn caf_b200_surface_detect_cfar_os(s: caf_b200_surface, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                           train_doppler: u32, train_delay: u32, rank: u32, scale: f64,
+                                           out: *mut caf_b200_cfar_detection, count: *mut usize) -> c_int;
+    pub fn caf_b200_detect_cfar_os_f64_dev(h: caf_b200_handle, surface: *const f64, p: usize, d: usize, n: usize,
+                                           freqs_hz: *const f64, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                           train_doppler: u32, train_delay: u32, rank: u32, scale: f64,
+                                           out: *mut caf_b200_cfar_detection, counts: *mut u64) -> c_int;
+    pub fn caf_b200_detect_cfar_os_f32_dev(h: caf_b200_handle, surface: *const f32, p: usize, d: usize, n: usize,
+                                           freqs_hz: *const f64, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                           train_doppler: u32, train_delay: u32, rank: u32, scale: f64,
+                                           out: *mut caf_b200_cfar_detection, counts: *mut u64) -> c_int;
+    pub fn caf_b200_cfar_os_noise_f64_dev(h: caf_b200_handle, surface: *const f64, p: usize, d: usize, n: usize,
+                                          guard_doppler: u32, guard_delay: u32, train_doppler: u32, train_delay: u32,
+                                          rank: u32, noise_out: *mut f64) -> c_int;
+    pub fn caf_b200_cfar_os_noise_f32_dev(h: caf_b200_handle, surface: *const f32, p: usize, d: usize, n: usize,
+                                          guard_doppler: u32, guard_delay: u32, train_doppler: u32, train_delay: u32,
+                                          rank: u32, noise_out: *mut f64) -> c_int;
+    // detection on the owned rows of a row block of a sharded surface (records carry global rows), and the merge of
+    // the ranks' lists (device memory)
+    pub fn caf_b200_detect_rows_f64_dev(h: caf_b200_handle, surface: *const f64, d_buf: usize, n: usize,
+                                        freqs_hz: *const f64, row_lo: usize, row_hi: usize, row_offset: u64,
+                                        d_global: usize, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                        min_ratio: f64, out: *mut caf_b200_detection, count: *mut u64) -> c_int;
+    pub fn caf_b200_detect_rows_f32_dev(h: caf_b200_handle, surface: *const f32, d_buf: usize, n: usize,
+                                        freqs_hz: *const f64, row_lo: usize, row_hi: usize, row_offset: u64,
+                                        d_global: usize, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                        min_ratio: f64, out: *mut caf_b200_detection, count: *mut u64) -> c_int;
+    pub fn caf_b200_detect_cfar_rows_f64_dev(h: caf_b200_handle, surface: *const f64, d_buf: usize, n: usize,
+                                             freqs_hz: *const f64, row_lo: usize, row_hi: usize, row_offset: u64,
+                                             d_global: usize, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                             train_doppler: u32, train_delay: u32, scale: f64,
+                                             out: *mut caf_b200_cfar_detection, count: *mut u64) -> c_int;
+    pub fn caf_b200_detect_cfar_rows_f32_dev(h: caf_b200_handle, surface: *const f32, d_buf: usize, n: usize,
+                                             freqs_hz: *const f64, row_lo: usize, row_hi: usize, row_offset: u64,
+                                             d_global: usize, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                             train_doppler: u32, train_delay: u32, scale: f64,
+                                             out: *mut caf_b200_cfar_detection, count: *mut u64) -> c_int;
+    pub fn caf_b200_detect_cfar_os_rows_f64_dev(h: caf_b200_handle, surface: *const f64, d_buf: usize, n: usize,
+                                                freqs_hz: *const f64, row_lo: usize, row_hi: usize, row_offset: u64,
+                                                d_global: usize, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                                train_doppler: u32, train_delay: u32, rank: u32, scale: f64,
+                                                out: *mut caf_b200_cfar_detection, count: *mut u64) -> c_int;
+    pub fn caf_b200_detect_cfar_os_rows_f32_dev(h: caf_b200_handle, surface: *const f32, d_buf: usize, n: usize,
+                                                freqs_hz: *const f64, row_lo: usize, row_hi: usize, row_offset: u64,
+                                                d_global: usize, k_max: usize, guard_doppler: u32, guard_delay: u32,
+                                                train_doppler: u32, train_delay: u32, rank: u32, scale: f64,
+                                                out: *mut caf_b200_cfar_detection, count: *mut u64) -> c_int;
+    pub fn caf_b200_detect_merge_dev(h: caf_b200_handle, lists: *const caf_b200_detection, counts: *const u64,
+                                     world: usize, k_max: usize, min_ratio: f64, out: *mut caf_b200_detection,
+                                     count: *mut u64) -> c_int;
+    pub fn caf_b200_cfar_merge_dev(h: caf_b200_handle, lists: *const caf_b200_cfar_detection, counts: *const u64,
+                                   world: usize, k_max: usize, out: *mut caf_b200_cfar_detection, count: *mut u64) -> c_int;
     // read_file_c64 straight onto the device, and device memory for callers without a CUDA runtime of their own
     pub fn caf_b200_load_c64_dev_f64(h: caf_b200_handle, path: *const c_char, first_sample: usize, max_samples: usize,
                                      dev_out: *mut *mut Complex64, n_out: *mut usize) -> c_int;
@@ -115,6 +168,12 @@ extern "C" {
     pub fn caf_b200_surface_sharded_f64(h: caf_b200_handle, c: caf_b200_comm, needle: *const Complex64,
                                         haystack: *const Complex64, l: usize, freqs_hz: *const f64, d: usize, fs: u32,
                                         surface_local: *mut f64, peak: *mut caf_b200_peak) -> c_int;
+    pub fn caf_b200_detect_allgather_dev(h: caf_b200_handle, c: caf_b200_comm, local: *const caf_b200_detection,
+                                         local_count: *const u64, k_max: usize, min_ratio: f64,
+                                         out: *mut caf_b200_detection, count: *mut u64) -> c_int;
+    pub fn caf_b200_cfar_allgather_dev(h: caf_b200_handle, c: caf_b200_comm, local: *const caf_b200_cfar_detection,
+                                       local_count: *const u64, k_max: usize, out: *mut caf_b200_cfar_detection,
+                                       count: *mut u64) -> c_int;
 }
 
 #[repr(C)]

@@ -91,3 +91,55 @@ for forced in (None, "0"):
     run_checks(comm)
     comm.close()
 print(f"rank {rank}/{world}: rows ok, global peak (69.0 Hz, delay 202, row 338) via the library's NCCL communicator; exchange transports exercised: {transports}", flush=True)
+
+
+# Sharded detection: every rank's merged list must be the list rank 0 gets from detecting the whole surface on one GPU,
+# through the library's communicator (Comm.detect_sharded) and through torch.distributed (dist.detect_sharded).
+import torch.distributed as tdist
+from caf_cookoff_b200 import api
+from caf_cookoff_b200.dist import detect_sharded
+tdist.init_process_group("nccl", device_id=torch.device("cuda", local))
+comm = Comm(h, world, rank, id_path + "_detect")
+nd = torch.from_numpy(needle).cuda(); hd = torch.from_numpy(hay).cuda(); fd = torch.from_numpy(freqs.copy()).cuda()
+S = torch.empty((freqs.size, 8192), dtype=torch.float64, device="cuda")
+torch.cuda.synchronize()
+assert h._lib.caf_b200_batch_f64_dev(h.raw, nd.data_ptr(), hd.data_ptr(), 1, 4096, fd.data_ptr(), freqs.size, 48000,
+                                     S.data_ptr(), None, None, None) == 0
+kw = dict(guard_doppler=2, guard_delay=2, train_doppler=4, train_delay=16)
+for det in ("detect", "cfar", "cfar_os"):
+    out = torch.empty((16, 6 if det == "detect" else 8), dtype=torch.float64, device="cuda")
+    cnt = torch.empty(1, dtype=torch.int64, device="cuda")
+    N = api.cfar_train_cells(2, 2, 4, 16)
+    args = (S.data_ptr(), 1, freqs.size, 8192, fd.data_ptr(), 16, out.data_ptr(), cnt.data_ptr())
+    if det == "detect":
+        api.detect_dev(*args, guard_doppler=2, guard_delay=2, handle=h)
+    elif det == "cfar":
+        api.detect_cfar_dev(*args, scale=api.cfar_scale(1e-6, N), handle=h, **kw)
+    else:
+        rk = (3 * N + 3) // 4
+        api.detect_cfar_os_dev(*args, rank=rk, scale=api.cfar_os_scale(1e-6, N, rk), handle=h, **kw)
+    h.sync()
+    want = torch.cat([out.view(torch.int64).reshape(-1), cnt])
+    ref = want.clone()
+    tdist.broadcast(ref, 0)                                   # rank 0's whole-surface list
+    assert torch.equal(want, ref), "the whole-surface call differs between ranks"
+    args = (det, nd, hd, fd, 48000, 16)
+    for name, fn in (("Comm", comm.detect_sharded), ("torch.distributed", detect_sharded)):
+        res, c = fn(*args, **(kw if det != "detect" else dict(guard_doppler=2, guard_delay=2)))
+        got = torch.cat([res.view(torch.int64).reshape(-1), c])
+        assert torch.equal(got, ref), (det, name, int(c[0]), int(ref[-1]))
+# a rank whose block detection is refused (a window beyond the limits) still enters the exchange; its peers get EREMOTE
+# (through the library's communicator and through torch.distributed alike)
+from caf_cookoff_b200.api import CafError
+bad = world > 1 and rank == world - 1
+for fn in (comm.detect_sharded, detect_sharded):
+    try:
+        fn("cfar", nd, hd, fd, 48000, 16, guard_doppler=2, guard_delay=2, train_doppler=40 if bad else 4,
+           train_delay=16)
+        status = 0
+    except CafError as e:
+        status = e.status
+    assert status == (-1 if bad else (-7 if world > 1 else 0)), (fn, status)
+comm.close()
+tdist.destroy_process_group()
+print(f"rank {rank}/{world}: sharded detect / CA-CFAR / OS-CFAR equal the whole-surface lists of rank 0", flush=True)
