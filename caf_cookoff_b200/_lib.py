@@ -176,6 +176,10 @@ SYMBOLS = {
     "caf_b200_cfar_merge_dev": (_int, [_vp, _vp, _vp, _sz, _sz, _vp, _vp]),
     "caf_b200_detect_allgather_dev": (_int, [_vp, _vp, _vp, _vp, _sz, _dbl, _vp, _vp]),
     "caf_b200_cfar_allgather_dev": (_int, [_vp, _vp, _vp, _vp, _sz, _vp, _vp]),
+    "caf_b200_integrate_f64_dev": (_int, _batch),
+    "caf_b200_integrate_f32_dev": (_int, _batch),
+    "caf_b200_surface_create_integrated_f64": (_int, [_vp, _vp, _vp, _sz, _sz, _vp, _sz, _u32, C.POINTER(_vp)]),
+    "caf_b200_surface_create_integrated_f32": (_int, [_vp, _vp, _vp, _sz, _sz, _vp, _sz, _u32, C.POINTER(_vp)]),
 }
 
 _lib = None

@@ -12,6 +12,7 @@ All arithmetic happens in libcaf_b200.so on the GPU — this module never comput
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -263,7 +264,13 @@ class XcorF32(Xcor):
 
 class DeviceSurface:
     """A surface kept in device memory (caf_b200_surface_create_*): find_peak and row peaks come back at once, rows
-    cross PCIe only when fetched, and detect() searches the surface where it lies."""
+    cross PCIe only when fetched, and detect() searches the surface where it lies.
+
+    `looks` is how many segments' |xcor|^2 surfaces each cell sums: 1 for a surface of one pair, K for
+    DeviceSurface.integrate over K segments.  The CFAR detectors' default thresholds follow it."""
+
+    looks = 1
+    _rdt = None                                  # fetch_rows' dtype when it is not the variant's (integrated: float64)
 
     def __init__(self, needle, haystack, freqs_hz, fs: int, *, variant=_Variant, handle: Optional[Handle] = None):
         n_ = np.ascontiguousarray(needle, dtype=variant.cdt).ravel()
@@ -278,9 +285,38 @@ class DeviceSurface:
         fn = getattr(self._lib, "caf_b200_surface_create_" + variant.sfx)
         _check(fn(self.handle.raw, _ptr(n_), _ptr(h_), n_.size, _ptr(f_), f_.size, int(fs), C.byref(self._s)))
         self.freqs_hz = f_
+        self._read_shape()
+
+    def _read_shape(self):
         rows, cells = C.c_size_t(), C.c_size_t()
         _check(self._lib.caf_b200_surface_shape(self._s, C.byref(rows), C.byref(cells)))
         self.shape = (rows.value, cells.value)
+
+    @classmethod
+    def integrate(cls, needles, haystacks, freqs_hz, fs: int, *, variant=_Variant,
+                  handle: Optional[Handle] = None) -> "DeviceSurface":
+        """caf_b200_surface_create_integrated_*: needles, haystacks [K, L] (K segment pairs; a capture cut into consecutive
+        segments is capture[:K * L].reshape(K, L)).  The surface object holds S = the cell-by-cell sum, in double and in
+        ascending k, of the K segments' |xcor|^2 surfaces, for either input precision (fetch_rows gives float64), with
+        looks = K.  find_peak, row peaks and the detectors work on it as on any surface object."""
+        n_ = np.ascontiguousarray(needles, dtype=variant.cdt)
+        h_ = np.ascontiguousarray(haystacks, dtype=variant.cdt)
+        f_ = np.ascontiguousarray(freqs_hz, dtype=np.float64).ravel()
+        if n_.shape != h_.shape or n_.ndim != 2:
+            raise CafPanic("needles and haystacks must both be [K, L] (xcor_rustfft.rs:54-55)")
+        self = cls.__new__(cls)
+        self.handle = handle or default_handle()
+        self.variant = variant
+        self._lib = _lib.load()
+        self._s = C.c_void_p()
+        k, l = n_.shape
+        fn = getattr(self._lib, "caf_b200_surface_create_integrated_" + variant.sfx)
+        _check(fn(self.handle.raw, _ptr(n_), _ptr(h_), k, l, _ptr(f_), f_.size, int(fs), C.byref(self._s)))
+        self.freqs_hz = f_
+        self.looks = int(k)
+        self._rdt = np.float64
+        self._read_shape()
+        return self
 
     @property
     def raw(self):
@@ -293,7 +329,7 @@ class DeviceSurface:
 
     def fetch_rows(self, row0: int = 0, count: Optional[int] = None) -> np.ndarray:
         count = self.shape[0] - row0 if count is None else count
-        out = np.empty((count, self.shape[1]), dtype=self.variant.rdt)
+        out = np.empty((count, self.shape[1]), dtype=self._rdt or self.variant.rdt)
         _check(self._lib.caf_b200_surface_fetch_rows(self._s, int(row0), int(count), _ptr(out)))
         return out
 
@@ -310,10 +346,11 @@ class DeviceSurface:
     def detect_cfar(self, k_max: int, guard_doppler: int = 1, guard_delay: int = 1, train_doppler: int = 2,
                     train_delay: int = 16, scale: Optional[float] = None) -> List[_lib.CfarDetection]:
         """caf_b200_surface_detect_cfar: the local maxima that exceed scale x their local noise estimate, best first (only
-        the `count` valid records; possibly none).  scale defaults to cfar_scale(1e-6, cfar_train_cells(...)).  Same
-        handle rule as detect()."""
+        the `count` valid records; possibly none).  scale defaults to cfar_scale(1e-6, cfar_train_cells(...),
+        looks=self.looks).  Same handle rule as detect()."""
         if scale is None:
-            scale = cfar_scale(1e-6, cfar_train_cells(guard_doppler, guard_delay, train_doppler, train_delay))
+            scale = cfar_scale(1e-6, cfar_train_cells(guard_doppler, guard_delay, train_doppler, train_delay),
+                               looks=self.looks)
         out = (_lib.CfarDetection * max(int(k_max), 1))()
         count = C.c_size_t()
         _check(self._lib.caf_b200_surface_detect_cfar(self._s, int(k_max), int(guard_doppler), int(guard_delay),
@@ -326,7 +363,12 @@ class DeviceSurface:
                        scale: Optional[float] = None) -> List[_lib.CfarDetection]:
         """caf_b200_surface_detect_cfar_os: as detect_cfar, against the rank-th smallest training cell (scaled to the
         cell's training cells) instead of their mean.  rank defaults to ceil(3N / 4) and scale to
-        cfar_os_scale(1e-6, N, rank), N = cfar_train_cells(...).  Same handle rule as detect()."""
+        cfar_os_scale(1e-6, N, rank), N = cfar_train_cells(...).  That scale assumes exponential cells; on an integrated
+        surface (looks > 1) no closed form exists, so scale must be given there (ValueError otherwise).  Same handle rule
+        as detect()."""
+        if scale is None and self.looks > 1:
+            raise ValueError("detect_cfar_os on a surface of %d looks needs an explicit scale: cfar_os_scale assumes one "
+                             "look (exponential cells)" % self.looks)
         N = cfar_train_cells(guard_doppler, guard_delay, train_doppler, train_delay)
         if rank is None:
             rank = (3 * N + 3) // 4
@@ -369,19 +411,52 @@ def cfar_train_cells(guard_doppler: int, guard_delay: int, train_doppler: int, t
     return (2 * R + 1) * (2 * Cd + 1) - (2 * guard_doppler + 1) * (2 * guard_delay + 1)
 
 
-def cfar_scale(pfa: float, train_cells: int) -> float:
-    """The CA-CFAR threshold factor alpha = N (Pfa^(-1/N) - 1) for N training cells.
+def cfar_scale(pfa: float, train_cells: int, looks: int = 1) -> float:
+    """The CA-CFAR threshold factor alpha for N training cells of surfaces that sum `looks` segments each.
 
-    For N i.i.d. exponential training cells (|.|^2 of complex Gaussian noise) and a test cell of the same law,
-    P(v > alpha * mean) = (1 + alpha / N)^-N = Pfa.  That is the false-alarm probability of the threshold test alone,
-    before the local-maximum rule, at a cell with all N training cells; edge rows have fewer, and the correlation a CAF
-    puts between neighbouring cells is not modelled.  Pure host arithmetic."""
-    pfa, n = float(pfa), int(train_cells)
+    looks = 1: for N i.i.d. exponential training cells (|.|^2 of complex Gaussian noise) and a test cell of the same law,
+    P(v > alpha * mean) = (1 + alpha / N)^-N = Pfa, so alpha = N (Pfa^(-1/N) - 1).
+    looks = K (DeviceSurface.integrate over K segments): every cell of noise is the sum of K independent exponential cells,
+    Gamma(K), and with t = alpha / N, P(v > alpha * mean) = sum_{i=0}^{K-1} C(NK + i - 1, i) t^i (1 + t)^-(NK + i), the
+    exceedance of a Gamma(K) cell over the mean of N Gamma(K) cells; it is solved for alpha by bisection on logarithms
+    (K = 1 gives the closed form above, which is what looks = 1 returns).
+    Either way that is the false-alarm probability of the threshold test alone, before the local-maximum rule, at a cell
+    with all N training cells; edge rows have fewer, and the correlation a CAF puts between neighbouring cells is not
+    modelled.  Pure host arithmetic."""
+    pfa, n, k = float(pfa), int(train_cells), int(looks)
     if not 0.0 < pfa < 1.0:
         raise ValueError("pfa must be in (0, 1)")
     if n < 1:
         raise ValueError("train_cells must be >= 1")
-    return n * (pfa ** (-1.0 / n) - 1.0)
+    if k < 1 or k != looks:
+        raise ValueError("looks must be a whole number >= 1")
+    if k == 1:
+        return n * (pfa ** (-1.0 / n) - 1.0)
+    target = math.log(pfa)
+    lo, hi = 0.0, n * (pfa ** (-1.0 / n) - 1.0)      # P(0) = 1 > Pfa
+    while cfar_log_pfa(hi, n, k) >= target:
+        lo, hi = hi, 2.0 * hi
+    while True:
+        mid = 0.5 * (lo + hi)
+        if mid <= lo or mid >= hi:
+            return hi
+        if cfar_log_pfa(mid, n, k) >= target:
+            lo = mid
+        else:
+            hi = mid
+
+
+def cfar_log_pfa(scale: float, train_cells: int, looks: int = 1) -> float:
+    """log P(v > scale * mean) for a Gamma(looks) test cell v over the mean of train_cells Gamma(looks) cells, i.e. the
+    log of sum_{i<K} C(NK + i - 1, i) t^i (1 + t)^-(NK + i), t = scale / N, as a log-sum-exp (cfar_scale solves it)."""
+    n, k, t = int(train_cells), int(looks), float(scale) / int(train_cells)
+    m = n * k
+    if t == 0.0:
+        return 0.0
+    lt, l1t, lgm = math.log(t), math.log1p(t), math.lgamma(m)
+    terms = [math.lgamma(m + i) - math.lgamma(i + 1) - lgm + i * lt - (m + i) * l1t for i in range(k)]
+    top = max(terms)
+    return top + math.log(sum(math.exp(x - top) for x in terms))
 
 
 def detect_cfar_dev(surface_ptr: int, p: int, d: int, n: int, freqs_ptr: int, k_max: int, out_ptr: int, counts_ptr: int,
@@ -394,6 +469,19 @@ def detect_cfar_dev(surface_ptr: int, p: int, d: int, n: int, freqs_ptr: int, k_
     _check(fn(h.raw, C.c_void_p(surface_ptr), int(p), int(d), int(n), C.c_void_p(freqs_ptr), int(k_max),
               int(guard_doppler), int(guard_delay), int(train_doppler), int(train_delay), float(scale),
               C.c_void_p(out_ptr), C.c_void_p(counts_ptr)))
+
+
+def integrate_dev(needles_ptr: int, haystacks_ptr: int, k: int, l: int, freqs_ptr: int, d: int, fs: int, surface_ptr: int,
+                  row_peak_val_ptr: int = 0, row_peak_idx_ptr: int = 0, peak_ptr: int = 0, *, f32: bool = False,
+                  handle: Optional[Handle] = None):
+    """caf_b200_integrate_{f64,f32}_dev on device pointers (e.g. torch tensors' data_ptr()): needles, haystacks [k][l]
+    (complex128, or complex64 with f32), freqs [d]; surface [d][2l] float64 (required, for both precisions), row peaks
+    [d] float64 / uint64 and the 32-byte peak optional (0 = none).  Asynchronous on the handle's stream."""
+    h = handle or default_handle()
+    fn = getattr(_lib.load(), "caf_b200_integrate_f32_dev" if f32 else "caf_b200_integrate_f64_dev")
+    _check(fn(h.raw, C.c_void_p(needles_ptr or None), C.c_void_p(haystacks_ptr or None), int(k), int(l),
+              C.c_void_p(freqs_ptr or None), int(d), int(fs), C.c_void_p(surface_ptr or None),
+              C.c_void_p(row_peak_val_ptr or None), C.c_void_p(row_peak_idx_ptr or None), C.c_void_p(peak_ptr or None)))
 
 
 def cfar_noise_dev(surface_ptr: int, p: int, d: int, n: int, noise_ptr: int, *, guard_doppler: int = 1,

@@ -27,6 +27,7 @@
 #include "caf_detect.cuh"
 #include "caf_cfar.cuh"
 #include "caf_cfar_os.cuh"
+#include "caf_integrate.cuh"
 #include "overlap_policy.hpp"
 
 namespace {
@@ -63,6 +64,13 @@ struct DevBuf {
 };
 
 template <typename T> struct Tables { caf::cx<T>* tw1 = nullptr; caf::cx<T>* tw2 = nullptr; caf::cx<T>* g = nullptr; };
+
+// Scratch budget of caf_b200_integrate_*: the segment surfaces of one chunk.  Measured on a B200 at config 1, K = 64, f64
+// (DESIGN.md section 13): chunks small enough for the scratch to stay in L2 (2 surfaces, 50 MB) are the slowest, 40.0 us
+// per segment, because every chunk pays the batch launch's set-up and a read-modify-write of the 26 MB accumulator; 8 / 10
+// / 32 / 64 segments take 32.5 / 32.4 / 31.1 / 30.6 us.  256 MB keeps most of that (10 f64 or 20 f32 config-1 segments)
+// with a workspace that stays the same from K = 16 to K = 64; CAF_B200_INTEGRATE_MB trades memory for the rest.
+constexpr size_t kIntegrateMbDefault = 256;
 
 }  // namespace
 
@@ -146,6 +154,7 @@ struct caf_b200_handle_s {
     size_t h_stage_cap = 0;
     DevBuf lwbuf, lhtmp, lhbig, lpart;      // long-row path: chunk scratch, scratch of the H transform, H, partial row maxima
     DevBuf det, det_io;                     // detection: counters | candidate lists; host calls' grid | records | count
+    DevBuf integ, integ_aux;                // integration: a chunk's segment surfaces; row peaks | partial maxima | tickets
     long long* trace = nullptr;   // CAF_TRACE builds: device buffer for phase stamps
     // Launch-private state of single-pair surface launches, a ring of kRing slots indexed by launch number (epoch % kRing):
     // several such launches can be in flight at once (overlap, below).
@@ -183,6 +192,7 @@ struct caf_b200_handle_s {
     cudaEvent_t ev_head = nullptr, ev_copy = nullptr;
     // switches read ONCE, at handle creation (include/caf_b200.h lists them)
     size_t chunk_mb = 6144;                 // CAF_B200_CHUNK_MB
+    size_t integrate_mb = kIntegrateMbDefault;   // CAF_B200_INTEGRATE_MB
     bool allow_pipeline = true;             // CAF_B200_PIPELINE
     bool peak_zero_copy = true;             // CAF_B200_PEAK_ZEROCOPY
     bool ev_valid = false;
@@ -1118,6 +1128,7 @@ static int create_impl(int device, bool own_stream, void* cuda_stream, caf_b200_
     if (const char* e_ = getenv("CAF_B200_PULL")) h->allow_pull = e_[0] != '0';
     if (const char* e_ = getenv("CAF_B200_OVERLAP")) h->overlap_killed = e_[0] == '0';
     if (const char* e_ = getenv("CAF_B200_GATHER_AHEAD")) h->gather_ahead = atoi(e_);
+    if (const char* e_ = getenv("CAF_B200_INTEGRATE_MB")) { const long v_ = atol(e_); if (v_ > 0) h->integrate_mb = (size_t)v_; }
 
     if (!own_stream) { h->stream = (cudaStream_t)cuda_stream; h->own_stream = false; }   // 0 = legacy default stream
     else {
@@ -1165,7 +1176,7 @@ int caf_b200_destroy(caf_b200_handle h) {
     h->surf_pool.clear();
     if (h->copy_stream) cudaStreamSynchronize(h->copy_stream);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    for (DevBuf* b : {&h->in_block, &h->needle, &h->hay, &h->hperm, &h->freqs, &h->surface, &h->rowval, &h->rowidx, &h->peaks, &h->scratch, &h->layout, &h->lwbuf, &h->lhtmp, &h->lhbig, &h->lpart, &h->det, &h->det_io})
+    for (DevBuf* b : {&h->in_block, &h->needle, &h->hay, &h->hperm, &h->freqs, &h->surface, &h->rowval, &h->rowidx, &h->peaks, &h->scratch, &h->layout, &h->lwbuf, &h->lhtmp, &h->lhbig, &h->lpart, &h->det, &h->det_io, &h->integ, &h->integ_aux})
         b->release();
     for (void* q : {(void*)h->td.tw1, (void*)h->td.tw2, (void*)h->td.g, (void*)h->tf.tw1, (void*)h->tf.tw2, (void*)h->tf.g})
         if (q) cudaFree(q);
@@ -1403,6 +1414,21 @@ int caf_b200_batch_f32_dev(caf_b200_handle h, const caf_c64* needles, const caf_
 // ---- device-resident surface objects ------------------------------------------------------------------------
 extern "C++" {
 namespace {
+// s->dev: a buffer a released surface left behind, else a fresh one (cudaMalloc costs more than the whole computation)
+int surface_buffer(caf_b200_handle h, caf_b200_surface s) {
+    size_t best = (size_t)-1;
+    for (size_t i = 0; i < h->surf_pool.size(); ++i)
+        if (h->surf_pool[i].second >= s->bytes && (best == (size_t)-1 || h->surf_pool[i].second < h->surf_pool[best].second)) best = i;
+    if (best != (size_t)-1) {
+        s->dev = h->surf_pool[best].first; s->bytes = h->surf_pool[best].second;
+        h->surf_pool.erase(h->surf_pool.begin() + (long)best);
+        return CAF_B200_OK;
+    }
+    cudaError_t e = cudaMalloc(&s->dev, s->bytes);
+    if (e != cudaSuccess) { s->dev = nullptr; return fail(CAF_B200_ECUDA, std::string("surface buffer: ") + cudaGetErrorString(e)); }
+    return CAF_B200_OK;
+}
+
 template <typename T>
 int surface_create_impl(caf_b200_handle h, const caf::cx<T>* needle, const caf::cx<T>* hay, size_t l, const double* freqs,
                         size_t d, uint32_t fs, caf_b200_surface* out) {
@@ -1419,17 +1445,8 @@ int surface_create_impl(caf_b200_handle h, const caf::cx<T>* needle, const caf::
     s->freqs.assign(freqs, freqs + d);
     s->peak.value = 0.0; s->peak.freq_hz = 0.0; s->peak.doppler_idx = UINT64_MAX; s->peak.delay_idx = 0;
     if (d && l) {
-        // a buffer a released surface left behind, else a fresh one (cudaMalloc costs more than the whole computation)
-        size_t best = (size_t)-1;
-        for (size_t i = 0; i < h->surf_pool.size(); ++i)
-            if (h->surf_pool[i].second >= s->bytes && (best == (size_t)-1 || h->surf_pool[i].second < h->surf_pool[best].second)) best = i;
-        if (best != (size_t)-1) {
-            s->dev = h->surf_pool[best].first; s->bytes = h->surf_pool[best].second;
-            h->surf_pool.erase(h->surf_pool.begin() + (long)best);
-        } else {
-            cudaError_t e = cudaMalloc(&s->dev, s->bytes);
-            if (e != cudaSuccess) { delete s; return fail(CAF_B200_ECUDA, std::string("surface buffer: ") + cudaGetErrorString(e)); }
-        }
+        rc = surface_buffer(h, s);
+        if (rc) { delete s; return rc; }
         s->dev_ri = (unsigned long long*)((char*)s->dev + surf_bytes);
         s->dev_rv = (void*)(s->dev_ri + d);
         // nothing but the fused find_peak result comes back now: the call is a peak-only call that leaves the surface
@@ -1507,6 +1524,174 @@ int caf_b200_surface_destroy(caf_b200_surface s) {
     }
     delete s;
     return CAF_B200_OK;
+}
+
+// ---- non-coherent integration over K segments (caf_integrate.cuh, DESIGN.md section 13) ------------------------------
+extern "C++" {
+namespace {
+// blocks of one row in caf_integrate_kernel
+size_t integrate_parts(size_t l) { return (2 * l + caf::kIntCells - 1) / caf::kIntCells; }
+
+int check_integrate_shape(size_t k, size_t l, size_t d) {
+    if (k == 0) return fail(CAF_B200_EINVAL, "k must be at least one segment");
+    if ((double)d * (double)integrate_parts(l) > 2147483647.0) return fail(CAF_B200_EUNSUPPORTED, "too many rows for one launch");
+    return CAF_B200_OK;
+}
+
+// Segments per chunk: as many surfaces as the scratch budget (CAF_B200_INTEGRATE_MB) holds, at least one, at most k.
+size_t integrate_chunk(caf_b200_handle h, size_t k, size_t seg_bytes) {
+    size_t c = (h->integrate_mb << 20) / seg_bytes;
+    if (c < 1) c = 1;
+    if (c > k) c = k;
+    return c;
+}
+
+// The whole device-side integration; every pointer is device memory and the arguments are checked.  surface is the
+// accumulator; row peaks and peak may be null.
+template <typename T>
+int run_integrate_dev(caf_b200_handle h, const caf::cx<T>* needles, const caf::cx<T>* hays, size_t k, size_t l,
+                      const double* freqs, size_t d, uint32_t fs, double* surface, double* rowval,
+                      unsigned long long* rowidx, caf::PeakOut* peak) {
+    using namespace caf;
+    if (l == 0 || d == 0) {
+        // empty rows: xcor_peak_idx = 0, xcor_peak_val = 0.0 (mod.rs:143-144); find_peak -> dummy row
+        if (d && rowval) CK(cudaMemsetAsync(rowval, 0, sizeof(double) * d, h->stream));
+        if (d && rowidx) CK(cudaMemsetAsync(rowidx, 0, sizeof(unsigned long long) * d, h->stream));
+        if (peak) {
+            PeakOut z; z.value = 0.0; z.freq_hz = 0.0; z.doppler_idx = ~0ull; z.delay_idx = 0;
+            CK(cudaMemcpyAsync(peak, &z, sizeof z, cudaMemcpyDefault, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+        }
+        return CAF_B200_OK;
+    }
+    const size_t n = 2 * l, seg_bytes = sizeof(T) * d * n;
+    const size_t c = integrate_chunk(h, k, seg_bytes);
+    const int parts = (int)integrate_parts(l);
+    const bool rows = rowval || rowidx || peak;
+    CK(h->integ.ensure(seg_bytes * c));
+    // aux: row peak values | indices (when the caller's are null) | partial maxima | their indices | tickets
+    const size_t pv_off = 16 * d, pi_off = pv_off + sizeof(double) * d * (size_t)parts;
+    const size_t tk_off = pi_off + ((sizeof(int) * d * (size_t)parts + 15) & ~(size_t)15);
+    CK(h->integ_aux.ensure(tk_off + sizeof(unsigned int) * d));
+    char* aux = (char*)h->integ_aux.p;
+    IntegrateArgs<T> a{};
+    a.seg = (const T*)h->integ.p; a.acc = surface; a.d = (long long)d; a.n = (long long)n; a.parts = parts;
+    a.row_peak_val = rowval ? rowval : (double*)aux;
+    a.row_peak_idx = rowidx ? rowidx : (unsigned long long*)(aux + 8 * d);
+    a.part_val = (double*)(aux + pv_off); a.part_idx = (int*)(aux + pi_off); a.row_ticket = (unsigned int*)(aux + tk_off);
+    if (rows && parts > 1) CK(cudaMemsetAsync(a.row_ticket, 0, sizeof(unsigned int) * d, h->stream));
+    for (size_t k0 = 0; k0 < k; k0 += c) {
+        const size_t cc = k - k0 < c ? k - k0 : c;
+        // the chunk's surfaces, by the batch path exactly as caf_b200_batch_*_dev computes them
+        int rc = run_batch_dev<T>(h, needles + k0 * l, hays + k0 * l, cc, l, freqs, d, fs, (T*)h->integ.p, nullptr, nullptr,
+                                  nullptr);
+        if (rc) return rc;
+        a.c = (int)cc; a.first = k0 == 0; a.last = rows && k0 + cc == k;
+        // a plain stream-ordered launch: it waits for the chunk, and the next chunk's batch launch, which rewrites the
+        // scratch this one reads, follows a launch outside the overlap history and so waits for it (overlap_policy.hpp)
+        caf_integrate_kernel<T><<<(unsigned)(d * (size_t)parts), kIntThreads, 0, h->stream>>>(a);
+        h->launches++;
+        CK(cudaGetLastError());
+    }
+    if (peak) {
+        caf_peak_kernel<double><<<1, 256, 0, h->stream>>>(a.row_peak_val, a.row_peak_idx, freqs, (int)d, peak);
+        h->launches++;
+        CK(cudaGetLastError());
+    }
+    return CAF_B200_OK;
+}
+
+template <typename T>
+int integrate_dev_impl(caf_b200_handle h, const caf::cx<T>* needles, const caf::cx<T>* hays, size_t k, size_t l,
+                       const double* freqs, size_t d, uint32_t fs, double* surface, double* rowval, uint64_t* rowidx,
+                       caf_b200_peak* peak) {
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_integrate_shape(k, l, d);
+    if (rc) return rc;
+    if (!surface && d && l) return fail(CAF_B200_EINVAL, "null surface (the integrated surface is the accumulator)");
+    rc = check_common<T>(h, needles, hays, k, l, freqs, d, fs);
+    if (rc) return rc;
+    CK(cudaSetDevice(h->device));
+    return run_integrate_dev<T>(h, needles, hays, k, l, freqs, d, fs, surface, rowval, (unsigned long long*)rowidx,
+                                (caf::PeakOut*)peak);
+}
+
+// inputs up, the integration into the surface object's buffer, find_peak's answer down
+template <typename T>
+int integrated_fill(caf_b200_handle h, caf_b200_surface s, const caf::cx<T>* needles, const caf::cx<T>* hays, size_t k,
+                    size_t l, const double* freqs, uint32_t fs) {
+    using namespace caf;
+    const size_t sig_bytes = sizeof(cx<T>) * k * l, fr_bytes = sizeof(double) * s->d;
+    CK(h->needle.ensure(sig_bytes)); CK(h->hay.ensure(sig_bytes)); CK(h->freqs.ensure(fr_bytes));
+    CK(h->peaks.ensure(sizeof(PeakOut)));
+    CK(cudaMemcpyAsync(h->needle.p, needles, sig_bytes, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->hay.p, hays, sig_bytes, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->freqs.p, freqs, fr_bytes, cudaMemcpyHostToDevice, h->stream));
+    int rc = run_integrate_dev<T>(h, (const cx<T>*)h->needle.p, (const cx<T>*)h->hay.p, k, l, (const double*)h->freqs.p,
+                                  s->d, fs, (double*)s->dev, (double*)s->dev_rv, s->dev_ri, (PeakOut*)h->peaks.p);
+    if (rc) return rc;
+    PeakOut pk;
+    CK(cudaMemcpyAsync(&pk, h->peaks.p, sizeof pk, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    to_public(pk, &s->peak);
+    return CAF_B200_OK;
+}
+
+template <typename T>
+int surface_create_integrated_impl(caf_b200_handle h, const caf::cx<T>* needles, const caf::cx<T>* hays, size_t k,
+                                   size_t l, const double* freqs, size_t d, uint32_t fs, caf_b200_surface* out) {
+    if (!out) return fail(CAF_B200_EINVAL, "null out");
+    *out = nullptr;
+    if (!h) return fail(CAF_B200_EINVAL, "null handle");
+    int rc = check_integrate_shape(k, l, d);
+    if (rc) return rc;
+    rc = check_common<T>(h, needles, hays, k, l, freqs, d, fs);
+    if (rc) return rc;
+    CK(cudaSetDevice(h->device));
+    caf_b200_surface s = new (std::nothrow) caf_b200_surface_s();
+    if (!s) return fail(CAF_B200_EINVAL, "out of host memory");
+    s->h = h; s->device = h->device; s->f32 = false; s->d = d; s->n = 2 * l;       // an f64 surface for either input precision
+    const size_t surf_bytes = (sizeof(double) * d * 2 * l + 255) & ~(size_t)255;
+    s->bytes = surf_bytes + 16 * d;                       // surface | row_peak_idx (u64) | row_peak_val (f64)
+    s->freqs.assign(freqs, freqs + d);
+    s->peak.value = 0.0; s->peak.freq_hz = 0.0; s->peak.doppler_idx = UINT64_MAX; s->peak.delay_idx = 0;
+    if (d && l) {
+        rc = surface_buffer(h, s);
+        if (rc) { delete s; return rc; }
+        s->dev_ri = (unsigned long long*)((char*)s->dev + surf_bytes);
+        s->dev_rv = (void*)(s->dev_ri + d);
+        rc = integrated_fill<T>(h, s, needles, hays, k, l, freqs, fs);
+        if (rc) { const std::string why = g_err; caf_b200_surface_destroy(s); return fail(rc, why); }
+    } else {
+        s->peaks_on_host = true; s->pval.assign(d, 0.0); s->pidx.assign(d, 0);      // empty rows: peak 0.0 at index 0 (mod.rs:143-144)
+    }
+    *out = s;
+    return CAF_B200_OK;
+}
+}  // namespace
+}  // extern "C++"
+
+int caf_b200_integrate_f64_dev(caf_b200_handle h, const caf_c128* needles, const caf_c128* haystacks, size_t k, size_t l,
+                               const double* freqs_hz, size_t d, uint32_t fs, double* surface, double* row_peak_val,
+                               uint64_t* row_peak_idx, caf_b200_peak* peak) {
+    return integrate_dev_impl<double>(h, (const double2*)needles, (const double2*)haystacks, k, l, freqs_hz, d, fs, surface,
+                                      row_peak_val, row_peak_idx, peak);
+}
+int caf_b200_integrate_f32_dev(caf_b200_handle h, const caf_c64* needles, const caf_c64* haystacks, size_t k, size_t l,
+                               const double* freqs_hz, size_t d, uint32_t fs, double* surface, double* row_peak_val,
+                               uint64_t* row_peak_idx, caf_b200_peak* peak) {
+    return integrate_dev_impl<float>(h, (const float2*)needles, (const float2*)haystacks, k, l, freqs_hz, d, fs, surface,
+                                     row_peak_val, row_peak_idx, peak);
+}
+int caf_b200_surface_create_integrated_f64(caf_b200_handle h, const caf_c128* needles, const caf_c128* haystacks, size_t k,
+                                           size_t l, const double* freqs_hz, size_t d, uint32_t fs, caf_b200_surface* out) {
+    return surface_create_integrated_impl<double>(h, (const double2*)needles, (const double2*)haystacks, k, l, freqs_hz, d,
+                                                  fs, out);
+}
+int caf_b200_surface_create_integrated_f32(caf_b200_handle h, const caf_c64* needles, const caf_c64* haystacks, size_t k,
+                                           size_t l, const double* freqs_hz, size_t d, uint32_t fs, caf_b200_surface* out) {
+    return surface_create_integrated_impl<float>(h, (const float2*)needles, (const float2*)haystacks, k, l, freqs_hz, d, fs,
+                                                 out);
 }
 
 // ---- detection: the K strongest local maxima of stored surfaces (caf_detect.cuh) ------------------------------------

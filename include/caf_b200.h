@@ -23,6 +23,7 @@
  *
  * Environment (development / measurement switches, read ONCE when a handle is created; none is needed for normal use):
  *    CAF_B200_CHUNK_MB=<n>   scratch budget for rows longer than 8192 cells (default 6144)
+ *    CAF_B200_INTEGRATE_MB=<n>  caf_b200_integrate_*: scratch budget for one chunk of segment surfaces (default 256)
  *    CAF_B200_PIPELINE=0     host surface calls: one launch + one D2H copy instead of head/rest overlap
  *    CAF_B200_PEAK_ZEROCOPY=0  single-pair host calls: copy the peak back instead of storing it into pinned host memory
  *    CAF_B200_PULL=0         single-pair host calls: one H2D copy in front of the kernel instead of the kernel's own CTAs
@@ -395,6 +396,44 @@ int caf_b200_detect_merge_dev(caf_b200_handle h, const caf_b200_detection* lists
                               size_t k_max, double min_ratio, caf_b200_detection* out, uint64_t* count);
 int caf_b200_cfar_merge_dev(caf_b200_handle h, const caf_b200_cfar_detection* lists, const uint64_t* counts, size_t world,
                             size_t k_max, caf_b200_cfar_detection* out, uint64_t* count);
+
+/* ---- non-coherent integration: the CAF surfaces of K signal segments summed cell by cell ----------------------------
+ * A longer coherent window stops paying past a point (Doppler drift and oscillator instability decorrelate it, and the
+ * Doppler bins narrow as 1/T); the standard remedy is to cut the capture into K segments, compute each segment's CAF on
+ * the same Doppler grid and add the K |xcor|^2 surfaces.  The relative spread of the noise floor shrinks as 1/sqrt(K).
+ * needles, haystacks: [k][l] (the batch calls' layout: a capture split into consecutive segments is a [k, l] view);
+ * freqs_hz: d shifts shared by every segment; fs as in the surface calls.  s_i is the surface caf_b200_batch_*_dev gives
+ * for pair i.  The integrated surface, double [d][2l] for BOTH input precisions, is
+ *     S[r][c] = (((+0.0 + s_0[r][c]) + s_1[r][c]) + ...) + s_{k-1}[r][c]
+ * with f32 cells widened to double first (exact) and the adds in double in ascending i, nothing reassociated: the result
+ * does not depend on how the work is chunked, and a numpy loop `acc += s_i.astype(np.float64)` gives it bit for bit
+ * (np.sum, which adds pairwise, does not).  Row peaks and peak follow the surface calls' rules in double: a row's peak is
+ * its first cell holding the row's maximum (mod.rs:141-153), 0.0 at cell 0 for an all-zero row; peak is find_peak over
+ * the rows (mod.rs:31-42), the lowest row winning a tie.  l == 0 or d == 0 behave as in the batch calls.
+ * The detectors above run on S unchanged.  Their CFAR scales assume exponential cells, which one segment's |.|^2 of noise
+ * is; a sum of k is Gamma(k): the Python package's cfar_scale(pfa, N, looks=k) gives the CA-CFAR scale for it (no closed
+ * form exists for OS-CFAR).
+ * Limits: check_common's with p = k (k * d <= 2e9 and k, d <= 2^30); k == 0, a null required pointer or fs == 0 is
+ * CAF_B200_EINVAL, l > 2^19 is CAF_B200_EUNSUPPORTED; a call that fails writes nothing.
+ * Scratch, independent of k: the handle's grow-only workspace holds one chunk of c segment surfaces, c = max(1, min(k,
+ * CAF_B200_INTEGRATE_MB MB / (sizeof(cell) * d * 2l))), plus 20 + 12 * ceil(2l / 1024) bytes per row, plus what the batch
+ * calls use for c pairs. */
+/* every pointer is device memory; surface is required (unless d * l == 0), row_peak_val / row_peak_idx [d] and peak may be NULL.  Asynchronous
+ * on the handle's stream: per chunk the batch path's launches and one plain stream-ordered accumulation launch (they count
+ * in launch_count and end any overlap, caf_b200_set_overlap), then find_peak when peak is wanted. */
+int caf_b200_integrate_f64_dev(caf_b200_handle h, const caf_c128* needles, const caf_c128* haystacks, size_t k, size_t l,
+                               const double* freqs_hz, size_t d, uint32_t fs, double* surface, double* row_peak_val,
+                               uint64_t* row_peak_idx, caf_b200_peak* peak);
+int caf_b200_integrate_f32_dev(caf_b200_handle h, const caf_c64* needles, const caf_c64* haystacks, size_t k, size_t l,
+                               const double* freqs_hz, size_t d, uint32_t fs, double* surface, double* row_peak_val,
+                               uint64_t* row_peak_idx, caf_b200_peak* peak);
+/* host inputs; the result is an f64 surface object (whatever the input precision) on which caf_b200_surface_{shape,
+ * row_peaks, find_peak, fetch_rows (doubles), detect, detect_cfar, detect_cfar_os, destroy} work unchanged; synchronous */
+int caf_b200_surface_create_integrated_f64(caf_b200_handle h, const caf_c128* needles, const caf_c128* haystacks, size_t k,
+                                           size_t l, const double* freqs_hz, size_t d, uint32_t fs, caf_b200_surface* out);
+int caf_b200_surface_create_integrated_f32(caf_b200_handle h, const caf_c64* needles, const caf_c64* haystacks, size_t k,
+                                           size_t l, const double* freqs_hz, size_t d, uint32_t fs, caf_b200_surface* out);
+
 /* ---- the sibling programs' layouts of the same surface (SURVEY.md section 8(f)4) -------------------
  * The reference's Go and Python programs compute this correlation with the operands swapped and keep the
  * magnitude |xcor| (cmplx.Abs, np.abs) where the Rust crate keeps |xcor|^2 (norm_sqr):

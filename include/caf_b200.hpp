@@ -149,6 +149,24 @@ struct CafB200 {
         for (std::size_t r = 0; r < freqs_hz.size(); ++r) rows.emplace_back(surf, r);
         return rows;
     }
+    // Non-coherent integration (caf_b200_surface_create_integrated_f64): needles and haystacks hold k consecutive segments
+    // of l = needles.size() / k samples; the rows are ONE surface on the GPU, the cell-by-cell sum of the k segments'
+    // |xcor|^2 surfaces in double.  find_peak, the rows' fields and the detectors work on it as on caf_surface's rows, and
+    // like those it belongs to the calling thread's handle (detection refuses other threads).
+    static std::vector<CafSurfaceRow> integrate(const std::vector<Complex64>& needles, const std::vector<Complex64>& haystacks,
+                                                std::size_t k, const std::vector<double>& freqs_hz, uint32_t fs) {
+        if (needles.size() != haystacks.size()) throw Panic("assertion failed: a.len() == self.n (xcor_rustfft.rs:54-55)");
+        if (k == 0 || needles.size() % k) throw Panic("integrate needs k > 0 segments of equal length");
+        caf_b200_surface raw = nullptr;
+        check(caf_b200_surface_create_integrated_f64(thread_handle(), reinterpret_cast<const caf_c128*>(needles.data()),
+                                                     reinterpret_cast<const caf_c128*>(haystacks.data()), k, needles.size() / k,
+                                                     freqs_hz.data(), freqs_hz.size(), fs, &raw));
+        auto surf = std::make_shared<const DeviceSurface>(raw);
+        std::vector<CafSurfaceRow> rows;
+        rows.reserve(freqs_hz.size());
+        for (std::size_t r = 0; r < freqs_hz.size(); ++r) rows.emplace_back(surf, r);
+        return rows;
+    }
     // mod.rs:31-42: strict > from a dummy row (0.0, peak 0.0) in VECTOR order; consumes the surface like the reference.
     // When `arr` is what caf_surface returned, untouched (all rows of one surface, in order), that scan is exactly what
     // the kernel's fused find_peak already did; any other vector (reordered, truncated, rows of several surfaces) is

@@ -152,6 +152,25 @@ strategy!(CafB200, CafFFTW, CafRustFFT, CafRustFFTRayon, CafRustFFTIter, CafRust
           CafRustFFTThreadpool);
 
 impl CafB200 {
+    /// Non-coherent integration (include/caf_b200.h, caf_b200_surface_create_integrated_f64): `needles` and `haystacks`
+    /// hold `k` consecutive segments of `l = needles.len() / k` samples each; the result is the rows of ONE surface, the
+    /// cell-by-cell sum of the k segments' |xcor|^2 surfaces, in double, kept on the GPU like `caf_surface`'s.  find_peak,
+    /// the rows' fields and the detectors work on it unchanged (same thread rule).  Panics when k is 0 or does not divide
+    /// the lengths.
+    pub fn integrate(needles: &[Complex64], haystacks: &[Complex64], k: usize, freqs_hz: &[f64], fs: u32)
+                     -> Vec<CafSurfaceRow> {
+        assert!(needles.len() == haystacks.len());           // xcor_rustfft.rs:54-55
+        assert!(k > 0 && needles.len() % k == 0, "integrate needs k > 0 segments of equal length");
+        let l = needles.len() / k;
+        let mut raw: ffi::caf_b200_surface = std::ptr::null_mut();
+        ffi::HANDLE.with(|h| ffi::check(unsafe {
+            ffi::caf_b200_surface_create_integrated_f64(h.0, needles.as_ptr(), haystacks.as_ptr(), k, l, freqs_hz.as_ptr(),
+                                                        freqs_hz.len(), fs, &mut raw)
+        }));
+        let surface = Arc::new(DeviceSurface { raw, rows: freqs_hz.len(), cells: 2 * l, peaks: OnceCell::new(),
+                                               owner: std::thread::current().id() });
+        (0..freqs_hz.len()).map(|row| CafSurfaceRow { surface: surface.clone(), row }).collect()
+    }
     /// The `k_max` strongest local maxima of the surface behind `arr`, best first, each refined below the grid
     /// (include/caf_b200.h, caf_b200_surface_detect).  `arr` must be what `caf_surface` returned, untouched: a reordered or
     /// partial vector no longer names one surface, so it panics.  It also panics off the thread that called `caf_surface`:

@@ -1,6 +1,6 @@
 //! Hand-written extern "C" block for include/caf_b200.h (only what the crate API needs).
 #![allow(non_camel_case_types, dead_code)]
-use num_complex::Complex64;
+use num_complex::{Complex32, Complex64};
 use std::os::raw::{c_char, c_int, c_void};
 
 #[repr(C)]
@@ -64,6 +64,19 @@ extern "C" {
     pub fn caf_b200_surface_find_peak(s: caf_b200_surface, out: *mut caf_b200_peak) -> c_int;
     pub fn caf_b200_surface_fetch_rows(s: caf_b200_surface, row0: usize, count: usize, out: *mut c_void) -> c_int;
     pub fn caf_b200_surface_destroy(s: caf_b200_surface) -> c_int;
+    // non-coherent integration: the surfaces of k segment pairs [k][l] summed cell by cell into one f64 surface
+    pub fn caf_b200_surface_create_integrated_f64(h: caf_b200_handle, needles: *const Complex64, haystacks: *const Complex64,
+                                                  k: usize, l: usize, freqs_hz: *const f64, d: usize, fs: u32,
+                                                  out: *mut caf_b200_surface) -> c_int;
+    pub fn caf_b200_surface_create_integrated_f32(h: caf_b200_handle, needles: *const Complex32, haystacks: *const Complex32,
+                                                  k: usize, l: usize, freqs_hz: *const f64, d: usize, fs: u32,
+                                                  out: *mut caf_b200_surface) -> c_int;
+    pub fn caf_b200_integrate_f64_dev(h: caf_b200_handle, needles: *const Complex64, haystacks: *const Complex64, k: usize,
+                                      l: usize, freqs_hz: *const f64, d: usize, fs: u32, surface: *mut f64,
+                                      row_peak_val: *mut f64, row_peak_idx: *mut u64, peak: *mut caf_b200_peak) -> c_int;
+    pub fn caf_b200_integrate_f32_dev(h: caf_b200_handle, needles: *const Complex32, haystacks: *const Complex32, k: usize,
+                                      l: usize, freqs_hz: *const f64, d: usize, fs: u32, surface: *mut f64,
+                                      row_peak_val: *mut f64, row_peak_idx: *mut u64, peak: *mut caf_b200_peak) -> c_int;
     // detection: the strongest local maxima of a stored surface (host records), or of device surfaces [p][d][n]
     pub fn caf_b200_surface_detect(s: caf_b200_surface, k_max: usize, guard_doppler: u32, guard_delay: u32, min_ratio: f64,
                                    out: *mut caf_b200_detection, count: *mut usize) -> c_int;

@@ -4,7 +4,7 @@
 // ("Use CLAP to take in two c64 files as arguments", main.rs:1-2).  This is that program with the arguments:
 //
 //   caf_cli NEEDLE.c64 HAYSTACK.c64 [--fmin HZ] [--fmax HZ] [--fstep HZ] [--fs HZ]
-//           [--layout rust|go|python] [--dump FILE] [--device-load]
+//           [--layout rust|go|python] [--dump FILE] [--device-load] [--segments K]
 //           [--detect K [--guard-doppler R] [--guard-delay C] [--min-db X |
 //                        --cfar-db X [--train-doppler A] [--train-delay B] [--cfar-rank K]]]
 //
@@ -23,6 +23,11 @@
 // cells beyond the guards, default 2 x 16), at most K of them and possibly none; each line ends with its SNR.
 // --cfar-rank K (with --cfar-db) estimates the noise as the K-th smallest training cell instead of their mean
 // (ordered-statistic CFAR, caf_b200_surface_detect_cfar_os; 1 <= K <= the training cells); the lines are the same.
+// --segments K (default 1) integrates non-coherently: the needle file supplies K consecutive segments of L = len / K
+// samples (the tail is dropped) and the haystack file the same K windows; the report lines and --detect / --cfar-db /
+// --cfar-rank then run on the sum of the K segments' surfaces (caf_b200_surface_create_integrated_f64).  --cfar-db is a
+// scale in dB either way; cfar_scale(pfa, N, looks=K) of the Python package gives the one for a sum of K.  --segments 1
+// is the plain program.
 // Build: g++ -std=c++17 -O2 -Iinclude tools/caf_cli.cpp -Lcaf_cookoff_b200 -lcaf_b200 -Wl,-rpath,$PWD/caf_cookoff_b200
 #include <cmath>
 #include <cstdio>
@@ -58,6 +63,7 @@ int main(int argc, char** argv) {
     uint32_t train_doppler = 2, train_delay = 16;
     bool train_given = false;
     uint32_t cfar_rank = 0;                                     // 0: cell-averaging CFAR
+    std::size_t segments = 1;
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
         auto need = [&](const char* what) -> const char* {
@@ -92,10 +98,11 @@ int main(int argc, char** argv) {
         }
         else if (a == "--train-doppler") { train_doppler = (uint32_t)count_arg("--train-doppler", need("--train-doppler"), 0, 32); train_given = true; }
         else if (a == "--train-delay") { train_delay = (uint32_t)count_arg("--train-delay", need("--train-delay"), 0, 256); train_given = true; }
+        else if (a == "--segments") segments = count_arg("--segments", need("--segments"), 1, 1ul << 20);
         else if (a == "--cfar-rank") cfar_rank = (uint32_t)count_arg("--cfar-rank", need("--cfar-rank"), 1, 65 * 513);
         else if (a == "-h" || a == "--help") {
             std::printf("usage: caf_cli NEEDLE.c64 HAYSTACK.c64 [--fmin HZ] [--fmax HZ] [--fstep HZ] [--fs HZ] "
-                        "[--layout rust|go|python] [--dump FILE] [--device-load] "
+                        "[--layout rust|go|python] [--dump FILE] [--device-load] [--segments K] "
                         "[--detect K [--guard-doppler R] [--guard-delay C] "
                         "[--min-db X | --cfar-db X [--train-doppler A] [--train-delay B] [--cfar-rank K]]]\n");
             return 0;
@@ -113,6 +120,10 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "caf_cli: --detect goes with the default report (no --layout / --dump / --device-load)\n");
         return 2;
     }
+    if (segments > 1 && (device_load || layout != "rust" || !dump.empty())) {
+        std::fprintf(stderr, "caf_cli: --segments goes with the default report (no --layout / --dump / --device-load)\n");
+        return 2;
+    }
     try {
         if (device_load) {
             if (layout != "rust" || !dump.empty()) { std::fprintf(stderr, "caf_cli: --device-load goes with the default report (no --layout / --dump)\n"); return 2; }
@@ -125,13 +136,22 @@ int main(int argc, char** argv) {
         auto needle = read_file_c64(pos[0]);
         auto haystack = read_file_c64(pos[1]);
         haystack.resize(needle.size());                                  // main.rs:15
+        if (segments > 1) {                                              // K windows of L samples, the tail dropped
+            const std::size_t seg_l = needle.size() / segments;
+            if (seg_l == 0) { std::fprintf(stderr, "caf_cli: --segments %zu needs at least that many samples\n", segments); return 2; }
+            needle.resize(segments * seg_l);
+            haystack.resize(segments * seg_l);
+        }
         const auto shifts = gen_float_shifts(fmin, fmax, fstep);         // integer milli-Hz range, main.rs:18-22 / test.rs:335-352
         const std::size_t l = needle.size(), d = shifts.size();
         if (layout == "rust") {
-            if (detecting) {
-                const auto rows = CafB200::caf_surface(needle, haystack, shifts, fs);          // the surface stays on the GPU
+            if (detecting || segments > 1) {
+                // the surface (or the sum of the segments' surfaces) stays on the GPU
+                const auto rows = segments > 1 ? CafB200::integrate(needle, haystack, segments, shifts, fs)
+                                               : CafB200::caf_surface(needle, haystack, shifts, fs);
                 const auto [freq, idx] = CafB200::find_peak(rows);
                 std::printf("Frequency offset: %.1fHz\nTime offset: %zu samples (%.3fms)\n", freq, idx, (double)idx / ((double)fs / 1e3));
+                if (!detecting) return 0;
                 if (cfar) {
                     const double scale = std::pow(10.0, cfar_db / 10.0);
                     const auto dets = cfar_rank ? CafB200::detect_cfar_os(rows, detect_k, guard_doppler, guard_delay,
